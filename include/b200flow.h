@@ -237,8 +237,33 @@ B200_API int b200_corr3d_fwd(const float* xyz1, const float* feat1, const float*
                     float* out, float* scratch,
                     int B, int Cin, int Cout, int N1, int N2, int k, int precision, b200_stream_t stream);
 
+/* a5 backward: gradients of b200_corr3d_fwd with respect to both clouds, both feature maps and the 16 parameters.
+ * Replaces the autograd graph of models/pwc3d_core.py:69-117 (fp32 FFMA arithmetic, whatever precision the forward used).
+ *   inputs, knn12, knn11, w, B..k : exactly as given to the forward
+ *   grad_out    : [B,Cout,N1] channel-first, the gradient of `out`
+ *   fwd_scratch : the forward's scratch, unchanged since the forward returned (its point-major P [B,N1,Cout] is read)
+ *   grads       : output pointers, same shapes as the tensors they differentiate (xyz [B,3,N], feat [B,Cin,N], weights
+ *                 [out,in] / [out]).  NULL = not needed: its work is skipped and it is not written.  Every non-NULL
+ *                 output is overwritten (the callee zero-fills what it accumulates).
+ *   scratch     : >= b200_corr3d_bwd_scratch_floats(B,Cin,Cout,N1,N2,k) floats, 16-byte aligned.
+ * Gradients of the clouds, the feature maps and W1's feature columns are summed with float atomics, so they are not
+ * bit-reproducible from run to run; the other weight gradients are.  No host synchronisation, no allocation.
+ */
+typedef struct b200_corr3d_grads {
+    float *xyz1, *feat1, *xyz2, *feat2;
+    float *W1, *b1, *W2, *b2;
+    float *n1_Wa, *n1_ba, *n1_Wb, *n1_bb, *n1_Wc, *n1_bc;
+    float *n2_Wa, *n2_ba, *n2_Wb, *n2_bb, *n2_Wc, *n2_bc;
+} b200_corr3d_grads;
+
+B200_API int64_t b200_corr3d_bwd_scratch_floats(int B, int Cin, int Cout, int N1, int N2, int k);
+B200_API int b200_corr3d_bwd(const float* xyz1, const float* feat1, const float* xyz2, const float* feat2,
+                    const int64_t* knn12, const int64_t* knn11, const b200_corr3d_weights* w,
+                    const float* grad_out, const float* fwd_scratch, const b200_corr3d_grads* grads, float* scratch,
+                    int B, int Cin, int Cout, int N1, int N2, int k, b200_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------------
- * a9  event voxel grid, integer pixels + temporal bilinear (FlyingThings3D / EKubric).
+ * a9 event voxel grid, integer pixels + temporal bilinear (FlyingThings3D / EKubric).
  * Replaces: event_utils.py:109-128 (eventsToVoxel/eventsToVoxelTorch) -> :23-39, :264-303, :211-261, :162-208.
  *   events : [n,4] fp32 rows (x,y,t,p), time-sorted        vox : [bins*(polarity?2:1), H, W] fp32
  *   The kernel zero-fills vox itself.  status[0] counts events whose truncated pixel is outside the grid

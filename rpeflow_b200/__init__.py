@@ -6,6 +6,7 @@ Public surface (same names as the reference, danqu130/RPEFlow):
   projection  batch_indexing_channel_{first,last}, grid_sample_wrapper, project_feat_with_nn_corr,
               knn_interpolation, backwarp_3d, backwarp_2d, convex_upsample    (models/utils.py)
   pwc3d       Correlation3D, build_pc_pyramid                                 (models/pwc3d_core.py)
+              correlation3d, Correlation3DFunction — the same op with a backward (b200_corr3d_bwd)
   pointconv   PointConvDownSampling, PointConvNoSampling                      (models/pointconv.py)
   events      eventsToVoxel, eventsToVoxelInter                               (event_utils.py, dsec.py)
   install     install() — plug all of the above into an unmodified reference checkout
@@ -18,7 +19,8 @@ from .ops import (correlation2d, correlation2d_leaky, warp_correlate, furthest_p
                   k_nearest_neighbor, squared_distance, CorrelationFunction)
 from .projection import (batch_indexing_channel_first, batch_indexing_channel_last, grid_sample_wrapper,  # noqa: F401
                          project_feat_with_nn_corr, knn_interpolation, backwarp_3d, backwarp_2d, convex_upsample)
-from .pwc3d import Correlation3D, build_pc_pyramid, correlation3d_forward  # noqa: F401
+from .pwc3d import (Correlation3D, Correlation3DFunction, build_pc_pyramid, correlation3d,  # noqa: F401
+                    correlation3d_forward)
 from .pointconv import PointConvDownSampling, PointConvNoSampling, pointconv_forward  # noqa: F401
 from .events import eventsToVoxel, eventsToVoxelInter  # noqa: F401
 

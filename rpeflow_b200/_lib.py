@@ -9,7 +9,7 @@ import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("B200FLOW_LIB") or os.path.join(_HERE, "libb200flow.so")     # the override is for kernel A/B builds
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 c_i, c_i64, c_p = ctypes.c_int, ctypes.c_int64, ctypes.c_void_p
 
@@ -19,6 +19,12 @@ class Corr3dWeights(ctypes.Structure):
     NAMES = ("W1", "b1", "W2", "b2",
              "n1_Wa", "n1_ba", "n1_Wb", "n1_bb", "n1_Wc", "n1_bc",
              "n2_Wa", "n2_ba", "n2_Wb", "n2_bb", "n2_Wc", "n2_bc")
+    _fields_ = [(n, c_p) for n in NAMES]
+
+
+class Corr3dGrads(ctypes.Structure):
+    """struct b200_corr3d_grads (include/b200flow.h): the 4 input gradients, then the 16 parameter gradients."""
+    NAMES = ("xyz1", "feat1", "xyz2", "feat2") + Corr3dWeights.NAMES
     _fields_ = [(n, c_p) for n in NAMES]
 
 
@@ -57,6 +63,9 @@ SIGNATURES = {
     "b200_corr3d_scratch_floats": (c_i64, [c_i, c_i, c_i, c_i, c_i, c_i]),
     "b200_corr3d_fwd": (c_i, [c_p, c_p, c_p, c_p, c_p, c_p, ctypes.POINTER(Corr3dWeights), c_p, c_p,
                               c_i, c_i, c_i, c_i, c_i, c_i, c_i, c_p]),
+    "b200_corr3d_bwd_scratch_floats": (c_i64, [c_i, c_i, c_i, c_i, c_i, c_i]),
+    "b200_corr3d_bwd": (c_i, [c_p, c_p, c_p, c_p, c_p, c_p, ctypes.POINTER(Corr3dWeights), c_p, c_p,
+                              ctypes.POINTER(Corr3dGrads), c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_p]),
     "b200_event_voxel_int": (c_i, [c_p, c_i64, c_p, c_i, c_i, c_i, c_i, c_p, c_p]),
     "b200_event_voxel_trilinear": (c_i, [c_p, c_p, c_p, c_p, c_i64, c_p, c_i, c_i, c_i, c_i, c_p, c_p]),
 }
@@ -83,7 +92,7 @@ def _load():
 B200_ENOSUP = -3        # include/b200flow.h
 lib = _load()
 LAUNCHES = 0          # kernels of this library launched by this process (bench.py reports it as gpu_launches)
-KERNELS_PER_CALL = {"b200_knn_grid": 3, "b200_knn_grid_cf": 3, "b200_pointconv_fwd": 2, "b200_corr2d_bwd": 2, "b200_project_nn_corr": 2, "b200_corr3d_fwd": 5, "b200_event_voxel_trilinear": 3}
+KERNELS_PER_CALL = {"b200_knn_grid": 3, "b200_knn_grid_cf": 3, "b200_pointconv_fwd": 2, "b200_corr2d_bwd": 2, "b200_project_nn_corr": 2, "b200_corr3d_fwd": 5, "b200_corr3d_bwd": 10, "b200_event_voxel_trilinear": 3}
 
 
 class B200Error(RuntimeError):

@@ -40,7 +40,7 @@ int sm_count() {
 
 extern "C" {
 
-int b200_abi_version(void) { return 7; }
+int b200_abi_version(void) { return 8; }
 
 const char* b200_build_info(void) {
     return "libb200flow sm_100a; nvcc " B200_STR(__CUDACC_VER_MAJOR__) "." B200_STR(__CUDACC_VER_MINOR__)

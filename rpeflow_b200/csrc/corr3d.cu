@@ -291,6 +291,19 @@ static cudaError_t launch_stage1(const float* xyz1, const float* xyz2, const int
     return cudaGetLastError();
 }
 
+// passes 0 and 1 for the backward (corr3d_bwd.cu), which recomputes A1 / G2 into its own copy of the scratch layout
+cudaError_t corr3d_prep_and_linears(const float* feat1, const float* feat2, const b200_corr3d_weights* w, const Corr3dScratch& s,
+                                    int B, int Cin, int Cout, int N1, int N2, cudaStream_t st) {
+    const int Kin = 2 * Cin + 3;
+    corr3d_prep_weights<<<ceil_div(Cout * (Cout + 19), 256), 256, 0, st>>>(w->W1, w->W2, w->n1_Wc, w->n2_Wc, s.W2T, s.W1cT,
+                                                                         s.n1WcT, s.n2WcT, Cin, Cout);
+    pointwise_linear_kernel<<<dim3(ceil_div(N1, PL_TN), ceil_div(Cout, PL_TO), B), 256, 0, st>>>(feat1, w->W1, w->b1, s.A1, Cin,
+                                                                                               Kin, 0, Cout, N1);
+    pointwise_linear_kernel<<<dim3(ceil_div(N2, PL_TN), ceil_div(Cout, PL_TO), B), 256, 0, st>>>(feat2, w->W1, nullptr, s.G2, Cin,
+                                                                                               Kin, Cin, Cout, N2);
+    return cudaGetLastError();
+}
+
 }  // namespace b200
 
 extern "C" int64_t b200_corr3d_scratch_floats(int B, int Cin, int Cout, int N1, int N2, int k) {

@@ -88,6 +88,10 @@ __device__ __forceinline__ void weight_net_hidden_s(const float* s_wn, float dx,
 }
 
 
+// corr3d.cu: the weight transposes and the two pointwise linears (A1 with b1, G2) into s, fp32
+cudaError_t corr3d_prep_and_linears(const float* feat1, const float* feat2, const b200_corr3d_weights* w, const Corr3dScratch& s,
+                                    int B, int Cin, int Cout, int N1, int N2, cudaStream_t st);
+
 // corr3d_tc.cu: pass 2 on tcgen05 tensor cores (precision 1 = TF32, 2 = 3xTF32); false -> caller uses the fp32 kernel
 bool corr3d_stage1_tc_eligible(int Cout, int k, int precision);
 cudaError_t corr3d_stage1_tc(const float* xyz1, const float* xyz2, const int64_t* knn12, const Corr3dScratch& s,

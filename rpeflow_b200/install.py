@@ -22,6 +22,10 @@ What ``install()`` does
 Every re-bound callable decides PER CALL: the CUDA kernel runs only when all tensor arguments are fp32 (or index)
 CUDA tensors, autograd does not need a graph through the op, and the arguments are inside what the kernel was
 built for; anything else goes to the reference's own function, untouched.  ``stats()`` counts both routes per op.
+
+``install(train=True)`` additionally sends ``Correlation3D.forward`` calls that DO need a graph to
+``pwc3d.Correlation3DFunction`` (forward b200_corr3d_fwd, backward b200_corr3d_bwd), under the same limits, unless
+``torch.use_deterministic_algorithms(True)`` is set (the backward sums with float atomics): those go to the reference.
 """
 import importlib
 import sys
@@ -41,6 +45,7 @@ _SAVED = []            # (object, attribute, previous value) in the order they w
 _ADDED_MODULES = []    # sys.modules keys registered by install()
 _STATS = {}
 _OBSERVER = None
+_TRAIN = False         # install(train=True): Correlation3D calls that need a graph run Correlation3DFunction
 
 
 def stats(reset=False):
@@ -135,8 +140,15 @@ def _corr3d_forward(self, xyz1, feat1, xyz2, feat2, knn_indices_1in1=None):
     """Correlation3D.forward (pwc3d_core.py:69-117) through b200_corr3d_fwd when no graph is needed."""
     import torch.nn as nn
     plain = all(isinstance(c.norm_fn, nn.Identity) for mlp in (self.cost_mlp, self.weight_net1, self.weight_net2) for c in mlp.convs)
-    if (_needs_graph(self, xyz1, feat1, xyz2, feat2) or not _all_cuda_f32(xyz1, feat1, xyz2, feat2) or not plain
-            or self.k > 32 or feat1.shape[1] > 512):
+    fits = _all_cuda_f32(xyz1, feat1, xyz2, feat2) and plain and self.k <= 32 and feat1.shape[1] <= 512
+    if fits and _TRAIN and _needs_graph(self, xyz1, feat1, xyz2, feat2) and not torch.are_deterministic_algorithms_enabled():
+        _count("Correlation3D.forward", "b200")
+        knn12 = ops.k_nearest_neighbor(input_xyz=xyz2.detach(), query_xyz=xyz1.detach(), k=self.k)
+        if knn_indices_1in1 is None:
+            knn_indices_1in1 = ops.k_nearest_neighbor(input_xyz=xyz1.detach(), query_xyz=xyz1.detach(), k=self.k)
+        return pwc3d.correlation3d(xyz1, feat1, xyz2, feat2, pwc3d.param_weights(self), knn12, knn_indices_1in1,
+                                   getattr(self, "b200_precision", 2))
+    if _needs_graph(self, xyz1, feat1, xyz2, feat2) or not fits:
         _count("Correlation3D.forward", "reference")
         return self._b200_reference_forward(xyz1, feat1, xyz2, feat2, knn_indices_1in1)
     _count("Correlation3D.forward", "b200")
@@ -338,7 +350,11 @@ def patch_python_ops(patch_events=True, only=None):
             pass
 
 
-def install(patch_python=True, patch_events=False, only=None, extensions=True):
+def install(patch_python=True, patch_events=False, only=None, extensions=True, train=False):
+    """train=True: Correlation3D.forward calls that need an autograd graph run this library's forward and backward
+    (pwc3d.Correlation3DFunction) instead of the reference's torch code; the default routes them to the reference."""
+    global _TRAIN
+    _TRAIN = bool(train)
     if extensions:
         register_extension_shims()
     if patch_python:
@@ -347,6 +363,8 @@ def install(patch_python=True, patch_events=False, only=None, extensions=True):
 
 def uninstall():
     """Undo install(): every replaced attribute and sys.modules entry gets its previous value back."""
+    global _TRAIN
+    _TRAIN = False
     while _SAVED:
         obj, name, old = _SAVED.pop()
         if obj is sys.modules:
