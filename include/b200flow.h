@@ -198,6 +198,41 @@ B200_API int b200_pointconv_fwd(const float* xyz, const float* feat, const float
                        const b200_pointconv_weights* w, float* out, float* scratch,
                        int B, int C, int Cout, int N, int S, int k, int precision, b200_stream_t stream);
 
+/* f1 for training: the same call without the activation.  Same arguments and scratch as b200_pointconv_fwd; writes
+ *   out [B,Cout,S] = y, the nn.Linear output (models/pointconv.py before norm_fn / activation_fn), so that a caller can
+ *   apply any norm and activation itself.  LeakyReLU(0.1) of it equals b200_pointconv_fwd bit for bit.
+ * Limits: k == 16, Cout <= 256, N <= 65536 (B200_ENOSUP otherwise).
+ */
+B200_API int b200_pointconv_fwd_linear(const float* xyz, const float* feat, const float* sampled_xyz, const int64_t* knn,
+                       const b200_pointconv_weights* w, float* out, float* scratch,
+                       int B, int C, int Cout, int N, int S, int k, int precision, b200_stream_t stream);
+
+/* f1 backward: gradients of b200_pointconv_fwd_linear with respect to both clouds, the features and the six parameters.
+ * Replaces the autograd graph of models/pointconv.py:33-61 / :90-122 up to the Linear output.  M and the weight net are
+ * recomputed from the inputs; the two Linear-sized contractions (dM = dy.L, dL = dy^T.M) run on tcgen05 tensor cores
+ * (3xTF32), the rest in fp32.
+ *   inputs, knn, w, B..k : exactly as given to the forward
+ *   grad_y  : [B,Cout,S] channel-first, the gradient of y
+ *   grads   : output pointers, same shapes as the tensors they differentiate (xyz [B,3,N], feat [B,C,N], sampled_xyz
+ *             [B,3,S], weights as in b200_pointconv_weights).  NULL = not needed: its work is skipped and it is not
+ *             written.  Every non-NULL output is overwritten.  For PointConvNoSampling (sampled_xyz = xyz) the caller
+ *             adds the xyz and sampled_xyz gradients.
+ *   scratch : >= b200_pointconv_bwd_scratch_floats(B,C,Cout,N,S) floats, 16-byte aligned.  It holds the point-major
+ *             feature rows and their gradient (2 x B*N*roundup16(C+3) floats) and per-chunk M / dM images of at most
+ *             32 MB each, whatever the batch.
+ * Gradients of xyz, feat and sampled_xyz are summed with float atomics, so they are not bit-reproducible from run to
+ * run; the parameter gradients are (per-CTA partials, fixed-order reduction).  No host synchronisation, no allocation.
+ * Limits: k == 16, Cout <= 256, N <= 65536 (B200_ENOSUP otherwise).  B = 0 or S = 0 is a no-op; C = 0 is valid.
+ */
+typedef struct b200_pointconv_grads {
+    float *xyz, *feat, *sampled_xyz;
+    float *Wa, *ba, *Wb, *bb, *L, *bias;
+} b200_pointconv_grads;
+B200_API int64_t b200_pointconv_bwd_scratch_floats(int B, int C, int Cout, int N, int S);
+B200_API int b200_pointconv_bwd(const float* xyz, const float* feat, const float* sampled_xyz, const int64_t* knn,
+                       const b200_pointconv_weights* w, const float* grad_y, const b200_pointconv_grads* grads,
+                       float* scratch, int B, int C, int Cout, int N, int S, int k, b200_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------------
  * f2  inverse-distance interpolation over k nearest neighbours (SURVEY §8f rank 2).
  * Replaces: models/utils.py:140-156 (knn_interpolation) after its k_nearest_neighbor call — the two

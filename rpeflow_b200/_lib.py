@@ -34,6 +34,12 @@ class PointConvWeights(ctypes.Structure):
     _fields_ = [(n, c_p) for n in NAMES]
 
 
+class PointConvGrads(ctypes.Structure):
+    """struct b200_pointconv_grads (include/b200flow.h): the 3 input gradients, then the 6 parameter gradients."""
+    NAMES = ("xyz", "feat", "sampled_xyz") + PointConvWeights.NAMES
+    _fields_ = [(n, c_p) for n in NAMES]
+
+
 # name -> (restype, argtypes); one entry per symbol declared in include/b200flow.h
 SIGNATURES = {
     "b200_abi_version": (c_i, []),
@@ -59,6 +65,11 @@ SIGNATURES = {
     "b200_pointconv_scratch_floats": (c_i64, [c_i, c_i, c_i, c_i]),
     "b200_pointconv_fwd": (c_i, [c_p, c_p, c_p, c_p, ctypes.POINTER(PointConvWeights), c_p, c_p,
                                  c_i, c_i, c_i, c_i, c_i, c_i, c_i, c_p]),
+    "b200_pointconv_fwd_linear": (c_i, [c_p, c_p, c_p, c_p, ctypes.POINTER(PointConvWeights), c_p, c_p,
+                                        c_i, c_i, c_i, c_i, c_i, c_i, c_i, c_p]),
+    "b200_pointconv_bwd_scratch_floats": (c_i64, [c_i, c_i, c_i, c_i, c_i]),
+    "b200_pointconv_bwd": (c_i, [c_p, c_p, c_p, c_p, ctypes.POINTER(PointConvWeights), c_p, ctypes.POINTER(PointConvGrads),
+                                 c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_p]),
     "b200_knn_interpolate": (c_i, [c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_p]),
     "b200_corr3d_scratch_floats": (c_i64, [c_i, c_i, c_i, c_i, c_i, c_i]),
     "b200_corr3d_fwd": (c_i, [c_p, c_p, c_p, c_p, c_p, c_p, ctypes.POINTER(Corr3dWeights), c_p, c_p,
@@ -92,7 +103,7 @@ def _load():
 B200_ENOSUP = -3        # include/b200flow.h
 lib = _load()
 LAUNCHES = 0          # kernels of this library launched by this process (bench.py reports it as gpu_launches)
-KERNELS_PER_CALL = {"b200_knn_grid": 3, "b200_knn_grid_cf": 3, "b200_pointconv_fwd": 2, "b200_corr2d_bwd": 2, "b200_project_nn_corr": 2, "b200_corr3d_fwd": 5, "b200_corr3d_bwd": 10, "b200_event_voxel_trilinear": 3}
+KERNELS_PER_CALL = {"b200_knn_grid": 3, "b200_knn_grid_cf": 3, "b200_pointconv_fwd": 2, "b200_pointconv_fwd_linear": 2, "b200_pointconv_bwd": 6, "b200_corr2d_bwd": 2, "b200_project_nn_corr": 2, "b200_corr3d_fwd": 5, "b200_corr3d_bwd": 10, "b200_event_voxel_trilinear": 3}
 
 
 class B200Error(RuntimeError):

@@ -265,7 +265,7 @@ pointconv_tc_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
 // clouds of more than 65536 points and for A/B timing (B200_POINTCONV_V1=1)
 int pointconv_v2_run(const float* xyz, const float* feat, const float* sampled_xyz, const int64_t* knn,
                      const b200_pointconv_weights* w, float* out, float* scratch, int B, int C, int Cout, int N, int S,
-                     int precision, cudaStream_t st);
+                     int precision, int act, cudaStream_t st);
 int64_t pointconv_v2_scratch_floats(int B, int C, int Cout, int N);
 static bool pc_force_v1() {
     static const bool v = [] { const char* e = getenv("B200_POINTCONV_V1"); return e && e[0] == '1'; }();
@@ -283,6 +283,26 @@ extern "C" int64_t b200_pointconv_scratch_floats(int B, int C, int Cout, int N) 
     const int64_t v1 = (((int64_t)B * N * cp + 63) & ~int64_t(63)) + (int64_t)b200::pc_npad(Cout) * b200::PC_NW * cp;
     const int64_t v2 = b200::pointconv_v2_scratch_floats(B, C, Cout, N);
     return v1 > v2 ? v1 : v2;
+}
+
+extern "C" int b200_pointconv_fwd_linear(const float* xyz, const float* feat, const float* sampled_xyz, const int64_t* knn,
+                                         const b200_pointconv_weights* w, float* out, float* scratch, int B, int C, int Cout,
+                                         int N, int S, int k, int precision, b200_stream_t stream) {
+    using namespace b200;
+    B200_REQUIRE((B == 0 || S == 0) || (xyz && sampled_xyz && knn && w && out && scratch && (feat || C == 0)), "b200_pointconv_fwd_linear: null pointer");
+    B200_REQUIRE(w != nullptr || B == 0 || S == 0, "b200_pointconv_fwd_linear: null weight struct");
+    B200_REQUIRE(w == nullptr || (w->Wa && w->ba && w->Wb && w->bb && w->L && w->bias), "b200_pointconv_fwd_linear: null weight pointer");
+    B200_REQUIRE(B >= 0 && C >= 0 && Cout >= 1 && N >= 1 && S >= 0, "b200_pointconv_fwd_linear: bad sizes");
+    B200_REQUIRE(B <= 65535, "b200_pointconv_fwd_linear: B exceeds the grid limit");
+    B200_REQUIRE(precision >= 0 && precision <= 2, "b200_pointconv_fwd_linear: precision must be 0, 1 (TF32) or 2 (3xTF32), got %d", precision);
+    B200_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 15) == 0, "b200_pointconv_fwd_linear: scratch must be 16-byte aligned");
+    if (k != PC_K || Cout > 256 || N > 65536) {
+        set_error("b200_pointconv_fwd_linear: built for k = 16 neighbours, out_channels <= 256 and N <= 65536 (got k=%d, out=%d, N=%d)",
+                  k, Cout, N);
+        return B200_ENOSUP;
+    }
+    if (B == 0 || S == 0) return B200_OK;
+    return pointconv_v2_run(xyz, feat, sampled_xyz, knn, w, out, scratch, B, C, Cout, N, S, precision, 0, as_stream(stream));
 }
 
 extern "C" int b200_pointconv_fwd(const float* xyz, const float* feat, const float* sampled_xyz, const int64_t* knn,
@@ -303,7 +323,7 @@ extern "C" int b200_pointconv_fwd(const float* xyz, const float* feat, const flo
     if (B == 0 || S == 0) return B200_OK;
     cudaStream_t st = as_stream(stream);
     if (N <= 65536 && !pc_force_v1())
-        return pointconv_v2_run(xyz, feat, sampled_xyz, knn, w, out, scratch, B, C, Cout, N, S, precision, st);
+        return pointconv_v2_run(xyz, feat, sampled_xyz, knn, w, out, scratch, B, C, Cout, N, S, precision, 1, st);
     const int Cp = pc_cp(C), Npad = pc_npad(Cout);
     float* Fpm = scratch;
     float* Lp = scratch + (((int64_t)B * N * Cp + 63) & ~int64_t(63));

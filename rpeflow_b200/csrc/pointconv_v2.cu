@@ -29,37 +29,6 @@ constexpr int P2_SMEM_MAX = 232448;
 
 __device__ __forceinline__ float p2_lrelu(float v) { return v > 0.0f ? v : 0.1f * v; }
 
-// K-major operand, rows of 64 bytes, 64-byte swizzle (16-byte chunk index ^= address bits 7-8), 8-row groups 512 bytes apart
-__device__ __forceinline__ uint64_t umma_desc_sw64(uint32_t saddr) {
-    return (uint64_t)((saddr >> 4) & 0x3fffu) | ((uint64_t)(512u >> 4) << 32) | ((uint64_t)1 << 46) | ((uint64_t)4 << 61);
-}
-__device__ __forceinline__ uint32_t p2_sw64(uint32_t r, uint32_t q) { return r * 64u + ((q ^ ((r >> 1) & 3u)) << 4); }
-
-__device__ __forceinline__ void p2_mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ uint32_t p2_mbar_try(uint32_t bar, uint32_t parity) {
-    uint32_t done;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    return done;
-}
-// bounded wait: a protocol bug traps (launch error) instead of hanging the device; the fast path is one try_wait
-__device__ __noinline__ void p2_mbar_wait_slow(uint32_t bar, uint32_t parity) {
-    for (uint32_t spin = 0; !p2_mbar_try(bar, parity); ++spin)
-        if (spin > (1u << 26)) __trap();
-}
-__device__ __forceinline__ void p2_mbar_wait(uint32_t bar, uint32_t parity) {
-    if (!p2_mbar_try(bar, parity)) p2_mbar_wait_slow(bar, parity);
-}
-__device__ __forceinline__ void p2_tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]) : "r"(taddr));
-}
-
 // ---- pass 0 ---------------------------------------------------------------------------------------------------
 // grid (ceil(N/32), B): Fpm[b][n][0..Cp) = [xyz ; feat ; 0] point-major (Cp = roundup16(C+3)); on blockIdx.y == 0 also the
 // Linear weight as Limg[kb = cb*16 + w][hi|lo][o][c'] = L[o][w*(C+3) + cb*16 + c'] (zero beyond C+3 / out_channels),
@@ -87,7 +56,7 @@ pointconv_v2_prep_kernel(const float* __restrict__ xyz, const float* __restrict_
             if (n < N && c0 + tx < Cp) Fpm[((size_t)b * N + n) * Cp + c0 + tx] = tile[tx][ty * 4 + u];
         }
     }
-    if (b == 0) {
+    if (b == 0 && Limg != nullptr) {
         // K block kb = cb*16 + w: [hi | lo] tiles of Npad rows x 64 bytes, already in the swizzled operand layout
         const int total = P2_NW * Cp * Npad;                                  // (Cp/16 * 16 K blocks) * Npad * 16
         for (int e = blockIdx.x * 256 + threadIdx.x; e < total; e += gridDim.x * 256) {
@@ -143,7 +112,7 @@ pointconv_v2_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
                     const float* __restrict__ Fpm, const float* __restrict__ Limg, const float* __restrict__ Wa,
                     const float* __restrict__ ba, const float* __restrict__ Wb, const float* __restrict__ bb,
                     const float* __restrict__ bias, float* __restrict__ out, int Cp, int N, int S, int Cout, int Npad,
-                    uint32_t tmem_cols, int depth) {
+                    uint32_t tmem_cols, int depth, int act) {
     constexpr int SPLIT = MODE != 0;
     extern __shared__ uint8_t p2_smem_raw[];
     const uint32_t sbase = (tc_smem_u32(p2_smem_raw) + 1023u) & ~1023u;
@@ -342,7 +311,10 @@ pointconv_v2_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
                 const int o = c0 + c;
                 float v = __uint_as_float(r0[c]);
                 if (MODE == 1) v += __uint_as_float(r1[c]);
-                if (o < Cout && live) out[((size_t)b * Cout + o) * S + sp] = p2_lrelu(v + s_small[176 + o]);
+                if (o < Cout && live) {
+                    const float y = v + s_small[176 + o];
+                    out[((size_t)b * Cout + o) * S + sp] = act ? p2_lrelu(y) : y;      // act = 0: the Linear output (training)
+                }
             }
         }
     }
@@ -356,7 +328,8 @@ int p2_npad(int Cout) { return (Cout + 31) / 32 * 32; }
 
 template <int MODE>
 static int p2_launch(const float* xyz, const float* sampled, const int64_t* knn, const float* Fpm, const float* Limg,
-                     const b200_pointconv_weights* w, float* out, int B, int Cp, int N, int S, int Cout, int Npad, cudaStream_t st) {
+                     const b200_pointconv_weights* w, float* out, int B, int Cp, int N, int S, int Cout, int Npad, int act,
+                     cudaStream_t st) {
     const int split = MODE != 0;
     int depth = 4;
     while (depth > 1 && p2_layout(Npad, split, depth).total + 1024 > P2_SMEM_MAX) --depth;
@@ -371,7 +344,7 @@ static int p2_launch(const float* xyz, const float* sampled, const int64_t* knn,
     cudaError_t e = cudaFuncSetAttribute(pointconv_v2_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return cuda_fail(e, "pointconv_v2_kernel(attr)");
     pointconv_v2_kernel<MODE><<<dim3(ceil_div(S, P2_PTS), B), P2_THREADS, smem, st>>>(
-        xyz, sampled, knn, Fpm, Limg, w->Wa, w->ba, w->Wb, w->bb, w->bias, out, Cp, N, S, Cout, Npad, cols, depth);
+        xyz, sampled, knn, Fpm, Limg, w->Wa, w->ba, w->Wb, w->bb, w->bias, out, Cp, N, S, Cout, Npad, cols, depth, act);
     B200_LAUNCH_CHECK("pointconv_v2_kernel");
     return B200_OK;
 }
@@ -382,18 +355,26 @@ int64_t pointconv_v2_scratch_floats(int B, int C, int Cout, int N) {
     return (((int64_t)B * N * cp + 63) & ~int64_t(63)) + 2 * (int64_t)p2_npad(Cout) * P2_NW * cp;
 }
 
-// called by b200_pointconv_fwd (pointconv.cu) after its argument checks; scratch sized by b200_pointconv_scratch_floats
+// called by b200_pointconv_fwd / _fwd_linear (pointconv.cu) after their argument checks; scratch sized by
+// b200_pointconv_scratch_floats.  act = 1: LeakyReLU(0.1) epilogue; 0: the Linear output y.
 int pointconv_v2_run(const float* xyz, const float* feat, const float* sampled_xyz, const int64_t* knn,
                      const b200_pointconv_weights* w, float* out, float* scratch, int B, int C, int Cout, int N, int S,
-                     int precision, cudaStream_t st) {
+                     int precision, int act, cudaStream_t st) {
     const int Cp = p2_cp(C), Npad = p2_npad(Cout);
     float* Fpm = scratch;
     float* Limg = scratch + (((int64_t)B * N * Cp + 63) & ~int64_t(63));
     pointconv_v2_prep_kernel<<<dim3(ceil_div(N, 32), B), 256, 0, st>>>(xyz, feat, w->L, Fpm, Limg, C, Cp, N, Cout, Npad, precision != 1);
     B200_LAUNCH_CHECK("pointconv_v2_prep_kernel");
-    if (precision == 1) return p2_launch<0>(xyz, sampled_xyz, knn, Fpm, Limg, w, out, B, Cp, N, S, Cout, Npad, st);
-    return Npad <= 128 ? p2_launch<1>(xyz, sampled_xyz, knn, Fpm, Limg, w, out, B, Cp, N, S, Cout, Npad, st)
-                       : p2_launch<2>(xyz, sampled_xyz, knn, Fpm, Limg, w, out, B, Cp, N, S, Cout, Npad, st);
+    if (precision == 1) return p2_launch<0>(xyz, sampled_xyz, knn, Fpm, Limg, w, out, B, Cp, N, S, Cout, Npad, act, st);
+    return Npad <= 128 ? p2_launch<1>(xyz, sampled_xyz, knn, Fpm, Limg, w, out, B, Cp, N, S, Cout, Npad, act, st)
+                       : p2_launch<2>(xyz, sampled_xyz, knn, Fpm, Limg, w, out, B, Cp, N, S, Cout, Npad, act, st);
+}
+
+// the point-major rows alone (Fpm [B][N][p2_cp(C)] = [xyz ; feat ; 0]), for the backward (pointconv_bwd.cu)
+int pointconv_v2_rows(const float* xyz, const float* feat, float* Fpm, int B, int C, int N, cudaStream_t st) {
+    pointconv_v2_prep_kernel<<<dim3(ceil_div(N, 32), B), 256, 0, st>>>(xyz, feat, nullptr, Fpm, nullptr, C, p2_cp(C), N, 1, 32, 0);
+    B200_LAUNCH_CHECK("pointconv_v2_prep_kernel");
+    return B200_OK;
 }
 
 }  // namespace b200

@@ -1,4 +1,4 @@
-// umma_common.cuh — tcgen05 (5th-generation tensor core) PTX wrappers shared by corr3d_tc.cu and pointconv.cu:
+// umma_common.cuh — tcgen05 (5th-generation tensor core) PTX wrappers shared by corr3d_tc.cu and the PointConv kernels:
 // shared-memory matrix descriptors (K-major, 128-byte swizzle), the kind::tf32 instruction descriptor, MMA issue,
 // commit -> mbarrier, mbarrier wait, TMEM load.
 #pragma once
@@ -54,6 +54,38 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
           "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
         : "r"(taddr));
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+}
+
+// ---- SW64 operand layout, mbarrier ring and TMEM load of the second-generation PointConv (pointconv_v2.cu, pointconv_bwd.cu)
+// K-major operand, rows of 64 bytes, 64-byte swizzle (16-byte chunk index ^= address bits 7-8), 8-row groups 512 bytes apart
+__device__ __forceinline__ uint64_t umma_desc_sw64(uint32_t saddr) {
+    return (uint64_t)((saddr >> 4) & 0x3fffu) | ((uint64_t)(512u >> 4) << 32) | ((uint64_t)1 << 46) | ((uint64_t)4 << 61);
+}
+__device__ __forceinline__ uint32_t p2_sw64(uint32_t r, uint32_t q) { return r * 64u + ((q ^ ((r >> 1) & 3u)) << 4); }
+
+__device__ __forceinline__ void p2_mbar_arrive(uint32_t bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+}
+__device__ __forceinline__ uint32_t p2_mbar_try(uint32_t bar, uint32_t parity) {
+    uint32_t done;
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+        "selp.u32 %0, 1, 0, p;\n\t}"
+        : "=r"(done) : "r"(bar), "r"(parity) : "memory");
+    return done;
+}
+// bounded wait: a protocol bug traps (launch error) instead of hanging the device; the fast path is one try_wait
+static __device__ __noinline__ void p2_mbar_wait_slow(uint32_t bar, uint32_t parity) {
+    for (uint32_t spin = 0; !p2_mbar_try(bar, parity); ++spin)
+        if (spin > (1u << 26)) __trap();
+}
+__device__ __forceinline__ void p2_mbar_wait(uint32_t bar, uint32_t parity) {
+    if (!p2_mbar_try(bar, parity)) p2_mbar_wait_slow(bar, parity);
+}
+__device__ __forceinline__ void p2_tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]) : "r"(taddr));
 }
 
 __device__ __forceinline__ float tf32_hi(float v) { return __uint_as_float(__float_as_uint(v) & 0xffffe000u); }

@@ -23,9 +23,12 @@ Every re-bound callable decides PER CALL: the CUDA kernel runs only when all ten
 CUDA tensors, autograd does not need a graph through the op, and the arguments are inside what the kernel was
 built for; anything else goes to the reference's own function, untouched.  ``stats()`` counts both routes per op.
 
-``install(train=True)`` additionally sends ``Correlation3D.forward`` calls that DO need a graph to
-``pwc3d.Correlation3DFunction`` (forward b200_corr3d_fwd, backward b200_corr3d_bwd), under the same limits, unless
-``torch.use_deterministic_algorithms(True)`` is set (the backward sums with float atomics): those go to the reference.
+``install(train=...)`` additionally sends calls that DO need a graph to this library's forward and backward, unless
+``torch.use_deterministic_algorithms(True)`` is set (the backwards sum with float atomics): those go to the reference.
+``train`` is a collection of op names: "Correlation3D" (``pwc3d.Correlation3DFunction``, b200_corr3d_fwd /
+b200_corr3d_bwd) and "PointConv" (``PointConvDownSampling`` / ``PointConvNoSampling``: ``pointconv.PointConvFunction``,
+b200_pointconv_fwd_linear / b200_pointconv_bwd, followed by the module's own ``norm_fn`` and ``activation_fn``, so a
+training-mode BatchNorm1d or SyncBatchNorm runs as the reference runs it).  ``train=True`` means {"Correlation3D"}.
 """
 import importlib
 import sys
@@ -45,7 +48,8 @@ _SAVED = []            # (object, attribute, previous value) in the order they w
 _ADDED_MODULES = []    # sys.modules keys registered by install()
 _STATS = {}
 _OBSERVER = None
-_TRAIN = False         # install(train=True): Correlation3D calls that need a graph run Correlation3DFunction
+_TRAIN = frozenset()   # ops whose calls that need a graph run this library's autograd Functions (install(train=...))
+TRAINABLE = ("Correlation3D", "PointConv")
 
 
 def stats(reset=False):
@@ -141,7 +145,7 @@ def _corr3d_forward(self, xyz1, feat1, xyz2, feat2, knn_indices_1in1=None):
     import torch.nn as nn
     plain = all(isinstance(c.norm_fn, nn.Identity) for mlp in (self.cost_mlp, self.weight_net1, self.weight_net2) for c in mlp.convs)
     fits = _all_cuda_f32(xyz1, feat1, xyz2, feat2) and plain and self.k <= 32 and feat1.shape[1] <= 512
-    if fits and _TRAIN and _needs_graph(self, xyz1, feat1, xyz2, feat2) and not torch.are_deterministic_algorithms_enabled():
+    if fits and "Correlation3D" in _TRAIN and _needs_graph(self, xyz1, feat1, xyz2, feat2) and not torch.are_deterministic_algorithms_enabled():
         _count("Correlation3D.forward", "b200")
         knn12 = ops.k_nearest_neighbor(input_xyz=xyz2.detach(), query_xyz=xyz1.detach(), k=self.k)
         if knn_indices_1in1 is None:
@@ -161,6 +165,22 @@ def _corr3d_forward(self, xyz1, feat1, xyz2, feat2, knn_indices_1in1=None):
         _OBSERVER("k_nearest_neighbor", (xyz2, xyz1, self.k), {}, knn12)
         _OBSERVER("Correlation3D.forward", (xyz1, feat1, xyz2, feat2, knn_indices_1in1), {}, out)
     return out
+
+
+def _pointconv_body_ok(self):
+    """The PointConv body (gathers, weight net, matmul, Linear) is what the kernels were built for: k = 16, at most 256
+    output channels, a weight net without norm and with LeakyReLU(0.1)."""
+    import torch.nn as nn
+    if self.k != 16 or self.linear.out_features > 256:
+        return False
+    return all(isinstance(c.norm_fn, nn.Identity) and isinstance(c.relu_fn, nn.LeakyReLU)
+               and abs(c.relu_fn.negative_slope - 0.1) <= 1e-12 for c in self.weight_net.convs)
+
+
+def _pointconv_train(self, xyz, tensors):
+    """True when this call needs a graph and goes to pointconv.PointConvFunction (install(train={"PointConv", ...}))."""
+    return ("PointConv" in _TRAIN and _needs_graph(self, *tensors) and _all_cuda_f32(*tensors)
+            and xyz.shape[2] <= 65536 and not torch.are_deterministic_algorithms_enabled() and _pointconv_body_ok(self))
 
 
 def _pointconv_weights(self):
@@ -189,7 +209,20 @@ def _pointconv_weights(self):
     return None
 
 
+def _pointconv_apply(self, xyz, features, sampled_xyz, knn):
+    """The Linear output y of the module's PointConv body through pointconv.PointConvFunction (trains the parameters)."""
+    w = pointconv.param_weights(self)
+    params = [w[n].contiguous() for n in pointconv.PointConvWeights.NAMES]
+    return pointconv.PointConvFunction.apply(xyz.contiguous(), features.contiguous(), sampled_xyz.contiguous(),
+                                             knn.to(torch.int64).contiguous(), getattr(self, "b200_precision", 2), *params)
+
+
 def _pointconv_down_forward(self, xyz, features, sampled_xyz):
+    if _pointconv_train(self, xyz, (xyz, features, sampled_xyz)):
+        _count("PointConvDownSampling.forward", "b200")
+        knn = ops.k_nearest_neighbor(xyz.detach(), sampled_xyz.detach(), self.k)
+        y = _pointconv_apply(self, xyz, features, sampled_xyz, knn)
+        return self.activation_fn(self.norm_fn(y))
     w = None if (_needs_graph(self, xyz, features, sampled_xyz) or not _all_cuda_f32(xyz, features, sampled_xyz)) \
         else _pointconv_weights(self)
     if w is None:
@@ -205,6 +238,12 @@ def _pointconv_down_forward(self, xyz, features, sampled_xyz):
 
 
 def _pointconv_nosample_forward(self, xyz, features, knn_indices=None):
+    if _pointconv_train(self, xyz, (xyz, features)):
+        _count("PointConvNoSampling.forward", "b200")
+        knn = knn_indices[:, :, :self.k] if knn_indices is not None else \
+            ops.k_nearest_neighbor(xyz.detach(), xyz.detach(), self.k)
+        y = _pointconv_apply(self, xyz, features, xyz, knn)          # autograd adds the two xyz gradients
+        return self.activation_fn(self.norm_fn(y))
     w = None if (_needs_graph(self, xyz, features) or not _all_cuda_f32(xyz, features)) else _pointconv_weights(self)
     if w is None:
         _count("PointConvNoSampling.forward", "reference")
@@ -351,10 +390,21 @@ def patch_python_ops(patch_events=True, only=None):
 
 
 def install(patch_python=True, patch_events=False, only=None, extensions=True, train=False):
-    """train=True: Correlation3D.forward calls that need an autograd graph run this library's forward and backward
-    (pwc3d.Correlation3DFunction) instead of the reference's torch code; the default routes them to the reference."""
+    """train: the ops whose calls that need an autograd graph run this library's forward and backward instead of the
+    reference's torch code — a collection of names from TRAINABLE ("Correlation3D": pwc3d.Correlation3DFunction;
+    "PointConv": pointconv.PointConvFunction under the module's own norm and activation).  True means
+    {"Correlation3D"}; False (the default) routes every such call to the reference."""
     global _TRAIN
-    _TRAIN = bool(train)
+    if isinstance(train, bool):
+        names = {"Correlation3D"} if train else set()
+    elif isinstance(train, str):
+        names = {train}
+    else:
+        names = set(train)
+    unknown = names - set(TRAINABLE)
+    if unknown:
+        raise ValueError(f"install(train=...): unknown op(s) {sorted(unknown)}; choose from {TRAINABLE}")
+    _TRAIN = frozenset(names)
     if extensions:
         register_extension_shims()
     if patch_python:
@@ -364,7 +414,7 @@ def install(patch_python=True, patch_events=False, only=None, extensions=True, t
 def uninstall():
     """Undo install(): every replaced attribute and sys.modules entry gets its previous value back."""
     global _TRAIN
-    _TRAIN = False
+    _TRAIN = frozenset()
     while _SAVED:
         obj, name, old = _SAVED.pop()
         if obj is sys.modules:
