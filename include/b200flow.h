@@ -281,8 +281,10 @@ B200_API int b200_corr3d_fwd(const float* xyz1, const float* feat1, const float*
  *                 [out,in] / [out]).  NULL = not needed: its work is skipped and it is not written.  Every non-NULL
  *                 output is overwritten (the callee zero-fills what it accumulates).
  *   scratch     : >= b200_corr3d_bwd_scratch_floats(B,Cin,Cout,N1,N2,k) floats, 16-byte aligned.
- * Gradients of the clouds, the feature maps and W1's feature columns are summed with float atomics, so they are not
- * bit-reproducible from run to run; the other weight gradients are.  No host synchronisation, no allocation.
+ * Only the 3->8->8 part of weight_net1 (n1_Wa, n1_ba, n1_Wb, n1_bb) is bit-reproducible from run to run.  Every other
+ * gradient depends on float-atomic sums whose order varies: dP, dG2, the clouds, the split-K dW1 / db1, and the
+ * per-CTA shared-memory sums of the weight-net output layers, W1's xyz columns and b2.  No host synchronisation, no
+ * allocation.
  */
 typedef struct b200_corr3d_grads {
     float *xyz1, *feat1, *xyz2, *feat2;

@@ -116,3 +116,14 @@ def check(rc, what):
     LAUNCHES += KERNELS_PER_CALL.get(what, 1)
     if rc != 0:
         raise B200Error(f"{what} failed ({rc}): {lib.b200_last_error().decode()}")
+
+
+def require_dense(what, **tensors):
+    """Raise unless every tensor is a contiguous CUDA tensor of the dtype the kernels read (int64 for names starting
+    with "knn", fp32 otherwise): the entry points pass raw data pointers and would read any other layout wrongly."""
+    import torch
+    for name, t in tensors.items():
+        want = torch.int64 if name.startswith("knn") else torch.float32
+        if not (t.is_cuda and t.dtype == want and t.is_contiguous()):
+            raise ValueError(f"{what}: {name} must be a contiguous CUDA {want} tensor, got {t.dtype} on {t.device}"
+                             f"{'' if t.is_contiguous() else ', not contiguous'} (the functional form converts it)")

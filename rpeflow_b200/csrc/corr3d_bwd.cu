@@ -17,7 +17,9 @@
 // Passes 1 and 2 are persistent: each CTA walks tiles and keeps its weight gradients in shared memory / registers,
 // except dW2 (Cout^2 floats, larger than what is left of shared memory next to the two row tiles), which each CTA
 // accumulates in its own slice of the scratch (L2-resident read-modify-write, no atomics).  Every weight gradient is
-// then one deterministic sum over the CTAs' partials; only dP, dG2, dxyz and the split-K dW1a/dW1b use float atomics.
+// then one fixed-order sum over the CTAs' partials.  The partials themselves are not reproducible: dP, dG2, dxyz and the
+// split-K dW1a/dW1b/db1 use global float atomics, and the Wc/bc, W1c and b2 partials shared-memory float atomics; every
+// stage-1 gradient reads dP.  Only the weight_net1 3->8->8 gradients (thread-owned sums) are bit-reproducible.
 #include <algorithm>
 
 #include "corr3d_common.cuh"

@@ -20,7 +20,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 from torch.autograd.function import once_differentiable
 
-from ._lib import PointConvGrads, PointConvWeights, check, lib
+from ._lib import PointConvGrads, PointConvWeights, check, lib, require_dense
 from .ops import k_nearest_neighbor
 
 __all__ = ["PointConvDownSampling", "PointConvNoSampling", "PointConvFunction", "pointconv", "pointconv_forward",
@@ -105,7 +105,10 @@ class PointConvFunction(torch.autograd.Function):
         if torch.are_deterministic_algorithms_enabled():
             raise RuntimeError("rpeflow_b200.pointconv: the backward sums gradients with float atomics and is not "
                                "deterministic; torch.use_deterministic_algorithms(True) is set")
-        out = _pointconv_run(xyz, features, sampled_xyz, knn, dict(zip(PointConvWeights.NAMES, params)), precision,
+        # a non-contiguous or non-fp32 argument used to be read through its raw pointer: silently wrong y and gradients
+        require_dense("PointConvFunction", xyz=xyz, features=features, sampled_xyz=sampled_xyz, knn=knn,
+                      **dict(zip(PointConvWeights.NAMES, params)))
+        out =_pointconv_run(xyz, features, sampled_xyz, knn, dict(zip(PointConvWeights.NAMES, params)), precision,
                              "b200_pointconv_fwd_linear")
         ctx.save_for_backward(xyz, features, sampled_xyz, knn, *params)
         return out

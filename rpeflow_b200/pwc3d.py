@@ -16,7 +16,7 @@ import torch
 import torch.nn as nn
 from torch.autograd.function import once_differentiable
 
-from ._lib import Corr3dGrads, Corr3dWeights, check, lib
+from ._lib import Corr3dGrads, Corr3dWeights, check, lib, require_dense
 from .ops import k_nearest_neighbor
 
 __all__ = ["Correlation3D", "Correlation3DFunction", "correlation3d", "correlation3d_forward", "pack_weights",
@@ -116,7 +116,10 @@ class Correlation3DFunction(torch.autograd.Function):
         if torch.are_deterministic_algorithms_enabled():
             raise RuntimeError("rpeflow_b200.correlation3d: the backward sums gradients with float atomics and is not "
                                "deterministic; torch.use_deterministic_algorithms(True) is set")
-        out, scratch = _corr3d_run(xyz1, feat1, xyz2, feat2, dict(zip(Corr3dWeights.NAMES, params)), knn12, knn11,
+        # a non-contiguous or non-fp32 argument used to be read through its raw pointer: silently wrong out and gradients
+        require_dense("Correlation3DFunction", xyz1=xyz1, feat1=feat1, xyz2=xyz2, feat2=feat2, knn12=knn12, knn11=knn11,
+                      **dict(zip(Corr3dWeights.NAMES, params)))
+        out, scratch =_corr3d_run(xyz1, feat1, xyz2, feat2, dict(zip(Corr3dWeights.NAMES, params)), knn12, knn11,
                                    precision)
         ctx.save_for_backward(xyz1, feat1, xyz2, feat2, knn12, knn11, scratch, *params)
         return out
