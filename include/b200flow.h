@@ -86,6 +86,30 @@ B200_API int b200_backwarp2d(const float* x_nchw, const float* flow, float* out_
 B200_API int b200_convex_upsample(const float* flow, const float* mask, float* out,
                          int B, int H, int W, int scale, b200_stream_t stream);
 
+/* f3 / f4 backwards (decoder_bwd.cu).  Shared rules:
+ *   - inputs, sizes and limits exactly as given to the matching forward; grad_* has the forward output's shape;
+ *   - a gradient output passed as NULL is not computed and not written; every other one is overwritten (the entry
+ *     zero-fills what it accumulates, with cudaMemsetAsync on `stream`);
+ *   - empty calls accept NULL pointers; bad arguments return B200_EINVAL before anything touches a device;
+ *   - no host synchronisation and no allocation (the calls can be captured in a CUDA graph).
+ * Taps, weights and softmax are recomputed from the inputs with the forward's own fp32 operations.
+ *
+ * backwarp2d: dx [B,C,H,W] is scattered with float atomics (not bit-reproducible); dflow [B,2,H,W] is reduced over the
+ * channels in a fixed order.  The flow gradient follows ATen's grid_sampler_2d backward with border padding: it is 0
+ * where the un-clamped sample coordinate is <= 0 or >= size - 1 (a sample exactly on the border counts as clipped).
+ */
+B200_API int b200_backwarp2d_bwd(const float* x_nchw, const float* flow, const float* grad_out_nchw,
+                        float* dx_nchw, float* dflow, int B, int C, int H, int W, b200_stream_t stream);
+
+/* convex_upsample: dflow [B,2,H,W], dmask [B,9*s*s,H,W]; grad_out [B,2,s*H,s*W], 16-byte aligned.  Two passes, no
+ * atomics: both gradients are bit-reproducible.  scratch : >= b200_convex_upsample_bwd_scratch_floats(B,H,W,s) floats
+ * (per low-res pixel the 9 taps' partial flow gradients); needed only when dflow is not NULL.
+ */
+B200_API int64_t b200_convex_upsample_bwd_scratch_floats(int B, int H, int W, int scale);
+B200_API int b200_convex_upsample_bwd(const float* flow, const float* mask, const float* grad_out,
+                             float* dflow, float* dmask, float* scratch,
+                             int B, int H, int W, int scale, b200_stream_t stream);
+
 /* a2  backward of a1.
  * Replaces: correlation.cpp:24-35 (correlation_backward_cuda) + correlation_backward_kernel.cu:4-89;
  *           binding `_correlation_backward_cuda` (correlation.cpp:40), called from wrapper.py:31.
@@ -244,6 +268,18 @@ B200_API int b200_pointconv_bwd(const float* xyz, const float* feat, const float
 B200_API int b200_knn_interpolate(const float* input_xyz, const float* input_feat, const float* query_xyz,
                          const int64_t* knn_idx, float* out, int B, int C, int M, int Q, int k,
                          b200_stream_t stream);
+
+/* f2 backward (decoder_bwd.cu), under the rules of the f3 / f4 backwards above.  knn_idx gets the forward's treatment
+ * (negative indices wrap once, out-of-range ones are clamped), so every gradient lands where the forward read.
+ *   d_input_xyz [B,3,M] and d_input_feat [B,C,M] are scattered with float atomics (not bit-reproducible);
+ *   d_query_xyz [B,3,Q] is written once per query.  The distance clamp at 1e-8 passes no gradient (torch's clamp_min
+ *   backward), so a query that coincides with one of its neighbours gives that pair no xyz gradient.
+ * When only d_input_feat is requested the channel reduction the xyz gradients need is skipped.
+ */
+B200_API int b200_knn_interpolate_bwd(const float* input_xyz, const float* input_feat, const float* query_xyz,
+                             const int64_t* knn_idx, const float* grad_out,
+                             float* d_input_xyz, float* d_input_feat, float* d_query_xyz,
+                             int B, int C, int M, int Q, int k, b200_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------------
  * a5  3-D point cost volume (pwc3d_core.Correlation3D.forward), forward only.

@@ -5,6 +5,7 @@ Public surface (same names as the reference, danqu130/RPEFlow):
               correlation2d_leaky, warp_correlate                             (RPEFlow_core.py:351,362 fused)
   projection  batch_indexing_channel_{first,last}, grid_sample_wrapper, project_feat_with_nn_corr,
               knn_interpolation, backwarp_3d, backwarp_2d, convex_upsample    (models/utils.py)
+              KnnInterpolationFunction, Backwarp2dFunction, ConvexUpsampleFunction — their backwards
   pwc3d       Correlation3D, build_pc_pyramid                                 (models/pwc3d_core.py)
               correlation3d, Correlation3DFunction — the same op with a backward (b200_corr3d_bwd)
   pointconv   PointConvDownSampling, PointConvNoSampling                      (models/pointconv.py)
@@ -18,7 +19,8 @@ from . import _lib  # noqa: F401  (raises ImportError when the CUDA library is m
 from .ops import (correlation2d, correlation2d_leaky, warp_correlate, furthest_point_sampling,  # noqa: F401
                   k_nearest_neighbor, squared_distance, CorrelationFunction)
 from .projection import (batch_indexing_channel_first, batch_indexing_channel_last, grid_sample_wrapper,  # noqa: F401
-                         project_feat_with_nn_corr, knn_interpolation, backwarp_3d, backwarp_2d, convex_upsample)
+                         project_feat_with_nn_corr, knn_interpolation, backwarp_3d, backwarp_2d, convex_upsample,
+                         KnnInterpolationFunction, Backwarp2dFunction, ConvexUpsampleFunction)
 from .pwc3d import (Correlation3D, Correlation3DFunction, build_pc_pyramid, correlation3d,  # noqa: F401
                     correlation3d_forward)
 from .pointconv import PointConvDownSampling, PointConvNoSampling, pointconv_forward  # noqa: F401

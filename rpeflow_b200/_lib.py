@@ -50,6 +50,9 @@ SIGNATURES = {
     "b200_corr2d_fwd_nchw_leaky": (c_i, [c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, ctypes.c_float, c_p]),
     "b200_backwarp2d": (c_i, [c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_p]),
     "b200_convex_upsample": (c_i, [c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_p]),
+    "b200_backwarp2d_bwd": (c_i, [c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_p]),
+    "b200_convex_upsample_bwd_scratch_floats": (c_i64, [c_i, c_i, c_i, c_i]),
+    "b200_convex_upsample_bwd": (c_i, [c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_p]),
     "b200_corr2d_bwd": (c_i, [c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_p]),
     "b200_fps": (c_i, [c_p, c_p, c_i, c_i, c_i, c_p]),
     "b200_knn": (c_i, [c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_p]),
@@ -71,6 +74,7 @@ SIGNATURES = {
     "b200_pointconv_bwd": (c_i, [c_p, c_p, c_p, c_p, ctypes.POINTER(PointConvWeights), c_p, ctypes.POINTER(PointConvGrads),
                                  c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_p]),
     "b200_knn_interpolate": (c_i, [c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_p]),
+    "b200_knn_interpolate_bwd": (c_i, [c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_p]),
     "b200_corr3d_scratch_floats": (c_i64, [c_i, c_i, c_i, c_i, c_i, c_i]),
     "b200_corr3d_fwd": (c_i, [c_p, c_p, c_p, c_p, c_p, c_p, ctypes.POINTER(Corr3dWeights), c_p, c_p,
                               c_i, c_i, c_i, c_i, c_i, c_i, c_i, c_p]),
@@ -103,7 +107,8 @@ def _load():
 B200_ENOSUP = -3        # include/b200flow.h
 lib = _load()
 LAUNCHES = 0          # kernels of this library launched by this process (bench.py reports it as gpu_launches)
-KERNELS_PER_CALL = {"b200_knn_grid": 3, "b200_knn_grid_cf": 3, "b200_pointconv_fwd": 2, "b200_pointconv_fwd_linear": 2, "b200_pointconv_bwd": 6, "b200_corr2d_bwd": 2, "b200_project_nn_corr": 2, "b200_corr3d_fwd": 5, "b200_corr3d_bwd": 10, "b200_event_voxel_trilinear": 3}
+KERNELS_PER_CALL = {"b200_knn_grid": 3, "b200_knn_grid_cf": 3, "b200_pointconv_fwd": 2, "b200_pointconv_fwd_linear": 2, "b200_pointconv_bwd": 6, "b200_corr2d_bwd": 2, "b200_project_nn_corr": 2, "b200_corr3d_fwd": 5, "b200_corr3d_bwd": 10, "b200_event_voxel_trilinear": 3,
+                    "b200_knn_interpolate_bwd": 1, "b200_backwarp2d_bwd": 1, "b200_convex_upsample_bwd": 2}
 
 
 class B200Error(RuntimeError):

@@ -14,6 +14,7 @@
 #include <cstring>
 
 #include "common.cuh"
+#include "decoder_common.cuh"
 #include "project_common.cuh"
 
 namespace b200 {
@@ -68,16 +69,7 @@ gather_cl_kernel(const uint32_t* __restrict__ data, const int64_t* __restrict__ 
     }
 }
 
-// ---- bilinear taps, exactly the arithmetic of models/utils.py:290-291 followed by grid_sample(align_corners=True) ----
-struct Taps {
-    int o00, o01, o10, o11;      // offsets inside one H*W plane, -1 when the tap is outside the image (zero padding)
-    float w00, w01, w10, w11;
-};
-__device__ __forceinline__ float renorm_coord(float x, int size) {
-    const float sm1 = (float)(size - 1);
-    const float g = __fsub_rn(__fdiv_rn(__fmul_rn(2.0f, x), sm1), 1.0f);        // 2*x/(size-1) - 1
-    return __fmul_rn(__fdiv_rn(__fadd_rn(g, 1.0f), 2.0f), sm1);                  // ((g+1)/2)*(size-1)
-}
+// zero-padding taps (Taps, renorm_coord: decoder_common.cuh)
 __device__ __forceinline__ Taps make_taps(float x, float y, int H, int W) {
     const float ix = renorm_coord(x, W), iy = renorm_coord(y, H);
     const float fx = floorf(ix), fy = floorf(iy);
@@ -153,26 +145,7 @@ grid_sample_pts_kernel(const float* __restrict__ feat, const float* __restrict__
     }
 }
 
-// f3: backwarp_2d (models/utils.py:186-198) with padding_mode='border': out[b,c,p] = bilinear(x[b,c], pixel p + flow[b,:,p]).
-// The grid takes the reference's round trip (mesh + flow, 2*g/(W-1)-1, then grid_sample's ((g+1)/2)*(W-1)), is then
-// clamped to [0, size-1] (ATen clip_coordinates) and sampled like a7; a clamped x0 = W-1 leaves the right tap outside
-// the image with weight 0, exactly as ATen's within_bounds test does.
-__device__ __forceinline__ Taps make_taps_border(float gx, float gy, int H, int W) {
-    float ix = renorm_coord(gx, W), iy = renorm_coord(gy, H);
-    ix = fminf((float)(W - 1), fmaxf(ix, 0.0f));
-    iy = fminf((float)(H - 1), fmaxf(iy, 0.0f));
-    const float fx = floorf(ix), fy = floorf(iy);
-    const float wx1 = ix - fx, wy1 = iy - fy, wx0 = (fx + 1.0f) - ix, wy0 = (fy + 1.0f) - iy;
-    const int x0 = (int)fx, y0 = (int)fy, x1 = x0 + 1, y1 = y0 + 1;          // clamped: always finite and in range
-    const bool vx1 = x1 < W, vy1 = y1 < H;
-    Taps t;
-    t.o00 = y0 * W + x0;                 t.w00 = wx0 * wy0;
-    t.o01 = vx1 ? y0 * W + x1 : -1;      t.w01 = wx1 * wy0;
-    t.o10 = vy1 ? y1 * W + x0 : -1;      t.w10 = wx0 * wy1;
-    t.o11 = (vy1 && vx1) ? y1 * W + x1 : -1; t.w11 = wx1 * wy1;
-    return t;
-}
-
+// f3: backwarp_2d with padding_mode='border' (taps: make_taps_border in decoder_common.cuh).
 // grid: (ceil(HW/128), csplit, B); two lanes per pixel as in grid_sample_pts_kernel
 __global__ void __launch_bounds__(256)
 backwarp2d_border_kernel(const float* __restrict__ x, const float* __restrict__ flow, float* __restrict__ out,
@@ -379,8 +352,6 @@ project_nn_corr_kernel(const float* __restrict__ xy, const float* __restrict__ f
 // f2: knn_interpolation (models/utils.py:140-156): out[b,c,q] = sum_s wn_s * feat[b,c,idx[b,q,s]], wn = normalised inverse
 // distances (clamped at 1e-8).  Thread per query (weights computed once), channels split over blockIdx.y.  Every
 // operation is rounded separately in the reference's order, so the result equals the oracle bit for bit.
-constexpr int KI_KMAX = 8;
-
 __global__ void __launch_bounds__(256)
 knn_interpolate_kernel(const float* __restrict__ in_xyz, const float* __restrict__ feat, const float* __restrict__ q_xyz,
                        const int64_t* __restrict__ idx, float* __restrict__ out, int C, int M, int Q, int k) {
@@ -392,19 +363,13 @@ knn_interpolate_kernel(const float* __restrict__ in_xyz, const float* __restrict
     float wsum = 0.0f;
     const float qx = __ldg(q_xyz + ((size_t)b * 3 + 0) * Q + q), qy = __ldg(q_xyz + ((size_t)b * 3 + 1) * Q + q),
                 qz = __ldg(q_xyz + ((size_t)b * 3 + 2) * Q + q);
+    const float* xyz = in_xyz + (size_t)b * 3 * M;
 #pragma unroll
     for (int s = 0; s < KI_KMAX; ++s) {
         if (s < k) {
-            int64_t t = __ldg(idx + ((size_t)b * Q + q) * k + s);
-            if (t < 0) t += M;
-            t = t < 0 ? 0 : (t >= M ? M - 1 : t);
-            j[s] = (int)t;
-            const float dx = __fsub_rn(__ldg(in_xyz + ((size_t)b * 3 + 0) * M + t), qx);
-            const float dy = __fsub_rn(__ldg(in_xyz + ((size_t)b * 3 + 1) * M + t), qy);
-            const float dz = __fsub_rn(__ldg(in_xyz + ((size_t)b * 3 + 2) * M + t), qz);
-            float d = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz)));
-            d = d < 1e-8f ? 1e-8f : d;                   // .clamp(1e-8)
-            w[s] = __fdiv_rn(1.0f, d);
+            j[s] = knn_point(__ldg(idx + ((size_t)b * Q + q) * k + s), M);
+            float u[3], r;
+            w[s] = idw_weight(xyz, M, j[s], qx, qy, qz, u, r);
             wsum = __fadd_rn(wsum, w[s]);
         }
     }

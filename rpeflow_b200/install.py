@@ -24,11 +24,20 @@ CUDA tensors, autograd does not need a graph through the op, and the arguments a
 built for; anything else goes to the reference's own function, untouched.  ``stats()`` counts both routes per op.
 
 ``install(train=...)`` additionally sends calls that DO need a graph to this library's forward and backward, unless
-``torch.use_deterministic_algorithms(True)`` is set (the backwards sum with float atomics): those go to the reference.
-``train`` is a collection of op names: "Correlation3D" (``pwc3d.Correlation3DFunction``, b200_corr3d_fwd /
-b200_corr3d_bwd) and "PointConv" (``PointConvDownSampling`` / ``PointConvNoSampling``: ``pointconv.PointConvFunction``,
-b200_pointconv_fwd_linear / b200_pointconv_bwd, followed by the module's own ``norm_fn`` and ``activation_fn``, so a
-training-mode BatchNorm1d or SyncBatchNorm runs as the reference runs it).  ``train=True`` means {"Correlation3D"}.
+``torch.use_deterministic_algorithms(True)`` is set and the op's backward sums with float atomics: those go to the
+reference.  ``train`` is a collection of op names from ``TRAINABLE``:
+- "Correlation3D": ``pwc3d.Correlation3DFunction``, b200_corr3d_fwd / b200_corr3d_bwd;
+- "PointConv": ``PointConvDownSampling`` / ``PointConvNoSampling`` through ``pointconv.PointConvFunction``,
+  b200_pointconv_fwd_linear / b200_pointconv_bwd, followed by the module's own ``norm_fn`` and ``activation_fn``, so a
+  training-mode BatchNorm1d or SyncBatchNorm runs as the reference runs it;
+- "knn_interpolation" (it also governs ``backwarp_3d``): ``projection.KnnInterpolationFunction``,
+  b200_knn_interpolate / b200_knn_interpolate_bwd;
+- "backwarp_2d": ``projection.Backwarp2dFunction``, b200_backwarp2d / b200_backwarp2d_bwd;
+- "convex_upsample": ``projection.ConvexUpsampleFunction``, b200_convex_upsample / b200_convex_upsample_bwd.  Its
+  backward has no atomics, so this one also trains here under deterministic mode.
+A call takes the train route when it needs a graph, its op is in ``train``, every floating tensor is CUDA fp32 and its
+arguments are inside what the kernels were built for; ``stats()`` counts it as "b200".  ``train=True`` means
+{"Correlation3D"}.
 """
 import importlib
 import sys
@@ -49,7 +58,7 @@ _ADDED_MODULES = []    # sys.modules keys registered by install()
 _STATS = {}
 _OBSERVER = None
 _TRAIN = frozenset()   # ops whose calls that need a graph run this library's autograd Functions (install(train=...))
-TRAINABLE = ("Correlation3D", "PointConv")
+TRAINABLE = ("Correlation3D", "PointConv", "knn_interpolation", "backwarp_2d", "convex_upsample")
 
 
 def stats(reset=False):
@@ -81,9 +90,9 @@ def _tensors(args, kwargs):
             yield a
 
 
-def _kernel_ok(tensors, float_dtypes=(torch.float32,)):
-    """All CUDA, floating tensors fp32, and no autograd graph needed through the op."""
-    need_graph = torch.is_grad_enabled()
+def _kernel_ok(tensors, float_dtypes=(torch.float32,), graph_ok=False):
+    """All CUDA, floating tensors fp32, and (unless graph_ok) no autograd graph needed through the op."""
+    need_graph = torch.is_grad_enabled() and not graph_ok
     for t in tensors:
         if not t.is_cuda:
             return False
@@ -97,15 +106,25 @@ def _kernel_ok(tensors, float_dtypes=(torch.float32,)):
     return True
 
 
-def _dispatch(name, fast, slow, extra_ok=None):
-    """Per-call choice between this library's kernel (fast) and the reference's own function (slow)."""
+def _dispatch(name, fast, slow, extra_ok=None, train=None, atomics=True):
+    """Per-call choice between this library's kernel (fast) and the reference's own function (slow).  train: the
+    TRAINABLE name under which a call that needs a graph may still run fast (whose autograd Function then builds it);
+    atomics: that op's backward sums with float atomics, so deterministic mode sends such calls to the reference."""
     def op(*args, **kwargs):
-        if _kernel_ok(_tensors(args, kwargs)) and (extra_ok is None or extra_ok(*args, **kwargs)):
+        tensors = list(_tensors(args, kwargs))
+
+        def fits():
+            return extra_ok is None or extra_ok(*args, **kwargs)
+        if _kernel_ok(tensors) and fits():
             _count(name, "b200")
             out = fast(*args, **kwargs)
             if _OBSERVER is not None:
                 _OBSERVER(name, args, kwargs, out)
             return out
+        if (train in _TRAIN and _kernel_ok(tensors, graph_ok=True)
+                and not (atomics and torch.are_deterministic_algorithms_enabled()) and fits()):
+            _count(name, "b200")
+            return fast(*args, **kwargs)
         _count(name, "reference")
         return slow(*args, **kwargs)
     op.__name__ = getattr(slow, "__name__", name)
@@ -320,7 +339,7 @@ def patch_python_ops(patch_events=True, only=None):
 
     def knn_interpolation(input_xyz, input_features, query_xyz, k=3):
         """models/utils.py:140-156: the k-nearest search, then gathers + inverse-distance weights + weighted sum in one kernel."""
-        idx = ops.k_nearest_neighbor(input_xyz, query_xyz, k)
+        idx = ops.k_nearest_neighbor(input_xyz.detach(), query_xyz.detach(), k)
         if _OBSERVER is not None:
             _OBSERVER("k_nearest_neighbor", (input_xyz, query_xyz, k), {}, idx)
         return projection.knn_interpolation(input_xyz, input_features, query_xyz, k, knn_indices=idx)
@@ -347,12 +366,14 @@ def patch_python_ops(patch_events=True, only=None):
         "project_feat_with_nn_corr": _dispatch("project_feat_with_nn_corr", projection.project_feat_with_nn_corr,
                                                ref["project_feat_with_nn_corr"]),
         "knn_interpolation": _dispatch("knn_interpolation", knn_interpolation, ref["knn_interpolation"],
-                                       lambda input_xyz, input_features, query_xyz, k=3: k <= 8),
-        "backwarp_3d": _dispatch("backwarp_3d", backwarp_3d, ref["backwarp_3d"], lambda xyz1, xyz2, flow12, k=3: k <= 8),
+                                       lambda input_xyz, input_features, query_xyz, k=3: k <= 8, train="knn_interpolation"),
+        "backwarp_3d": _dispatch("backwarp_3d", backwarp_3d, ref["backwarp_3d"], lambda xyz1, xyz2, flow12, k=3: k <= 8,
+                                 train="knn_interpolation"),
         "backwarp_2d": _dispatch("backwarp_2d", projection.backwarp_2d, ref["backwarp_2d"],
-                                 lambda x, flow12, padding_mode: padding_mode == "border"),
+                                 lambda x, flow12, padding_mode: padding_mode == "border", train="backwarp_2d"),
         "convex_upsample": _dispatch("convex_upsample", projection.convex_upsample, ref["convex_upsample"],
-                                     lambda flow, mask, scale_factor=8: scale_factor in (2, 4, 8) and flow.shape[1] == 2),
+                                     lambda flow, mask, scale_factor=8: scale_factor in (2, 4, 8) and flow.shape[1] == 2,
+                                     train="convex_upsample", atomics=False),
     }
     for modname in _MODULES:
         try:
@@ -392,7 +413,8 @@ def patch_python_ops(patch_events=True, only=None):
 def install(patch_python=True, patch_events=False, only=None, extensions=True, train=False):
     """train: the ops whose calls that need an autograd graph run this library's forward and backward instead of the
     reference's torch code — a collection of names from TRAINABLE ("Correlation3D": pwc3d.Correlation3DFunction;
-    "PointConv": pointconv.PointConvFunction under the module's own norm and activation).  True means
+    "PointConv": pointconv.PointConvFunction under the module's own norm and activation; "knn_interpolation" (with
+    backwarp_3d), "backwarp_2d", "convex_upsample": the projection module's autograd Functions).  True means
     {"Correlation3D"}; False (the default) routes every such call to the reference."""
     global _TRAIN
     if isinstance(train, bool):

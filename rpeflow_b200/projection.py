@@ -2,20 +2,44 @@
 
 Same signatures and return shapes as ``batch_indexing_channel_first`` (:119-137), ``batch_indexing_channel_last``
 (:101-116), ``grid_sample_wrapper`` (:288-294) and ``project_feat_with_nn_corr`` (:297-317); each is one or two
-sm_100a kernels behind include/b200flow.h.  Forward only: the reference calls the last two under
+sm_100a kernels behind include/b200flow.h.  Those are forward only: the reference calls the last two under
 ``torch.no_grad()`` everywhere (RPEFlow_core.py:52,105,156; models/utils.py:297), and the gathers are used on
 index/geometry tensors.  When autograd needs a gradient through a gather, keep the torch version.
+
+The decoder ops ``knn_interpolation`` / ``backwarp_3d`` (:140-169), ``backwarp_2d`` (:186-198) and ``convex_upsample``
+(:201-214) also have backwards.  Under ``torch.no_grad()``, or when no input requires grad, they run their forward
+kernel alone; when autograd needs a graph they go through ``KnnInterpolationFunction``, ``Backwarp2dFunction`` and
+``ConvexUpsampleFunction`` (the same forward kernel, bit for bit, and b200_*_bwd).  The first two sum gradients with
+float atomics and raise under ``torch.use_deterministic_algorithms(True)``; convex_upsample's backward is
+bit-reproducible and runs there too.
 """
 import torch
+from torch.autograd.function import once_differentiable
 
-from ._lib import check, lib
+from ._lib import check, lib, require_dense
 
 __all__ = ["batch_indexing_channel_first", "batch_indexing_channel_last", "grid_sample_wrapper", "backwarp_2d", "convex_upsample",
-           "project_feat_with_nn_corr", "knn_interpolation", "backwarp_3d"]
+           "project_feat_with_nn_corr", "knn_interpolation", "backwarp_3d", "KnnInterpolationFunction",
+           "Backwarp2dFunction", "ConvexUpsampleFunction"]
 
 
 def _stream(t):
     return torch.cuda.current_stream(t.device).cuda_stream
+
+
+def _require_cuda(what, *tensors):
+    if not all(t.is_cuda for t in tensors):
+        raise RuntimeError(f"rpeflow_b200.{what}: CUDA tensors required — no CPU/torch fallback")
+
+
+def _needs_graph(*tensors):
+    return torch.is_grad_enabled() and any(t.requires_grad for t in tensors)
+
+
+def _refuse_nondeterministic(what):
+    if torch.are_deterministic_algorithms_enabled():
+        raise RuntimeError(f"rpeflow_b200.{what}: the backward sums gradients with float atomics and is not "
+                           "deterministic; torch.use_deterministic_algorithms(True) is set")
 
 
 def _prep_data(data, name):
@@ -151,18 +175,7 @@ def grid_sample_wrapper(feat_2d, xy):
     return out
 
 
-def backwarp_2d(x, flow12, padding_mode="border"):
-    """x [B,C,H,W], flow12 [B,2,H,W] -> x sampled at (pixel + flow), bilinear, align_corners=True (models/utils.py:186-198).
-    The model only ever passes padding_mode='border' (RPEFlow_core.py:351); other modes are not built."""
-    if not (x.is_cuda and flow12.is_cuda):
-        raise RuntimeError("rpeflow_b200.backwarp_2d: CUDA tensors required — no CPU/torch fallback")
-    if padding_mode != "border":
-        raise RuntimeError("rpeflow_b200.backwarp_2d: only padding_mode='border' is built (the mode RPEFlow uses)")
-    assert x.shape[-2:] == flow12.shape[-2:]                       # models/utils.py:193
-    if torch.is_grad_enabled() and (x.requires_grad or flow12.requires_grad):
-        raise RuntimeError("rpeflow_b200.backwarp_2d: forward only; run training through the reference's torch ops")
-    feat = x.contiguous().float()
-    flow = flow12.contiguous().float()
+def _backwarp2d_run(feat, flow):
     B, C, H, W = feat.shape
     out = torch.empty_like(feat)
     with torch.cuda.device(feat.device):
@@ -171,23 +184,111 @@ def backwarp_2d(x, flow12, padding_mode="border"):
     return out
 
 
-def convex_upsample(flow, mask, scale_factor=8):
-    """flow [B,2,H,W], mask [B,9*s*s,H,W] -> [B,2,s*H,s*W]: convex combination of the 3x3 neighbourhood with softmax
-    weights (models/utils.py:201-214).  Forward only (the model trains through the reference's torch ops)."""
-    if not (flow.is_cuda and mask.is_cuda):
-        raise RuntimeError("rpeflow_b200.convex_upsample: CUDA tensors required — no CPU/torch fallback")
-    if torch.is_grad_enabled() and (flow.requires_grad or mask.requires_grad):
-        raise RuntimeError("rpeflow_b200.convex_upsample: forward only; run training through the reference's torch ops")
-    s = int(scale_factor)
-    B, C, H, W = flow.shape
-    if C != 2 or s not in (2, 4, 8) or tuple(mask.shape) != (B, 9 * s * s, H, W):
-        raise RuntimeError("rpeflow_b200.convex_upsample: needs flow [B,2,H,W], mask [B,9*s*s,H,W], s in {2,4,8}")
-    f, m = flow.contiguous().float(), mask.contiguous().float()
+class Backwarp2dFunction(torch.autograd.Function):
+    """apply(x [B,C,H,W], flow [B,2,H,W]), contiguous CUDA fp32.  Forward is b200_backwarp2d (border padding), backward
+    b200_backwarp2d_bwd; gradients autograd does not ask for are not computed.  dx is summed with float atomics, so
+    this raises under torch.use_deterministic_algorithms(True)."""
+
+    @staticmethod
+    def forward(ctx, x, flow):
+        _require_cuda("Backwarp2dFunction", x, flow)
+        _refuse_nondeterministic("backwarp_2d")
+        require_dense("Backwarp2dFunction", x=x, flow=flow)
+        ctx.save_for_backward(x, flow)
+        return _backwarp2d_run(x, flow)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_out):
+        x, flow = ctx.saved_tensors
+        dx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
+        dflow = torch.empty_like(flow) if ctx.needs_input_grad[1] else None
+        if dx is None and dflow is None:
+            return None, None
+        B, C, H, W = x.shape
+        g = grad_out.contiguous().float()
+        with torch.cuda.device(x.device):
+            check(lib.b200_backwarp2d_bwd(x.data_ptr(), flow.data_ptr(), g.data_ptr(),
+                                          dx.data_ptr() if dx is not None else None,
+                                          dflow.data_ptr() if dflow is not None else None, B, C, H, W, _stream(x)),
+                  "b200_backwarp2d_bwd")
+        return dx, dflow
+
+
+def backwarp_2d(x, flow12, padding_mode="border"):
+    """x [B,C,H,W], flow12 [B,2,H,W] -> x sampled at (pixel + flow), bilinear, align_corners=True (models/utils.py:186-198).
+    The model only ever passes padding_mode='border' (RPEFlow_core.py:351); other modes are not built.  Differentiable
+    in x and flow12 (Backwarp2dFunction) when autograd needs a graph."""
+    _require_cuda("backwarp_2d", x, flow12)
+    if padding_mode != "border":
+        raise RuntimeError("rpeflow_b200.backwarp_2d: only padding_mode='border' is built (the mode RPEFlow uses)")
+    assert x.shape[-2:] == flow12.shape[-2:]                       # models/utils.py:193
+    feat = x.contiguous().float()
+    flow = flow12.contiguous().float()
+    if _needs_graph(feat, flow):
+        return Backwarp2dFunction.apply(feat, flow)
+    return _backwarp2d_run(feat, flow)
+
+
+def _convex_upsample_run(f, m, s):
+    B, _, H, W = f.shape
     out = torch.empty((B, 2, H * s, W * s), dtype=torch.float32, device=f.device)
     with torch.cuda.device(f.device):
         check(lib.b200_convex_upsample(f.data_ptr(), m.data_ptr(), out.data_ptr(), B, H, W, s, _stream(f)),
               "b200_convex_upsample")
     return out
+
+
+class ConvexUpsampleFunction(torch.autograd.Function):
+    """apply(flow [B,2,H,W], mask [B,9*s*s,H,W], s), contiguous CUDA fp32.  Forward is b200_convex_upsample, backward
+    b200_convex_upsample_bwd: two fixed-order passes without atomics, so the gradients are bit-reproducible and the
+    op runs under torch.use_deterministic_algorithms(True)."""
+
+    @staticmethod
+    def forward(ctx, flow, mask, s):
+        _require_cuda("ConvexUpsampleFunction", flow, mask)
+        require_dense("ConvexUpsampleFunction", flow=flow, mask=mask)
+        ctx.save_for_backward(flow, mask)
+        ctx.s = s
+        return _convex_upsample_run(flow, mask, s)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_out):
+        flow, mask = ctx.saved_tensors
+        s = ctx.s
+        dflow = torch.empty_like(flow) if ctx.needs_input_grad[0] else None
+        dmask = torch.empty_like(mask) if ctx.needs_input_grad[1] else None
+        if dflow is None and dmask is None:
+            return None, None, None
+        B, _, H, W = flow.shape
+        g = grad_out.contiguous().float()
+        if g.data_ptr() % 16:                                        # the kernel reads grad_out with 16-byte loads
+            g = g.clone()
+        scratch = torch.empty((max(1, lib.b200_convex_upsample_bwd_scratch_floats(B, H, W, s)),), dtype=torch.float32,
+                              device=flow.device) if dflow is not None else None
+        with torch.cuda.device(flow.device):
+            check(lib.b200_convex_upsample_bwd(flow.data_ptr(), mask.data_ptr(), g.data_ptr(),
+                                               dflow.data_ptr() if dflow is not None else None,
+                                               dmask.data_ptr() if dmask is not None else None,
+                                               scratch.data_ptr() if scratch is not None else None, B, H, W, s,
+                                               _stream(flow)), "b200_convex_upsample_bwd")
+        return dflow, dmask, None
+
+
+def convex_upsample(flow, mask, scale_factor=8):
+    """flow [B,2,H,W], mask [B,9*s*s,H,W] -> [B,2,s*H,s*W]: convex combination of the 3x3 neighbourhood with softmax
+    weights (models/utils.py:201-214).  Differentiable in flow and mask (ConvexUpsampleFunction) when autograd needs a
+    graph."""
+    _require_cuda("convex_upsample", flow, mask)
+    s = int(scale_factor)
+    B, C, H, W = flow.shape
+    if C != 2 or s not in (2, 4, 8) or tuple(mask.shape) != (B, 9 * s * s, H, W):
+        raise RuntimeError("rpeflow_b200.convex_upsample: needs flow [B,2,H,W], mask [B,9*s*s,H,W], s in {2,4,8}")
+    f, m = flow.contiguous().float(), mask.contiguous().float()
+    if _needs_graph(f, m):
+        return ConvexUpsampleFunction.apply(f, m, s)
+    return _convex_upsample_run(f, m, s)
 
 
 @torch.no_grad()
@@ -223,26 +324,70 @@ def project_feat_with_nn_corr(xy, feat_2d, feat_3d, nn_indices=None, keep_sample
     return out
 
 
+def _knn_interpolate_run(xin, feat, xq, idx):
+    B, C, M = feat.shape
+    Q, k = xq.shape[2], idx.shape[2]
+    out = torch.empty((B, C, Q), dtype=torch.float32, device=xin.device)
+    with torch.cuda.device(xin.device):
+        check(lib.b200_knn_interpolate(xin.data_ptr(), feat.data_ptr(), xq.data_ptr(), idx.data_ptr(), out.data_ptr(),
+                                       B, C, M, Q, k, _stream(xin)), "b200_knn_interpolate")
+    return out
+
+
+class KnnInterpolationFunction(torch.autograd.Function):
+    """apply(input_xyz [B,3,M], input_feat [B,C,M], query_xyz [B,3,Q], knn_idx [B,Q,k] int64), contiguous CUDA fp32.
+    Forward is b200_knn_interpolate, backward b200_knn_interpolate_bwd (gradients of all three point tensors; those
+    autograd does not ask for are not computed).  The input gradients are summed with float atomics, so this raises
+    under torch.use_deterministic_algorithms(True)."""
+
+    @staticmethod
+    def forward(ctx, input_xyz, input_feat, query_xyz, knn_idx):
+        _require_cuda("KnnInterpolationFunction", input_xyz, input_feat, query_xyz, knn_idx)
+        _refuse_nondeterministic("knn_interpolation")
+        require_dense("KnnInterpolationFunction", input_xyz=input_xyz, input_feat=input_feat, query_xyz=query_xyz,
+                      knn_idx=knn_idx)
+        ctx.save_for_backward(input_xyz, input_feat, query_xyz, knn_idx)
+        return _knn_interpolate_run(input_xyz, input_feat, query_xyz, knn_idx)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_out):
+        xin, feat, xq, idx = ctx.saved_tensors
+        need = ctx.needs_input_grad
+        grads = [torch.empty_like(t) if need[n] else None for n, t in enumerate((xin, feat, xq))]
+        if all(g is None for g in grads):
+            return None, None, None, None
+        B, C, M = feat.shape
+        Q, k = xq.shape[2], idx.shape[2]
+        g = grad_out.contiguous().float()
+        ptr = [t.data_ptr() if t is not None else None for t in grads]
+        with torch.cuda.device(xin.device):
+            check(lib.b200_knn_interpolate_bwd(xin.data_ptr(), feat.data_ptr(), xq.data_ptr(), idx.data_ptr(),
+                                               g.data_ptr(), *ptr, B, C, M, Q, k, _stream(xin)),
+                  "b200_knn_interpolate_bwd")
+        return (*grads, None)
+
+
 def knn_interpolation(input_xyz, input_features, query_xyz, k=3, knn_indices=None):
     """input_xyz [B,3,M], input_features [B,C,M], query_xyz [B,3,Q] -> [B,C,Q] (models/utils.py:140-156): the k-nearest
-    search (cell-grid KNN) followed by ONE kernel for gathers + inverse-distance weights + weighted sum.  Forward only."""
-    if not (input_xyz.is_cuda and input_features.is_cuda and query_xyz.is_cuda):
-        raise RuntimeError("rpeflow_b200.knn_interpolation: CUDA tensors required — no CPU/torch fallback")
+    search (cell-grid KNN) followed by ONE kernel for gathers + inverse-distance weights + weighted sum.
+    Differentiable in all three point tensors (KnnInterpolationFunction) when autograd needs a graph; the neighbour
+    search itself carries no gradient, as in the reference."""
+    _require_cuda("knn_interpolation", input_xyz, input_features, query_xyz)
     from .ops import k_nearest_neighbor
     xin, feat, xq = (t.contiguous().float() for t in (input_xyz, input_features, query_xyz))
     if knn_indices is None:
-        knn_indices = k_nearest_neighbor(xin, xq, k)                          # [B,Q,k]
+        knn_indices = k_nearest_neighbor(xin.detach(), xq.detach(), k)        # [B,Q,k]
     idx = _prep_idx(knn_indices, xin.device)
     B, C, M = feat.shape
     Q = xq.shape[2]
     assert tuple(idx.shape) == (B, Q, k) and xin.shape == (B, 3, M)
-    out = torch.empty((B, C, Q), dtype=torch.float32, device=xin.device)
-    with torch.cuda.device(xin.device):
-        check(lib.b200_knn_interpolate(xin.data_ptr(), feat.data_ptr(), xq.data_ptr(), idx.data_ptr(), out.data_ptr(),
-                                       B, C, M, Q, int(k), _stream(xin)), "b200_knn_interpolate")
-    return out
+    if _needs_graph(xin, feat, xq):
+        return KnnInterpolationFunction.apply(xin, feat, xq, idx)
+    return _knn_interpolate_run(xin, feat, xq, idx)
 
 
 def backwarp_3d(xyz1, xyz2, flow12, k=3):
-    """models/utils.py:159-169: xyz2 + interpolation of -flow12 from the warped cloud xyz1 + flow12."""
+    """models/utils.py:159-169: xyz2 + interpolation of -flow12 from the warped cloud xyz1 + flow12.  Differentiable in
+    all three (autograd composes KnnInterpolationFunction with the add and the negation)."""
     return xyz2 + knn_interpolation(xyz1 + flow12, -flow12, xyz2, k)
