@@ -54,17 +54,6 @@ __device__ __forceinline__ float sqdist2_rule(float ax, float ay, float bx, floa
     return __fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy));
 }
 
-// Packed fp32x2 FMA (Blackwell FFMA2): d = a*b + d on both halves.
-__device__ __forceinline__ void ffma2(float2& d, const float2& a, const float2& b) {
-    unsigned long long dd, aa, bb;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(dd) : "f"(d.x), "f"(d.y));
-    asm("mov.b64 %0, {%1, %2};" : "=l"(aa) : "f"(a.x), "f"(a.y));
-    asm("mov.b64 %0, {%1, %2};" : "=l"(bb) : "f"(b.x), "f"(b.y));
-    asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(dd) : "l"(aa), "l"(bb));
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(d.x), "=f"(d.y) : "l"(dd));
-}
-
-
 // ---- packed fp32x2 arithmetic (Blackwell FADD2 / FFMA2): two independent fp32 lanes per instruction ----
 typedef unsigned long long u64;
 __device__ __forceinline__ u64 pack2(float lo, float hi) {
@@ -74,6 +63,15 @@ __device__ __forceinline__ u64 pack2(float lo, float hi) {
 }
 __device__ __forceinline__ void unpack2(u64 v, float& lo, float& hi) {
     asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
+}
+// d = a*b + d on both halves (FFMA2)
+__device__ __forceinline__ void fma2(u64& d, u64 a, u64 b) {
+    asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(d) : "l"(a), "l"(b));
+}
+__device__ __forceinline__ void ffma2(float2& d, const float2& a, const float2& b) {
+    u64 dd = pack2(d.x, d.y);
+    fma2(dd, pack2(a.x, a.y), pack2(b.x, b.y));
+    unpack2(dd, d.x, d.y);
 }
 __device__ __forceinline__ u64 sub2(u64 a, u64 b) {
     u64 r;
@@ -102,10 +100,40 @@ __device__ __forceinline__ u64 sqdist_pair(u64 ax, u64 ay, u64 az, u64 bx, u64 b
     return s;
 }
 
+// ---- shared-memory accesses by 32-bit shared address (ptxas folds "+ constant" into the LDS / STS immediate) ----
+__device__ __forceinline__ float lds_f32(uint32_t addr) {
+    float v;
+    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(addr));
+    return v;
+}
+__device__ __forceinline__ float2 lds_v2(uint32_t addr) {
+    float2 v;
+    asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(addr));
+    return v;
+}
+__device__ __forceinline__ u64 lds_b64(uint32_t addr) {      // two fp32 as one packed FFMA2 operand
+    u64 v;
+    asm volatile("ld.shared.b64 %0, [%1];" : "=l"(v) : "r"(addr));
+    return v;
+}
+__device__ __forceinline__ float4 lds_v4(uint32_t addr) {
+    float4 v;
+    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
+    return v;
+}
+__device__ __forceinline__ void sts_v4(uint32_t addr, float a, float b, float c, float d) {
+    asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
+}
+
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src, bool valid) {
     unsigned dst = (unsigned)__cvta_generic_to_shared(smem_dst);
     int bytes = valid ? 16 : 0;   // src-size 0 -> the 16 destination bytes are zero-filled
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(gmem_src), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void cp_async4(void* smem_dst, const void* gmem_src, bool valid) {
+    unsigned dst = (unsigned)__cvta_generic_to_shared(smem_dst);
+    int bytes = valid ? 4 : 0;    // src-size 0 -> the destination word is zero-filled
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(dst), "l"(gmem_src), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N>

@@ -23,12 +23,6 @@
 
 namespace b200 {
 
-__device__ __forceinline__ void cp_async4(void* smem_dst, const void* gmem_src, bool valid) {
-    unsigned dst = (unsigned)__cvta_generic_to_shared(smem_dst);
-    int bytes = valid ? 4 : 0;    // src-size 0 -> the destination word is zero-filled
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4, %2;" ::"r"(dst), "l"(gmem_src), "r"(bytes) : "memory");
-}
-
 constexpr int BT_TH = 8, BT_TW = 32, BT_P = 8, BT_CC = 32, BT_CB = 8, BT_MD = 4, BT_ND = 9;
 constexpr int BT_HR = BT_TH + 2 * BT_MD, BT_HC = BT_TW + 2 * BT_MD;          // 16 x 40 halo
 constexpr int BT_THREADS = 128;

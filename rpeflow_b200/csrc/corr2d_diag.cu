@@ -20,7 +20,7 @@
 //     the strip's parity so both are naturally aligned; the 8 strips of a row fill 192 contiguous bytes.
 #include <stdlib.h>
 
-#include "tma_common.cuh"
+#include "sm100_async.cuh"
 
 namespace b200 {
 
@@ -44,12 +44,6 @@ struct DAcc {                                    // the 9 column shifts of one p
     float s;
 };
 
-__device__ __forceinline__ float2 lds_64(uint32_t addr) {
-    float2 v;
-    asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(addr));
-    return v;
-}
-
 // One stage (8 channels) for one consumer thread.  pa: shared address of the thread's first in1 pixel (row 0 of its
 // rows) in channel 0 of the stage, pb: of its first in2 pixel.  ROWS = 2: the diagonal pair, ROWS = 1: a diagonal end.
 template <int ROWS>
@@ -61,12 +55,12 @@ __device__ __forceinline__ void corr2d_diag_consume(DAcc (&acc)[ROWS][D_P], uint
         for (int r = 0; r < ROWS; ++r)
 #pragma unroll
             for (int m = 0; m < D_P / 2; ++m) {
-                const float2 v = lds_64(pa + (D_B_BYTES + c * D_A_CH + r * D_PITCH * 4 + m * 8));
+                const float2 v = lds_v2(pa + (D_B_BYTES + c * D_A_CH + r * D_PITCH * 4 + m * 8));
                 a[r][2 * m] = v.x; a[r][2 * m + 1] = v.y;
             }
 #pragma unroll
         for (int m = 0; m < (D_P + 2 * D_MD) / 2; ++m) {
-            const float2 v = lds_64(pb + (c * D_B_CH + m * 8));
+            const float2 v = lds_v2(pb + (c * D_B_CH + m * 8));
             b[2 * m] = v.x; b[2 * m + 1] = v.y;
         }
 #pragma unroll
@@ -181,7 +175,7 @@ corr2d_fwd_diag_kernel(const __grid_constant__ CUtensorMap map1, const __grid_co
             mbar_init(bar_full + 8 * s, 1);
             mbar_init(bar_empty + 8 * s, D_CONSUMERS);
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     __syncthreads();
 
@@ -190,8 +184,8 @@ corr2d_fwd_diag_kernel(const __grid_constant__ CUtensorMap map1, const __grid_co
 
     if (warp == D_CONSUMERS) {                                    // ---------------- producer
         if (lane == 0) {
-            asm volatile("prefetch.tensormap [%0];" ::"l"(&map1) : "memory");
-            asm volatile("prefetch.tensormap [%0];" ::"l"(&map2) : "memory");
+            prefetch_tensormap(&map1);
+            prefetch_tensormap(&map2);
             int s = 0;
             uint32_t ph = 0;
             for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
@@ -199,7 +193,7 @@ corr2d_fwd_diag_kernel(const __grid_constant__ CUtensorMap map1, const __grid_co
                 const int ty = r / tiles_x, tx = r - ty * tiles_x;
                 const int y0 = ty * D_TH, x0 = tx * D_TW;
                 for (int ch = 0; ch < nchunks; ++ch) {
-                    while (!mbar_test(bar_empty + 8 * s, ph ^ 1u)) __nanosleep(64);    // consumers have drained this slot
+                    while (!mbar_try(bar_empty + 8 * s, ph ^ 1u)) __nanosleep(64);    // consumers have drained this slot
                     mbar_arrive_expect_tx(bar_full + 8 * s, D_STAGE);
                     // boxes are (x, y, channel, batch); out-of-image pixels and channels >= C arrive as zeros
                     tma_load_4d(base + s * D_STAGE, &map2, x0 - D_MD, y0 - D_MD, ch * D_CC, b, bar_full + 8 * s);

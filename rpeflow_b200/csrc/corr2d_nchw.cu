@@ -18,7 +18,7 @@
 //     profiles/microbench), so the kernel is bound by issue slots on the busiest scheduler (3 of the 9 consumer
 //     warps share one); the short strip keeps registers at ~120 so the loop body carries no spill or fix-up moves.
 //   * epilogue: a thread's 8 pixels are 2 aligned float4 per displacement: plain 16-byte streaming stores.
-#include "tma_common.cuh"
+#include "sm100_async.cuh"
 
 namespace b200 {
 
@@ -50,12 +50,6 @@ struct NAcc {                                    // the 9 column shifts of one p
     float s;
 };
 
-__device__ __forceinline__ float4 lds_128(uint32_t addr) {
-    float4 v;
-    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
-    return v;
-}
-
 // One stage (16 channels) for one consumer thread.  pa / pb: shared addresses of the thread's first in1 / in2 pixel
 // in channel 0 of stage 0; SOFF: byte offset of the stage (compile time -> LDS immediates).
 template <int SOFF>
@@ -67,12 +61,12 @@ __device__ __forceinline__ void corr2d_nchw_consume(NAcc (&acc)[N_P], uint32_t p
         float a[N_P], b[N_P + 2 * N_MD];
 #pragma unroll
         for (int m = 0; m < N_P / 4; ++m) {
-            const float4 v = lds_128(pa + (SOFF + N_B_BYTES + m * 16));
+            const float4 v = lds_v4(pa + (SOFF + N_B_BYTES + m * 16));
             a[4 * m] = v.x; a[4 * m + 1] = v.y; a[4 * m + 2] = v.z; a[4 * m + 3] = v.w;
         }
 #pragma unroll
         for (int m = 0; m < (N_P + 2 * N_MD) / 4; ++m) {
-            const float4 v = lds_128(pb + (SOFF + m * 16));
+            const float4 v = lds_v4(pb + (SOFF + m * 16));
             b[4 * m] = v.x; b[4 * m + 1] = v.y; b[4 * m + 2] = v.z; b[4 * m + 3] = v.w;
         }
 #pragma unroll
@@ -104,7 +98,7 @@ corr2d_fwd_nchw_kernel(const __grid_constant__ CUtensorMap map1, const __grid_co
             mbar_init(bar_full + 8 * s, 1);
             mbar_init(bar_empty + 8 * s, N_CONSUMERS);
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     __syncthreads();
 
@@ -113,8 +107,8 @@ corr2d_fwd_nchw_kernel(const __grid_constant__ CUtensorMap map1, const __grid_co
 
     if (warp == N_CONSUMERS) {                                    // ---------------- producer
         if (lane == 0) {
-            asm volatile("prefetch.tensormap [%0];" ::"l"(&map1) : "memory");
-            asm volatile("prefetch.tensormap [%0];" ::"l"(&map2) : "memory");
+            prefetch_tensormap(&map1);
+            prefetch_tensormap(&map2);
             int s = 0;
             uint32_t ph = 0;
             for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
@@ -122,7 +116,7 @@ corr2d_fwd_nchw_kernel(const __grid_constant__ CUtensorMap map1, const __grid_co
                 const int ty = r / tiles_x, tx = r - ty * tiles_x;
                 const int y0 = ty * N_TH, x0 = tx * N_TW;
                 for (int ch = 0; ch < nchunks; ++ch) {
-                    while (!mbar_test(bar_empty + 8 * s, ph ^ 1u)) __nanosleep(128);   // consumers have drained this slot
+                    while (!mbar_try(bar_empty + 8 * s, ph ^ 1u)) __nanosleep(128);   // consumers have drained this slot
                     mbar_arrive_expect_tx(bar_full + 8 * s, N_STAGE);
                     // boxes are (x, y, channel, batch); out-of-image pixels and channels >= C arrive as zeros
                     tma_load_4d(base + s * N_STAGE, &map2, x0 - N_MD, y0 - N_MD, ch * N_CC, b, bar_full + 8 * s);
@@ -181,10 +175,10 @@ corr2d_fwd_nchw_kernel(const __grid_constant__ CUtensorMap map1, const __grid_co
                     cb[(i * N_ND + 8) * 32] = acc[i].s;
                     acc[i].s = 0.0f;
                 }
-                asm volatile("bar.sync 1, 64;" ::: "memory");
+                named_bar_sync<1, 64>();
                 continue;                                         // warp 8 stores the plane
             }
-            asm volatile("bar.sync 1, 64;" ::: "memory");
+            named_bar_sync<1, 64>();
 #pragma unroll
             for (int i = 0; i < N_P; ++i) {
 #pragma unroll

@@ -23,7 +23,7 @@
 //     7-pixel strip would exceed).
 //   * epilogue: pair-sum, scale by 1/C; neighbouring strips trade two values by shuffle so that every store is an
 //     aligned 16-byte st.global.cs (scalar stores when W % 4 != 0).
-#include "tma_common.cuh"
+#include "sm100_async.cuh"
 
 namespace b200 {
 
@@ -41,12 +41,6 @@ constexpr int T_CONSUMERS = T_ND;              // warps
 constexpr int T_THREADS = (T_CONSUMERS + 1) * 32;
 constexpr size_t T_SMEM = (size_t)T_NSTAGE * T_STAGE + 1024 + 64;
 
-__device__ __forceinline__ u64 lds_64(uint32_t addr) {      // ptxas folds "+ constant" into the LDS immediate
-    u64 v;
-    asm volatile("ld.shared.b64 %0, [%1];" : "=l"(v) : "r"(addr));
-    return v;
-}
-
 // One stage (32 channels) of one tile for one consumer thread, two channels (one FFMA2 operand pair) per step.
 // SOFF = byte offset of the stage (compile time: rides in the LDS immediates).  pa0 / pb0 = shared address of the
 // thread's first in1 / in2 line with the thread's swizzle phase folded in; XOR with step<<3 selects the channel
@@ -58,10 +52,10 @@ __device__ __forceinline__ void corr2d_consume(u64 (&acc)[T_P][T_ND], uint32_t p
         const uint32_t aq = pa0 ^ (uint32_t)(step << 3), bq = pb0 ^ (uint32_t)(step << 3);
         u64 a[T_P];
 #pragma unroll
-        for (int i = 0; i < T_P; ++i) a[i] = lds_64(aq + (SOFF + T_B_BYTES + i * T_TH * 128));
+        for (int i = 0; i < T_P; ++i) a[i] = lds_b64(aq + (SOFF + T_B_BYTES + i * T_TH * 128));
 #pragma unroll
         for (int j = 0; j < T_P + 2 * T_MD; ++j) {
-            const u64 v = lds_64(bq + (SOFF + j * T_HR * 128));
+            const u64 v = lds_b64(bq + (SOFF + j * T_HR * 128));
 #pragma unroll
             for (int i = 0; i < T_P; ++i) {
                 const int d = j - i;                     // column shift index, dx = d - 4
@@ -87,7 +81,7 @@ corr2d_fwd_tma_kernel(const __grid_constant__ CUtensorMap map1, const __grid_con
             mbar_init(bar_full + 8 * s, 1);
             mbar_init(bar_empty + 8 * s, T_CONSUMERS);
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     __syncthreads();
 
@@ -96,8 +90,8 @@ corr2d_fwd_tma_kernel(const __grid_constant__ CUtensorMap map1, const __grid_con
 
     if (warp == T_CONSUMERS) {                                    // ---------------- producer
         if (lane == 0) {
-            asm volatile("prefetch.tensormap [%0];" ::"l"(&map1) : "memory");
-            asm volatile("prefetch.tensormap [%0];" ::"l"(&map2) : "memory");
+            prefetch_tensormap(&map1);
+            prefetch_tensormap(&map2);
             int it = 0;
             for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
                 const int b = tile / per_img, r = tile - b * per_img;
@@ -106,7 +100,7 @@ corr2d_fwd_tma_kernel(const __grid_constant__ CUtensorMap map1, const __grid_con
                 for (int ch = 0; ch < nchunks; ++ch, ++it) {
                     const int s = it & 1;
                     const uint32_t ph = (uint32_t)(it >> 1) & 1u;
-                    while (!mbar_test(bar_empty + 8 * s, ph ^ 1u)) __nanosleep(128);   // consumers have drained this slot
+                    while (!mbar_try(bar_empty + 8 * s, ph ^ 1u)) __nanosleep(128);   // consumers have drained this slot
                     mbar_arrive_expect_tx(bar_full + 8 * s, T_STAGE);
                     tma_load_4d(base + s * T_STAGE, &map2, ch * T_CC, y0 - T_MD, x0 - T_MD, b, bar_full + 8 * s);
                     tma_load_4d(base + s * T_STAGE + T_B_BYTES, &map1, ch * T_CC, y0, x0, b, bar_full + 8 * s);

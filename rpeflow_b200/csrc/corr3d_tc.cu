@@ -19,7 +19,7 @@
 //             summed by recursive halving (30 shuffles per 32 columns), lane m ends with columns 2m, 2m+1 -> one
 //             coalesced 128-byte store of P per point and column chunk.
 #include "corr3d_common.cuh"
-#include "umma_common.cuh"
+#include "sm100_async.cuh"
 
 namespace b200 {
 
@@ -57,8 +57,8 @@ corr3d_stage1_tc_kernel(const float* __restrict__ xyz1, const float* __restrict_
                         const float* __restrict__ WcT, const float* __restrict__ bc, float* __restrict__ P,
                         int Cout, int N1, int N2, uint32_t tmem_cols, int tiles_per_cta) {
     extern __shared__ uint8_t tc_smem_raw[];
-    const uint32_t sbase = (tc_smem_u32(tc_smem_raw) + 1023u) & ~1023u;
-    uint8_t* gbase = tc_smem_raw + (sbase - tc_smem_u32(tc_smem_raw));
+    const uint32_t sbase = (smem_u32(tc_smem_raw) + 1023u) & ~1023u;
+    uint8_t* gbase = tc_smem_raw + (sbase - smem_u32(tc_smem_raw));
     const TcSmem L = tc_layout(Cout, SPLIT);
     float* s_epi = reinterpret_cast<float*>(gbase + L.epi);
     float* s_w1c = reinterpret_cast<float*>(gbase + L.w1c);
@@ -72,13 +72,12 @@ corr3d_stage1_tc_kernel(const float* __restrict__ xyz1, const float* __restrict_
     const int b = blockIdx.y;
 
     if (tid == 0) {
-        tc_mbar_init(bar_free, 1);
-        tc_mbar_init(bar_done, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init(bar_free, 1);
+        mbar_init(bar_done, 1);
+        mbar_init_fence();
     }
     if (warp == 0) {                                   // tensor-memory columns for the 128 x Cout fp32 accumulator
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc(tmem_slot, tmem_cols);
     }
 
     // per-CTA constants: epilogue table, W1c; then the tensor-memory base address
@@ -90,9 +89,9 @@ corr3d_stage1_tc_kernel(const float* __restrict__ xyz1, const float* __restrict_
     }
     for (int e = tid; e < 3 * Cout; e += TC_THREADS) s_w1c[e] = __ldg(W1cT + e);
     weight_net_stage(s_wn, Wa, ba, Wb, bb, tid, TC_THREADS);
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tcgen05_fence_after();
     const uint32_t tmem = *tmem_slot_ptr;
 
     const int nkb = Cout / TC_KB;
@@ -124,7 +123,7 @@ corr3d_stage1_tc_kernel(const float* __restrict__ xyz1, const float* __restrict_
     // ---- K loop: produce a stage, one thread issues its MMAs
     for (int kb = 0; kb < nkb; ++kb, ++it) {
         constexpr int st = 0;
-        if (it >= 1) tc_mbar_wait(bar_free, (it - 1) & 1u);               // the MMAs that read the stage are done
+        if (it >= 1) mbar_wait(bar_free, (it - 1) & 1u);               // the MMAs that read the stage are done
         const uint32_t stage = sbase;
         const int c0 = kb * TC_KB + 4 * q;
         const float4 wx = *reinterpret_cast<const float4*>(s_w1c + c0);
@@ -166,10 +165,10 @@ corr3d_stage1_tc_kernel(const float* __restrict__ xyz1, const float* __restrict_
                 *reinterpret_cast<float4*>(gbase + st * L.stage_bytes + L.w_hi + off) = v;
             }
         }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> visible to the MMA's async proxy
+        fence_proxy_async();   // generic-proxy writes -> visible to the MMA's async proxy
         __syncthreads();
         if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tcgen05_fence_after();
 #pragma unroll
             for (int ks = 0; ks < TC_KB / 8; ++ks) {   // one MMA consumes K = 8 tf32 = 32 bytes of every row
                 const uint64_t ah = umma_desc_sw128(stage + L.a_hi + ks * 32), wh = umma_desc_sw128(stage + L.w_hi + ks * 32);
@@ -184,8 +183,8 @@ corr3d_stage1_tc_kernel(const float* __restrict__ xyz1, const float* __restrict_
             if (kb == nkb - 1) umma_commit(bar_done);
         }
     }
-    tc_mbar_wait(bar_done, (uint32_t)(tt & 1));        // accumulator complete (one commit per tile)
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    mbar_wait(bar_done, (uint32_t)(tt & 1));        // accumulator complete (one commit per tile)
+    tcgen05_fence_after();
 
     // ---- epilogue: thread = row (TMEM lane), 32 columns at a time
     const int m = lane & 15;                           // position in the 16-row group of one point
@@ -193,7 +192,8 @@ corr3d_stage1_tc_kernel(const float* __restrict__ xyz1, const float* __restrict_
     float* prow = P + ((size_t)b * N1 + min(pt, N1 - 1)) * Cout;
     for (int cb = 0; cb < Cout; cb += 32) {
         uint32_t raw[32];
-        tmem_ld32(tmem + ((uint32_t)(warp * 32) << 16) + (uint32_t)cb, raw);
+        tmem_ld(tmem + ((uint32_t)(warp * 32) << 16) + (uint32_t)cb, raw);
+        tmem_ld_wait();
         float v[32];
 #pragma unroll
         for (int c = 0; c < 32; ++c) {
@@ -222,12 +222,12 @@ corr3d_stage1_tc_kernel(const float* __restrict__ xyz1, const float* __restrict_
         if (pt < N1) *reinterpret_cast<float2*>(prow + cb + 2 * m) = make_float2(v[0], v[1]);
     }
     // every warp has read its accumulator rows before the next tile's first MMA overwrites them (and before s_j / s_d change)
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tcgen05_fence_after();
     }   // tiles of this CTA
 
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(tmem_cols) : "memory");
+    if (warp == 0) tmem_dealloc(tmem, tmem_cols);
 }
 
 bool corr3d_stage1_tc_eligible(int Cout, int k, int precision) {

@@ -25,7 +25,7 @@
 #include <stdlib.h>
 
 #include "corr3d_common.cuh"
-#include "umma_common.cuh"
+#include "sm100_async.cuh"
 
 #ifdef V2_TRACE
 // debug builds only (profiles/build_variant.sh trace "-DV2_TRACE"): clock64 stamps of CTA 0's first worker thread per tile
@@ -51,43 +51,6 @@ constexpr int V2_ROWS = 128, V2_KB = 32, V2_K = 16;
 #define V2_PREJ 0
 #endif
 constexpr int V2_TILE = V2_ROWS * 128;                  // one 128-row operand tile: 16 KB
-
-// ---- mbarrier / bulk-copy helpers --------------------------------------------------------------------------------
-__device__ __forceinline__ void v2_mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void v2_mbar_arrive_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-// bounded wait: a protocol bug traps (launch error) instead of hanging the device
-__device__ __forceinline__ void v2_mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t done = 0;
-    for (uint32_t spin = 0; !done; ++spin) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-        if (spin > (1u << 26)) __trap();
-    }
-}
-__device__ __forceinline__ void v2_bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-template <int NWT>
-__device__ __forceinline__ void v2_worker_sync() { asm volatile("bar.sync 1, %0;" ::"n"(NWT) : "memory"); }
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-          "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// byte offset of 16-byte chunk q of row r inside a K-major tile with rows of 128 bytes and the 128-byte swizzle
-__host__ __device__ __forceinline__ uint32_t sw128(uint32_t r, uint32_t q) { return r * 128u + ((q ^ (r & 7u)) << 4); }
 
 // ---- weight images (once per call) ---------------------------------------------------------------------------------
 // W2img  [nkb][hi|lo][C rows x 128 B]  : W2[o][kb*32 .. +32) split into TF32 hi/lo, in the swizzled layout of the B tile
@@ -213,8 +176,8 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
                         float* __restrict__ P, int C, int N1, int N2, int B, uint32_t tmem_cols, int nbuf) {
     constexpr int NWT = NW * 32;                            // worker threads
     extern __shared__ uint8_t v2_smem_raw[];
-    const uint32_t sbase = (tc_smem_u32(v2_smem_raw) + 1023u) & ~1023u;
-    uint8_t* gbase = v2_smem_raw + (sbase - tc_smem_u32(v2_smem_raw));
+    const uint32_t sbase = (smem_u32(v2_smem_raw) + 1023u) & ~1023u;
+    uint8_t* gbase = v2_smem_raw + (sbase - smem_u32(v2_smem_raw));
     const V2Smem L = v2_layout(C, true, false, DEPTH);
     float* s_w1c = reinterpret_cast<float*>(gbase + L.w1c);
     float* s_wn = reinterpret_cast<float*>(gbase + L.wn);
@@ -239,17 +202,16 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
 
     if (tid == 0) {
         for (int s = 0; s < 2; ++s) {
-            tc_mbar_init(bar_full(s), NWT);
-            tc_mbar_init(bar_empty(s), 1);
-            tc_mbar_init(bar_accf(s), 1);
-            tc_mbar_init(bar_acce(s), NWT);
+            mbar_init(bar_full(s), NWT);
+            mbar_init(bar_empty(s), 1);
+            mbar_init(bar_accf(s), 1);
+            mbar_init(bar_acce(s), NWT);
         }
-        tc_mbar_init(bar_wres, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init(bar_wres, 1);
+        mbar_init_fence();
     }
     if (warp == NW) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc(tmem_slot, tmem_cols);
     }
     if (tid < NWT) {
         for (int e = tid; e < 3 * C; e += NWT) s_w1c[e] = __ldg(W1cT + e);
@@ -261,11 +223,11 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
         }
         for (int e = tid; e < C * 8; e += NWT)              // Wc / bias image: already in tile layout
             reinterpret_cast<float4*>(gbase + L.wc)[e] = __ldg(reinterpret_cast<const float4*>(wcimg) + e);
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        fence_proxy_async();
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tcgen05_fence_after();
     const uint32_t tmem = *tmem_slot_ptr;
     const uint32_t idesc = umma_idesc_tf32(V2_ROWS, C);
 
@@ -273,9 +235,9 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
         // =============================== MMA warp ===============================
         if (lane == 0) {
             if (resident) {
-                v2_mbar_arrive_tx(bar_wres, (uint32_t)L.wbytes);
-                v2_bulk_g2s(sbase + L.wres, W2img, (uint32_t)L.wbytes, bar_wres);
-                v2_mbar_wait(bar_wres, 0);
+                mbar_arrive_expect_tx(bar_wres, (uint32_t)L.wbytes);
+                bulk_g2s(sbase + L.wres, W2img, (uint32_t)L.wbytes, bar_wres);
+                mbar_wait(bar_wres, 0);
             }
             uint32_t it = 0, lt = 0;                        // ring items / tiles handled by this CTA so far
             for (uint32_t item = blockIdx.x; item < items; item += gridDim.x, ++lt) {
@@ -284,12 +246,12 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
                 const uint32_t wc = sbase + L.wc, hid = sbase + HID_OFF(lt % DEPTH);
                 for (int kb = 0; kb < nkb; ++kb, ++it) {
                     const uint32_t s = it % DEPTH, ph = it / DEPTH;
-                    v2_mbar_wait(bar_full(s), ph & 1u);
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    mbar_wait(bar_full(s), ph & 1u);
+                    tcgen05_fence_after();
                     if (kb == 0) {
                         if (use >= 1) {                     // the epilogue that last read this accumulator pair is done
-                            v2_mbar_wait(bar_acce(buf), (use - 1) & 1u);
-                            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                            mbar_wait(bar_acce(buf), (use - 1) & 1u);
+                            tcgen05_fence_after();
                         }
                         // weights: D_w = hid_hi.Wc_hi + hid_hi.Wc_lo + hid_lo.Wc_hi + 1.(bc_hi, bc_lo)
                         umma_tf32(accw, umma_desc_sw128(hid), umma_desc_sw128(wc), idesc, 0u);
@@ -373,14 +335,14 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
                 if (NW == 8) {                              // two threads per row: `half` selects four of the eight outputs
                     float hd[4];
                     v2_hidden_half(s_wn, dx, dy, dz, half, hd);
-                    v2_worker_sync<NWT>();                  // every produce() read of the previous tile's s_j / s_d is done
+                    named_bar_sync<1, NWT>();                  // every produce() read of the previous tile's s_j / s_d is done
                     const float4 hi = make_float4(tf32_hi(hd[0]), tf32_hi(hd[1]), tf32_hi(hd[2]), tf32_hi(hd[3]));
                     *reinterpret_cast<float4*>(hid + sw128(row, half)) = hi;
                     *reinterpret_cast<float4*>(hid + sw128(row, 2 + half)) = make_float4(hd[0] - hi.x, hd[1] - hi.y, hd[2] - hi.z, hd[3] - hi.w);
                 } else {
                     float hd[8];
                     v2_hidden_full(s_wn, dx, dy, dz, hd);
-                    v2_worker_sync<NWT>();
+                    named_bar_sync<1, NWT>();
 #pragma unroll
                     for (int u = 0; u < 2; ++u) {
                         const float4 hi = make_float4(tf32_hi(hd[4 * u]), tf32_hi(hd[4 * u + 1]), tf32_hi(hd[4 * u + 2]), tf32_hi(hd[4 * u + 3]));
@@ -392,7 +354,7 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
                 // (the HID tile of this buffer is free: the MMAs of the tile that used it last were waited for by an
                 // epilogue that precedes this call in every worker's program order)
                 if (half == 0) { s_j[row] = (int)j; s_d[row] = make_float4(dx, dy, dz, 0.0f); }
-                v2_worker_sync<NWT>();
+                named_bar_sync<1, NWT>();
             }
             V2_STAMP(2);
             // ---- K blocks: this thread handles chunk q = tid & 7 of rows (step * NWT + tid) >> 3
@@ -423,12 +385,12 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
                             gn[step] = __ldg(reinterpret_cast<const float4*>(g_base + g_off[step] + (kb + 1) * V2_KB));
                         }
                     }
-                    if (ph >= 1) v2_mbar_wait(bar_empty(s), (ph - 1) & 1u);
+                    if (ph >= 1) mbar_wait(bar_empty(s), (ph - 1) & 1u);
                     uint8_t* a_hi = gbase + A_OFF(s);
                     uint8_t* a_lo = a_hi + V2_TILE;
                     if (!resident && tid == 0) {
-                        v2_mbar_arrive_tx(bar_full(s), (uint32_t)L.wbytes);
-                        v2_bulk_g2s(sbase + W_OFF(s), W2img + (size_t)kb * 2 * C * 32, (uint32_t)L.wbytes, bar_full(s));
+                        mbar_arrive_expect_tx(bar_full(s), (uint32_t)L.wbytes);
+                        bulk_g2s(sbase + W_OFF(s), W2img + (size_t)kb * 2 * C * 32, (uint32_t)L.wbytes, bar_full(s));
                     }
                     const int c0 = kb * V2_KB + 4 * q;
                     const float4 wx = *reinterpret_cast<const float4*>(s_w1c + c0);
@@ -436,8 +398,8 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
                     const float4 wz = *reinterpret_cast<const float4*>(s_w1c + 2 * C + c0);
 #pragma unroll
                     for (int step = 0; step < STEPS; ++step) convert(a[step], g[step], (step * NWT + tid) >> 3, q, wx, wy, wz, a_hi, a_lo);
-                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                    if (!(!resident && tid == 0)) v2_mbar_arrive(bar_full(s));   // thread 0's arrival was the expect_tx one
+                    fence_proxy_async();
+                    if (!(!resident && tid == 0)) mbar_arrive(bar_full(s));   // thread 0's arrival was the expect_tx one
                     if (kb + 1 < nkb) {
 #pragma unroll
                         for (int step = 0; step < STEPS; ++step) { a[step] = an[step]; g[step] = gn[step]; }
@@ -446,12 +408,12 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
             } else {
                 for (int kb = 0; kb < nkb; ++kb, ++it) {
                     const uint32_t s = it % DEPTH, ph = it / DEPTH;
-                    if (ph >= 1) v2_mbar_wait(bar_empty(s), (ph - 1) & 1u);
+                    if (ph >= 1) mbar_wait(bar_empty(s), (ph - 1) & 1u);
                     uint8_t* a_hi = gbase + A_OFF(s);
                     uint8_t* a_lo = a_hi + V2_TILE;
                     if (!resident && tid == 0) {
-                        v2_mbar_arrive_tx(bar_full(s), (uint32_t)L.wbytes);
-                        v2_bulk_g2s(sbase + W_OFF(s), W2img + (size_t)kb * 2 * C * 32, (uint32_t)L.wbytes, bar_full(s));
+                        mbar_arrive_expect_tx(bar_full(s), (uint32_t)L.wbytes);
+                        bulk_g2s(sbase + W_OFF(s), W2img + (size_t)kb * 2 * C * 32, (uint32_t)L.wbytes, bar_full(s));
                     }
                     const int c0 = kb * V2_KB + 4 * q;
                     const float4 wx = *reinterpret_cast<const float4*>(s_w1c + c0);
@@ -469,8 +431,8 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
 #pragma unroll
                         for (int u = 0; u < GROUP; ++u) convert(a[u], g[u], ((s0 + u) * NWT + tid) >> 3, q, wx, wy, wz, a_hi, a_lo);
                     }
-                    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                    if (!(!resident && tid == 0)) v2_mbar_arrive(bar_full(s));
+                    fence_proxy_async();
+                    if (!(!resident && tid == 0)) mbar_arrive(bar_full(s));
                 }
             }
             V2_STAMP(3);
@@ -481,16 +443,16 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
             const int i0 = (int)(item - b * tiles) * 8;
             const uint32_t buf = nbuf == 2 ? (lt & 1u) : 0u, use = nbuf == 2 ? (lt >> 1) : lt;
             V2_STAMP(4);
-            v2_mbar_wait(bar_accf(buf), use & 1u);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            mbar_wait(bar_accf(buf), use & 1u);
+            tcgen05_fence_after();
             V2_STAMP(5);
             const uint32_t acc = tmem + buf * 2u * (uint32_t)C + ((uint32_t)(lq * 32) << 16);
             const int pt = i0 + lq * 2 + (lane >> 4);
             float* prow = P + ((size_t)b * N1 + min(pt, N1 - 1)) * C;
             for (int cb = ch * 16; cb < C; cb += 16 * (NW / 4)) {   // the warps of a lane quarter take alternate 16-column chunks
                 uint32_t rm[16], rw[16];
-                tmem_ld16(acc + (uint32_t)cb, rm);
-                tmem_ld16(acc + (uint32_t)(C + cb), rw);
+                tmem_ld(acc + (uint32_t)cb, rm);
+                tmem_ld(acc + (uint32_t)(C + cb), rw);
                 tmem_ld_wait();
                 float v[16];
 #pragma unroll
@@ -498,8 +460,8 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
                 const float tot = v2_reduce16(v, m);
                 if (pt < N1) prow[cb + m] = tot;
             }
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            v2_mbar_arrive(bar_acce(buf));
+            tcgen05_fence_before();
+            mbar_arrive(bar_acce(buf));
             V2_STAMP(6);
         };
 
@@ -521,10 +483,10 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
             ++lt;
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    if (warp == NW) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(tmem_cols) : "memory");
+    tcgen05_fence_after();
+    if (warp == NW) tmem_dealloc(tmem, tmem_cols);
 }
 
 // =====================================================================================================================
@@ -540,8 +502,8 @@ corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restric
                         uint32_t tmem_cols) {
     constexpr int NWT = NW * 32;
     extern __shared__ uint8_t v2_smem_raw[];
-    const uint32_t sbase = (tc_smem_u32(v2_smem_raw) + 1023u) & ~1023u;
-    uint8_t* gbase = v2_smem_raw + (sbase - tc_smem_u32(v2_smem_raw));
+    const uint32_t sbase = (smem_u32(v2_smem_raw) + 1023u) & ~1023u;
+    uint8_t* gbase = v2_smem_raw + (sbase - smem_u32(v2_smem_raw));
     const V2Smem L = v2_layout(C, false, true, DEPTH);
     float* s_wn = reinterpret_cast<float*>(gbase + L.wn);
     int* s_j = reinterpret_cast<int*>(gbase + L.meta_j);    // [2][256]: slot = (tile parity, thread) — private to a thread
@@ -556,15 +518,14 @@ corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restric
 
     if (tid == 0) {
         for (int s = 0; s < 2; ++s) {
-            tc_mbar_init(bar_full(s), NWT);
-            tc_mbar_init(bar_accf(s), 1);
-            tc_mbar_init(bar_acce(s), NWT);
+            mbar_init(bar_full(s), NWT);
+            mbar_init(bar_accf(s), 1);
+            mbar_init(bar_acce(s), NWT);
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     if (warp == NW) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc(tmem_slot, tmem_cols);
     }
     if (tid < NWT) {
         weight_net_stage(s_wn, Wa, ba, Wb, bb, tid, NWT);
@@ -574,11 +535,11 @@ corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restric
         }
         for (int e = tid; e < C * 8; e += NWT)
             reinterpret_cast<float4*>(gbase + L.wc)[e] = __ldg(reinterpret_cast<const float4*>(wcimg) + e);
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        fence_proxy_async();
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tcgen05_fence_after();
     const uint32_t tmem = *tmem_slot_ptr;
     const uint32_t idesc = umma_idesc_tf32(V2_ROWS, C);
 
@@ -589,11 +550,11 @@ corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restric
             for (uint32_t item = blockIdx.x; item < items; item += gridDim.x) {
                 for (int t4 = 0; t4 < 4; ++t4, ++lt) {
                     const uint32_t buf = lt % DEPTH, use = lt / DEPTH;
-                    v2_mbar_wait(bar_full(buf), use & 1u);
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    mbar_wait(bar_full(buf), use & 1u);
+                    tcgen05_fence_after();
                     if (use >= 1) {
-                        v2_mbar_wait(bar_acce(buf), (use - 1) & 1u);
-                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                        mbar_wait(bar_acce(buf), (use - 1) & 1u);
+                        tcgen05_fence_after();
                     }
                     const uint32_t accw = tmem + buf * (uint32_t)C, wc = sbase + L.wc, hid = sbase + HID_OFF(buf);
                     umma_tf32(accw, umma_desc_sw128(hid), umma_desc_sw128(wc), idesc, 0u);
@@ -655,8 +616,8 @@ corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restric
                         make_float4(hd[4 * u] - hi.x, hd[4 * u + 1] - hi.y, hd[4 * u + 2] - hi.z, hd[4 * u + 3] - hi.w);
                 }
             }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            v2_mbar_arrive(bar_full(buf));
+            fence_proxy_async();
+            mbar_arrive(bar_full(buf));
             return (int)j;
         };
         constexpr int CSTEP = 16 * (NW / 4);                // the warps of a lane quarter take alternate 16-column chunks
@@ -666,13 +627,13 @@ corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restric
         };
         auto epilogue = [&](uint32_t g, const float* prow, float4 (&p4)[4]) {
             const uint32_t buf = g % DEPTH, use = g / DEPTH;
-            v2_mbar_wait(bar_accf(buf), use & 1u);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            mbar_wait(bar_accf(buf), use & 1u);
+            tcgen05_fence_after();
             const uint32_t accw = tmem + buf * (uint32_t)C + ((uint32_t)(lq * 32) << 16);
             const int ptl = (int)(g & 3u) * 8 + lq * 2 + (lane >> 4);   // point index inside the 32-point item
             for (int cb = ch * 16; cb < C; cb += CSTEP) {
                 uint32_t rw[16];
-                tmem_ld16(accw + (uint32_t)cb, rw);
+                tmem_ld(accw + (uint32_t)cb, rw);
                 float4 pn[4];
                 if (cb + CSTEP < C) load_p(prow, cb + CSTEP, pn);
                 tmem_ld_wait();
@@ -691,8 +652,8 @@ corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restric
                     for (int u = 0; u < 4; ++u) p4[u] = pn[u];
                 }
             }
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            v2_mbar_arrive(bar_acce(buf));
+            tcgen05_fence_before();
+            mbar_arrive(bar_acce(buf));
         };
 
         const uint32_t ntiles = blockIdx.x < items ? ((items - 1u - blockIdx.x) / gridDim.x + 1u) * 4u : 0u;
@@ -723,22 +684,22 @@ corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restric
                 }
                 jcur = jnext;
                 if ((g & 3u) == 3u) {                       // the [C][33] tile of this 32-point item is complete
-                    v2_worker_sync<NWT>();
+                    named_bar_sync<1, NWT>();
                     const int g0 = i0 - 24;
                     for (int e = tid; e < 32 * C; e += NWT) {
                         const int o = e >> 5, pt = e & 31;
                         if (g0 + pt < N1) out[((size_t)b * C + o) * N1 + g0 + pt] = s_out[o * 33 + pt];
                     }
-                    v2_worker_sync<NWT>();                  // ... and read before the next item overwrites it
+                    named_bar_sync<1, NWT>();                  // ... and read before the next item overwrites it
                 }
                 b = bn; i0 = in0;
             }
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    if (warp == NW) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(tmem_cols) : "memory");
+    tcgen05_fence_after();
+    if (warp == NW) tmem_dealloc(tmem, tmem_cols);
 }
 
 // =====================================================================================================================
@@ -757,8 +718,8 @@ corr3d_v2_linear_kernel(const float* __restrict__ feat1, const float* __restrict
                         uint32_t tmem_cols, int nbuf) {
     constexpr int NW = 4, NWT = 128, DEPTH = 2;
     extern __shared__ uint8_t v2_smem_raw[];
-    const uint32_t sbase = (tc_smem_u32(v2_smem_raw) + 1023u) & ~1023u;
-    uint8_t* gbase = v2_smem_raw + (sbase - tc_smem_u32(v2_smem_raw));
+    const uint32_t sbase = (smem_u32(v2_smem_raw) + 1023u) & ~1023u;
+    uint8_t* gbase = v2_smem_raw + (sbase - smem_u32(v2_smem_raw));
     const int which = blockIdx.y;
     const float* X = which ? feat2 : feat1;
     float* out = which ? G2 : A1;
@@ -779,21 +740,20 @@ corr3d_v2_linear_kernel(const float* __restrict__ feat1, const float* __restrict
 
     if (tid == 0) {
         for (int s = 0; s < 2; ++s) {
-            tc_mbar_init(bar_full(s), NWT);
-            tc_mbar_init(bar_empty(s), 1);
-            tc_mbar_init(bar_accf(s), 1);
-            tc_mbar_init(bar_acce(s), NWT);
+            mbar_init(bar_full(s), NWT);
+            mbar_init(bar_empty(s), 1);
+            mbar_init(bar_accf(s), 1);
+            mbar_init(bar_acce(s), NWT);
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     if (warp == NW) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc(tmem_slot, tmem_cols);
     }
     for (int e = tid; e < C; e += blockDim.x) s_bias[e] = (which == 0 && b1) ? __ldg(b1 + e) : 0.0f;
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tcgen05_fence_after();
     const uint32_t tmem = *tmem_slot_ptr;
     const uint32_t idesc = umma_idesc_tf32(V2_ROWS, C);
 
@@ -805,11 +765,11 @@ corr3d_v2_linear_kernel(const float* __restrict__ feat1, const float* __restrict
                 const uint32_t acc = tmem + buf * (uint32_t)C;
                 for (int kb = 0; kb < nkb; ++kb, ++it) {
                     const uint32_t s = it % DEPTH, ph = it / DEPTH;
-                    v2_mbar_wait(bar_full(s), ph & 1u);
-                    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                    mbar_wait(bar_full(s), ph & 1u);
+                    tcgen05_fence_after();
                     if (kb == 0 && use >= 1) {
-                        v2_mbar_wait(bar_acce(buf), (use - 1) & 1u);
-                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                        mbar_wait(bar_acce(buf), (use - 1) & 1u);
+                        tcgen05_fence_after();
                     }
                     const uint32_t a_hi = sbase + a_off + s * 2 * V2_TILE, a_lo = a_hi + V2_TILE;
                     const uint32_t w_hi = sbase + w_off + s * wbytes, w_lo = w_hi + (uint32_t)C * 128u;
@@ -838,10 +798,10 @@ corr3d_v2_linear_kernel(const float* __restrict__ feat1, const float* __restrict
                 float v[V2_KB];
 #pragma unroll
                 for (int c = 0; c < V2_KB; ++c) v[c] = __ldg(x + (size_t)(kb * V2_KB + c) * N);      // coalesced over the warp's points
-                if (ph >= 1) v2_mbar_wait(bar_empty(s), (ph - 1) & 1u);
+                if (ph >= 1) mbar_wait(bar_empty(s), (ph - 1) & 1u);
                 if (tid == 0) {
-                    v2_mbar_arrive_tx(bar_full(s), (uint32_t)wbytes);
-                    v2_bulk_g2s(sbase + w_off + s * wbytes, Wimg + (size_t)kb * 2 * C * 32, (uint32_t)wbytes, bar_full(s));
+                    mbar_arrive_expect_tx(bar_full(s), (uint32_t)wbytes);
+                    bulk_g2s(sbase + w_off + s * wbytes, Wimg + (size_t)kb * 2 * C * 32, (uint32_t)wbytes, bar_full(s));
                 }
                 uint8_t* a_hi = gbase + a_off + s * 2 * V2_TILE;
                 uint8_t* a_lo = a_hi + V2_TILE;
@@ -852,21 +812,21 @@ corr3d_v2_linear_kernel(const float* __restrict__ feat1, const float* __restrict
                     *reinterpret_cast<float4*>(a_hi + off) = hi;
                     *reinterpret_cast<float4*>(a_lo + off) = make_float4(v[4 * q] - hi.x, v[4 * q + 1] - hi.y, v[4 * q + 2] - hi.z, v[4 * q + 3] - hi.w);
                 }
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                if (tid != 0) v2_mbar_arrive(bar_full(s));
+                fence_proxy_async();
+                if (tid != 0) mbar_arrive(bar_full(s));
             }
         };
         auto epilogue = [&](uint32_t item, uint32_t lt) {
             const uint32_t b = item / tiles;
             const int n = (int)(item - b * tiles) * V2_ROWS + row;
             const uint32_t buf = nbuf == 2 ? (lt & 1u) : 0u, use = nbuf == 2 ? (lt >> 1) : lt;
-            v2_mbar_wait(bar_accf(buf), use & 1u);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            mbar_wait(bar_accf(buf), use & 1u);
+            tcgen05_fence_after();
             const uint32_t acc = tmem + buf * (uint32_t)C + ((uint32_t)(warp * 32) << 16);
             float* orow = out + ((size_t)b * N + min(n, N - 1)) * C;
             for (int cb = 0; cb < C; cb += 16) {
                 uint32_t r[16];
-                tmem_ld16(acc + (uint32_t)cb, r);
+                tmem_ld(acc + (uint32_t)cb, r);
                 tmem_ld_wait();
                 if (n < N) {
 #pragma unroll
@@ -878,8 +838,8 @@ corr3d_v2_linear_kernel(const float* __restrict__ feat1, const float* __restrict
                     }
                 }
             }
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            v2_mbar_arrive(bar_acce(buf));
+            tcgen05_fence_before();
+            mbar_arrive(bar_acce(buf));
         };
         uint32_t cur = blockIdx.x, lt = 0;
         if (cur < items) produce(cur);
@@ -896,10 +856,10 @@ corr3d_v2_linear_kernel(const float* __restrict__ feat1, const float* __restrict
             ++lt;
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    if (warp == NW) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(tmem_cols) : "memory");
+    tcgen05_fence_after();
+    if (warp == NW) tmem_dealloc(tmem, tmem_cols);
 }
 
 // W1 [C, 2C+3] -> two swizzled images (columns 0..C-1 and C..2C-1), each [nkb][hi|lo][C rows x 32 floats]

@@ -19,7 +19,7 @@
 // precision 1 = TF32 operands, 2 = 3xTF32 (hi/lo split of both operands, three MMAs: fp32-level accuracy).
 #include <stdlib.h>
 
-#include "umma_common.cuh"
+#include "sm100_async.cuh"
 
 namespace b200 {
 
@@ -91,8 +91,8 @@ pointconv_tc_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
                     const float* __restrict__ bias, float* __restrict__ out, int Cp, int N, int S, int Cout, int Npad,
                     uint32_t tmem_cols) {
     extern __shared__ uint8_t pc_smem_raw[];
-    const uint32_t sbase = (tc_smem_u32(pc_smem_raw) + 1023u) & ~1023u;
-    uint8_t* g = pc_smem_raw + (sbase - tc_smem_u32(pc_smem_raw));
+    const uint32_t sbase = (smem_u32(pc_smem_raw) + 1023u) & ~1023u;
+    uint8_t* g = pc_smem_raw + (sbase - smem_u32(pc_smem_raw));
     const PcSmem Ls = pc_layout(Npad, SPLIT);
     float* s_wt = reinterpret_cast<float*>(g + Ls.wt);
     int* s_j = reinterpret_cast<int*>(g + Ls.jj);
@@ -104,13 +104,12 @@ pointconv_tc_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
     const int b = blockIdx.y, s0 = blockIdx.x * PC_PTS;
 
     if (tid == 0) {
-        tc_mbar_init(bar_free, 1);
-        tc_mbar_init(bar_done, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init(bar_free, 1);
+        mbar_init(bar_done, 1);
+        mbar_init_fence();
     }
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc(tmem_slot, tmem_cols);
     }
     for (int e = tid; e < 176 + Npad; e += PC_THREADS) {
         float v;
@@ -149,9 +148,9 @@ pointconv_tc_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
             s_wt[p * PC_WT_STRIDE + o * PC_K + kk] = lrelu01(v);
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tcgen05_fence_after();
     const uint32_t tmem = *tmem_slot_ptr;
 
     // ---- K loop
@@ -193,7 +192,7 @@ pointconv_tc_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
 #pragma unroll
                     for (int c = 0; c < 8; ++c) acc[c] = fmaf(ws[u], f[k4 * 4 + u][c], acc[c]);
             }
-            if (kbi >= 1) tc_mbar_wait(bar_free, (uint32_t)((kbi - 1) & 1));     // the MMAs reading the tiles are done
+            if (kbi >= 1) mbar_wait(bar_free, (uint32_t)((kbi - 1) & 1));     // the MMAs reading the tiles are done
 #pragma unroll
             for (int h = 0; h < 2; ++h) {                  // two 16-byte chunks of row p
                 const float4 v = make_float4(acc[4 * h], acc[4 * h + 1], acc[4 * h + 2], acc[4 * h + 3]);
@@ -221,10 +220,10 @@ pointconv_tc_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
                     *reinterpret_cast<float4*>(g + Ls.w_hi + off) = v;
                 }
             }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            fence_proxy_async();
             __syncthreads();
             if (tid == 0) {
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                tcgen05_fence_after();
 #pragma unroll
                 for (int ks = 0; ks < PC_KB / 8; ++ks) {
                     const uint64_t ah = umma_desc_sw128(sbase + Ls.a_hi + ks * 32), wh = umma_desc_sw128(sbase + Ls.w_hi + ks * 32);
@@ -240,15 +239,16 @@ pointconv_tc_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
             }
         }
     }
-    tc_mbar_wait(bar_done, 0u);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    mbar_wait(bar_done, 0u);
+    tcgen05_fence_after();
 
     // ---- epilogue: warps 0 and 1 own TMEM lanes 0..63 = the tile's points
     if (warp < 2) {
         const int sp = s0 + warp * 32 + lane;
         for (int cb = 0; cb < Npad; cb += 32) {
             uint32_t raw[32];
-            tmem_ld32(tmem + ((uint32_t)(warp * 32) << 16) + (uint32_t)cb, raw);
+            tmem_ld(tmem + ((uint32_t)(warp * 32) << 16) + (uint32_t)cb, raw);
+            tmem_ld_wait();
 #pragma unroll
             for (int c = 0; c < 32; ++c) {
                 const int o = cb + c;
@@ -256,9 +256,9 @@ pointconv_tc_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
             }
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(tmem_cols) : "memory");
+    if (warp == 0) tmem_dealloc(tmem, tmem_cols);
 }
 
 // second generation (pointconv_v2.cu): 128 points per CTA, warp-specialised; this file's kernel stays as the route for

@@ -20,7 +20,7 @@
 //                               per-split partials (each owned by one CTA; chunks add in launch order)
 // After the last chunk: pcb_reduce_kernel sums the partials in a fixed order (dL, dbias, dWa, dba, dWb, dbb are bit-
 // reproducible); pcb_finish_kernel turns the point-major dF rows into dfeat [B,C,N] and adds dF[0:3] into dxyz.
-#include "umma_common.cuh"
+#include "sm100_async.cuh"
 
 namespace b200 {
 
@@ -106,7 +106,7 @@ __device__ __forceinline__ float pb_load_b(const GemmArgs& a, int n, int k) {
 }
 __device__ __forceinline__ void pb_put(uint8_t* tile, int r, int kk, float v) {
     float* t = reinterpret_cast<float*>(tile);
-    const uint32_t off = (p2_sw64((uint32_t)r, (uint32_t)(kk >> 2)) >> 2) + (uint32_t)(kk & 3);
+    const uint32_t off = (sw64((uint32_t)r, (uint32_t)(kk >> 2)) >> 2) + (uint32_t)(kk & 3);
     const float hi = tf32_hi(v);
     t[off] = hi;
     t[G_TILE / 4 + off] = v - hi;
@@ -115,8 +115,8 @@ __device__ __forceinline__ void pb_put(uint8_t* tile, int r, int kk, float v) {
 template <int OP>
 __global__ void __launch_bounds__(G_THREADS, 1) pcb_gemm_kernel(GemmArgs a) {
     extern __shared__ uint8_t pb_smem_raw[];
-    const uint32_t sbase = (tc_smem_u32(pb_smem_raw) + 1023u) & ~1023u;
-    uint8_t* g = pb_smem_raw + (sbase - tc_smem_u32(pb_smem_raw));
+    const uint32_t sbase = (smem_u32(pb_smem_raw) + 1023u) & ~1023u;
+    uint8_t* g = pb_smem_raw + (sbase - smem_u32(pb_smem_raw));
     const uint32_t bars = sbase + G_DEPTH * G_STAGE;                 // empty[s] = bars + 8s, accf = bars + 32, slot = bars + 40
     const uint32_t bar_accf = bars + 32u, tmem_slot = bars + 40u;
     volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(g + G_DEPTH * G_STAGE + 40);
@@ -143,23 +143,22 @@ __global__ void __launch_bounds__(G_THREADS, 1) pcb_gemm_kernel(GemmArgs a) {
         return;
     }
     if (tid == 0) {
-        for (uint32_t s = 0; s < G_DEPTH; ++s) tc_mbar_init(bars + 8u * s, 1);
-        tc_mbar_init(bar_accf, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        for (uint32_t s = 0; s < G_DEPTH; ++s) mbar_init(bars + 8u * s, 1);
+        mbar_init(bar_accf, 1);
+        mbar_init_fence();
     }
     if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(256) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc(tmem_slot, 256);
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tcgen05_fence_after();
     const uint32_t tmem = *tmem_slot_ptr;
     const uint32_t idesc1 = umma_idesc_tf32(128, 128), idesc2 = umma_idesc_tf32(128, 256);
 
     for (int i = 0; i < nkb; ++i) {
         const int s = i % G_DEPTH, kbase = (kb0 + i) * 16;
-        if (i >= G_DEPTH) p2_mbar_wait(bars + 8u * s, (uint32_t)((i / G_DEPTH - 1) & 1));   // the MMAs that read it are done
+        if (i >= G_DEPTH) mbar_wait(bars + 8u * s, (uint32_t)((i / G_DEPTH - 1) & 1));   // the MMAs that read it are done
         uint8_t* st = g + s * G_STAGE;
 #pragma unroll
         for (int u = 0; u < 8; ++u) {
@@ -173,10 +172,10 @@ __global__ void __launch_bounds__(G_THREADS, 1) pcb_gemm_kernel(GemmArgs a) {
             const int e = tid + u * G_THREADS, r = e & 127, kk = e >> 7;
             pb_put(st + 2 * G_TILE, r, kk, pb_load_b<OP>(a, n0 + r, kbase + kk));
         }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        fence_proxy_async();
         __syncthreads();
         if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            tcgen05_fence_after();
             const uint32_t a_hi = sbase + s * G_STAGE, a_lo = a_hi + G_TILE, b_hi = a_hi + 2 * G_TILE;
 #pragma unroll
             for (int ks = 0; ks < 2; ++ks) {
@@ -188,16 +187,16 @@ __global__ void __launch_bounds__(G_THREADS, 1) pcb_gemm_kernel(GemmArgs a) {
         }
     }
     if (tid == 0) umma_commit(bar_accf);
-    p2_mbar_wait(bar_accf, 0u);
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    mbar_wait(bar_accf, 0u);
+    tcgen05_fence_after();
     {   // epilogue: warp -> TMEM lane quarter (warp & 3), column half (warp >> 2)
         const int qd = warp & 3, row = qd * 32 + lane, m = m0 + row;
         const uint32_t tbase = tmem + ((uint32_t)(qd * 32) << 16);
         for (int c0 = (warp >> 2) * 64; c0 < (warp >> 2) * 64 + 64; c0 += 8) {
             uint32_t r0[8], r1[8];
-            p2_tmem_ld8(tbase + (uint32_t)c0, r0);
-            p2_tmem_ld8(tbase + (uint32_t)(128 + c0), r1);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            tmem_ld(tbase + (uint32_t)c0, r0);
+            tmem_ld(tbase + (uint32_t)(128 + c0), r1);
+            tmem_ld_wait();
             if (m >= Mreal) continue;
 #pragma unroll
             for (int c = 0; c < 8; ++c) {
@@ -209,9 +208,9 @@ __global__ void __launch_bounds__(G_THREADS, 1) pcb_gemm_kernel(GemmArgs a) {
             }
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(256) : "memory");
+    if (warp == 0) tmem_dealloc(tmem, 256);
 }
 
 // ---- pass 2: per point ------------------------------------------------------------------------------------------

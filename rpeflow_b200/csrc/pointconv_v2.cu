@@ -17,7 +17,7 @@
 //     operand layout; one thread of warp 0 brings it into the stage with cp.async.bulk (expect_tx on the stage's "full"
 //     barrier) as soon as the stage is free; the weight-net outputs of the next K block are fetched under this block's FMAs.
 // precision 1 = TF32 operands, 2 (and 0) = 3xTF32.
-#include "umma_common.cuh"
+#include "sm100_async.cuh"
 
 namespace b200 {
 
@@ -63,7 +63,7 @@ pointconv_v2_prep_kernel(const float* __restrict__ xyz, const float* __restrict_
             const int cc = e & 15, o = (e >> 4) % Npad, kb = (e >> 4) / Npad;
             const int c = (kb >> 4) * P2_CB + cc, w = kb & 15;
             const float v = (o < Cout && c < Cf) ? __ldg(L + (size_t)o * P2_NW * Cf + (size_t)w * Cf + c) : 0.0f;
-            const uint32_t off = (p2_sw64((uint32_t)o, (uint32_t)(cc >> 2)) >> 2) + (uint32_t)(cc & 3);
+            const uint32_t off = (sw64((uint32_t)o, (uint32_t)(cc >> 2)) >> 2) + (uint32_t)(cc & 3);
             float* tile = Limg + (size_t)kb * (split ? 2 : 1) * Npad * 16;
             if (split) {
                 const float hi = tf32_hi(v);
@@ -97,14 +97,6 @@ __host__ __device__ inline P2Smem p2_layout(int Npad, int split, int depth) {
     return S;
 }
 
-__device__ __forceinline__ void p2_mbar_arrive_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void p2_bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-
 // MODE 0: TF32 (one MMA per k-step); 1: 3xTF32, B halves stacked along N (two MMAs, Npad <= 128); 2: 3xTF32, three MMAs.
 template <int MODE>
 __global__ void __launch_bounds__(P2_THREADS, 1)
@@ -115,8 +107,8 @@ pointconv_v2_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
                     uint32_t tmem_cols, int depth, int act) {
     constexpr int SPLIT = MODE != 0;
     extern __shared__ uint8_t p2_smem_raw[];
-    const uint32_t sbase = (tc_smem_u32(p2_smem_raw) + 1023u) & ~1023u;
-    uint8_t* g = p2_smem_raw + (sbase - tc_smem_u32(p2_smem_raw));
+    const uint32_t sbase = (smem_u32(p2_smem_raw) + 1023u) & ~1023u;
+    uint8_t* g = p2_smem_raw + (sbase - smem_u32(p2_smem_raw));
     const P2Smem Ls = p2_layout(Npad, SPLIT, depth);
     float* s_wt = reinterpret_cast<float*>(g + Ls.wt);
     uint16_t* s_j = reinterpret_cast<uint16_t*>(g + Ls.jj);
@@ -132,15 +124,14 @@ pointconv_v2_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
 
     if (tid == 0) {
         for (uint32_t s = 0; s < 4; ++s) {
-            tc_mbar_init(bars + 8u * s, P2_WORKERS / 32 + 1);      // one arrival per worker warp + the bulk copy's expect_tx arrival
-            tc_mbar_init(bars + 32u + 8u * s, 1);                  // stage free: tcgen05.commit
+            mbar_init(bars + 8u * s, P2_WORKERS / 32 + 1);      // one arrival per worker warp + the bulk copy's expect_tx arrival
+            mbar_init(bars + 32u + 8u * s, 1);                  // stage free: tcgen05.commit
         }
-        tc_mbar_init(bar_accf, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init(bar_accf, 1);
+        mbar_init_fence();
     }
     if (warp == P2_WORKERS / 32) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(tmem_cols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc(tmem_slot, tmem_cols);
     }
     for (int e = tid; e < 176 + Npad; e += P2_THREADS) {
         float v;
@@ -151,9 +142,9 @@ pointconv_v2_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
         else v = e - 176 < Cout ? __ldg(bias + e - 176) : 0.0f;
         s_small[e] = v;
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tcgen05_fence_after();
     const uint32_t tmem = *tmem_slot_ptr;
 
     if (warp == P2_WORKERS / 32) {
@@ -163,8 +154,8 @@ pointconv_v2_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
             const uint32_t a_bytes = (uint32_t)Ls.a_bytes, blo = (uint32_t)Npad * 64u;
             uint32_t s = 0, ph = 0;
             for (int kbi = 0; kbi < nkb; ++kbi) {
-                p2_mbar_wait(bars + 8u * s, ph & 1u);
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+                mbar_wait(bars + 8u * s, ph & 1u);
+                tcgen05_fence_after();
                 const uint32_t a_hi = sbase + Ls.ring + s * stage_bytes, a_lo = a_hi + P2_A_TILE;
                 const uint32_t b_hi = a_hi + a_bytes, b_lo = b_hi + blo;
 #pragma unroll
@@ -228,13 +219,13 @@ pointconv_v2_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
             for (int o = 0; o < P2_NW; ++o)
                 *reinterpret_cast<float4*>(s_wt + p * P2_WT_STRIDE + o * P2_K + 4 * q) = make_float4(wv[o][0], wv[o][1], wv[o][2], wv[o][3]);
         }
-        asm volatile("bar.sync 1, %0;" ::"n"(P2_WORKERS) : "memory");
+        named_bar_sync<1, P2_WORKERS>();
 
         // ---- K loop: K block kbi = (cb, w).  Per block: wait for the stage, 64 FMAs with the weights fetched one block ahead, one
         // 16-byte chunk of the A row (hi, lo) into the stage, one arrival per warp.
         const float* frow = Fpm + (size_t)b * N * Cp + 4 * q;
         const float4* wt4 = reinterpret_cast<const float4*>(s_wt + p * P2_WT_STRIDE);
-        uint8_t* const st0 = g + Ls.ring + p2_sw64((uint32_t)p, (uint32_t)q);
+        uint8_t* const st0 = g + Ls.ring + sw64((uint32_t)p, (uint32_t)q);
         const uint8_t* bsrc = reinterpret_cast<const uint8_t*>(Limg);      // this K block's B tile in global memory
         const uint32_t bdst0 = sbase + Ls.ring + (uint32_t)Ls.a_bytes;
         uint8_t* st = st0;                                      // this thread's chunk of the A row in the current stage
@@ -257,10 +248,10 @@ pointconv_v2_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
 #pragma unroll 1
             for (int w = 1; w <= P2_NW; ++w) {
                 if (warp == 0) {                                // warp 0 takes the stage first: one thread starts the bulk copy of the B tile
-                    p2_mbar_wait(bar_f + 32u, par_e);           // the MMAs that read this stage are done
+                    mbar_wait(bar_f + 32u, par_e);           // the MMAs that read this stage are done
                     if (lane == 0) {
-                        p2_mbar_arrive_tx(bar_f, b_bytes);
-                        p2_bulk_g2s(bdst, bsrc, b_bytes, bar_f);
+                        mbar_arrive_expect_tx(bar_f, b_bytes);
+                        bulk_g2s(bdst, bsrc, b_bytes, bar_f);
                     }
                     bsrc += b_bytes;
                 }
@@ -275,7 +266,7 @@ pointconv_v2_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
                         for (int c = 0; c < 4; ++c) acc[c] = fmaf(ws[u], f[k4 * 4 + u][c], acc[c]);
                     wc[k4] = wnx[k4];
                 }
-                if (warp != 0) p2_mbar_wait(bar_f + 32u, par_e);    // the other warps need the stage only now, after their FMAs
+                if (warp != 0) mbar_wait(bar_f + 32u, par_e);    // the other warps need the stage only now, after their FMAs
                 if (SPLIT) {
                     const float4 hi = make_float4(tf32_hi(acc[0]), tf32_hi(acc[1]), tf32_hi(acc[2]), tf32_hi(acc[3]));
                     *reinterpret_cast<float4*>(st) = hi;
@@ -283,9 +274,9 @@ pointconv_v2_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
                 } else {
                     *reinterpret_cast<float4*>(st) = make_float4(acc[0], acc[1], acc[2], acc[3]);
                 }
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                fence_proxy_async();
                 __syncwarp();
-                if (lane == 0) p2_mbar_arrive(bar_f);
+                if (lane == 0) mbar_arrive(bar_f);
                 if (++s == (uint32_t)depth) { s = 0; par_e ^= 1u; st = st0; bdst = bdst0; bar_f = bars; }
                 else { st += stage_bytes; bdst += stage_bytes; bar_f += 8u; }
             }
@@ -295,17 +286,17 @@ pointconv_v2_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
 
     // ---- epilogue, all 16 warps: warp -> TMEM lane quarter (warp & 3) = 32 points, column group (warp >> 2) = Npad/4 channels
     {
-        p2_mbar_wait(bar_accf, 0u);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        mbar_wait(bar_accf, 0u);
+        tcgen05_fence_after();
         const int qd = warp & 3, cg = warp >> 2, ncol = Npad >> 2;
         const int row = qd * 32 + lane, sp = s0 + row;
         const bool live = row < P2_PTS && sp < S;
         const uint32_t tbase = tmem + ((uint32_t)(qd * 32) << 16);
         for (int c0 = cg * ncol; c0 < (cg + 1) * ncol; c0 += 8) {
             uint32_t r0[8], r1[8];
-            p2_tmem_ld8(tbase + (uint32_t)c0, r0);
-            if (MODE == 1) p2_tmem_ld8(tbase + (uint32_t)(Npad + c0), r1);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            tmem_ld(tbase + (uint32_t)c0, r0);
+            if (MODE == 1) tmem_ld(tbase + (uint32_t)(Npad + c0), r1);
+            tmem_ld_wait();
 #pragma unroll
             for (int c = 0; c < 8; ++c) {
                 const int o = c0 + c;
@@ -318,9 +309,9 @@ pointconv_v2_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
             }
         }
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tcgen05_fence_before();
     __syncthreads();
-    if (warp == P2_WORKERS / 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(tmem_cols) : "memory");
+    if (warp == P2_WORKERS / 32) tmem_dealloc(tmem, tmem_cols);
 }
 
 int p2_cp(int C) { return (C + 3 + 15) / 16 * 16; }

@@ -25,7 +25,7 @@
 // neighbouring tile comes by (ncu: 1.9 GB read for a 0.98 GB map with 64 x 16 tiles, 1.2-1.3 GB with these).
 // The feat_3d copy to pixels (output channels 3..) stays the gather kernel of gather.cu, fed by point-major rows T.
 #include "project_common.cuh"
-#include "tma_common.cuh"
+#include "sm100_async.cuh"
 
 namespace b200 {
 
@@ -75,12 +75,6 @@ __device__ __forceinline__ float pt_blend(float f00, float f01, float f10, float
     const float r = __fmaf_rn(f11, w11, __fmaf_rn(f01, w01, 0.0f));
     return __fadd_rn(l, r);
 }
-__device__ __forceinline__ float lds_f32(uint32_t addr) {
-    float v;
-    asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(addr));
-    return v;
-}
-
 __device__ __forceinline__ int pt_tile_of(const TapXY& t, int H, int W, int tiles_x) {
     const int cx = min(max(t.x0, 0), W - 1), cy = min(max(t.y0, 0), H - 1);
     return (cy / PT_TH) * tiles_x + cx / PT_TW;
@@ -189,15 +183,6 @@ project_prep_kernel(const float* __restrict__ xy, const float* __restrict__ feat
 }
 
 // ---- the tile kernel ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ float4 lds_v4(uint32_t addr) {
-    float4 v;
-    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
-    return v;
-}
-__device__ __forceinline__ void sts_v4(uint32_t addr, float a, float b, float c, float d) {
-    asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
-}
-
 __global__ void __launch_bounds__(PT_THREADS, 1)
 project_tile_kernel(const __grid_constant__ CUtensorMap map, const float* __restrict__ feat2d, const float* __restrict__ xy,
                     const int64_t* __restrict__ nn, const int* __restrict__ list, const int* __restrict__ pos,
@@ -218,7 +203,7 @@ project_tile_kernel(const __grid_constant__ CUtensorMap map, const float* __rest
             mbar_init(bar_full + 8 * s, 1);
             mbar_init(bar_empty + 8 * s, CW);
         }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     __syncthreads();
 
@@ -227,14 +212,14 @@ project_tile_kernel(const __grid_constant__ CUtensorMap map, const float* __rest
 
     if (warp == CW) {                                             // ---------------- producer
         if (lane == 0) {
-            asm volatile("prefetch.tensormap [%0];" ::"l"(&map) : "memory");
+            prefetch_tensormap(&map);
             int s = 0;
             uint32_t ph = 0;
             for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
                 const int b = tile / per_img, r = tile - b * per_img;
                 const int ty = r / tiles_x, tx = r - ty * tiles_x;
                 for (int ch = 0; ch < nchunks; ++ch) {
-                    while (!mbar_test(bar_empty + 8 * s, ph ^ 1u)) __nanosleep(32);
+                    while (!mbar_try(bar_empty + 8 * s, ph ^ 1u)) __nanosleep(32);
                     mbar_arrive_expect_tx(bar_full + 8 * s, PT_STAGE);
                     tma_load_4d(base + s * PT_STAGE, &map, tx * PT_TW - PT_HALO, ty * PT_TH - PT_HALO, ch * PT_CC, b,
                                 bar_full + 8 * s);
@@ -373,7 +358,7 @@ project_tile_kernel(const __grid_constant__ CUtensorMap map, const float* __rest
                     *reinterpret_cast<float4*>(srow_b + (size_t)n * C2p + c0) = make_float4(v[0], v[1], v[2], v[3]);
                 }
             }
-            asm volatile("bar.sync 1, %0;" ::"n"(PT_CONSUMERS) : "memory");       // the chunk's table is complete
+            named_bar_sync<1, PT_CONSUMERS>();       // the chunk's table is complete
             // pixel job, table pixels: branch-free — 4 LDS.128 of own features (one per channel), 4 LDS.128 of S (one per
             // pixel), 16 FMAs.  Pixels on the other two paths load slot 0 and discard the product.
             float own[PT_CC][4];

@@ -2,6 +2,7 @@
 declares, rejects bad arguments without touching a GPU, the product never imports the oracle, and the shims
 satisfy the unmodified reference wrapper's import block (when a reference tree is staged under oracle/_ref)."""
 import ctypes
+import glob
 import os
 import re
 import subprocess
@@ -79,6 +80,23 @@ def test_product_never_touches_the_oracle():
                 text = open(os.path.join(base, f)).read()
                 assert not re.search(r"^\s*(from|import)\s+oracle\b", text, flags=re.M), f
                 assert "liboracle" not in text and "/root/reference" not in text, f
+
+
+ASYNC_PTX = ("mbarrier.", "tcgen05.", "cp.async.bulk", "fence.proxy", "fence.mbarrier_init", "bar.sync")
+
+
+def test_kernels_call_the_async_ptx_helpers():
+    """mbarrier, bulk/TMA copy, tcgen05, proxy-fence and named-barrier PTX is written once, in csrc/sm100_async.cuh
+    (one bounded mbarrier wait for every kernel); no kernel file spells it out in a string literal of its own."""
+    found = []
+    for path in sorted(glob.glob(os.path.join(ROOT, "rpeflow_b200", "csrc", "*.cu"))):
+        code = re.sub(r"/\*.*?\*/", lambda m: "\n" * m.group().count("\n"), open(path).read(), flags=re.S)
+        for n, line in enumerate(code.split("\n"), 1):
+            for tok in re.finditer(r'"(?:[^"\\\n]|\\.)*"|//.*', line):      # the first "//" outside a string ends the code
+                if tok.group().startswith("//"):
+                    break
+                found += [f"{os.path.basename(path)}:{n}: {line.strip()}" for op in ASYNC_PTX if op in tok.group()]
+    assert not found, "inline async PTX outside sm100_async.cuh:\n" + "\n".join(found)
 
 
 def test_same_names_as_the_reference_wrapper():
