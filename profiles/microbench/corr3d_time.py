@@ -1,5 +1,5 @@
 """Correlation3D at the five pyramid levels, batch 74 (the bench batch): device time per call, L2 flushed between calls.
-B200_CORR3D_V1=1 selects the first-generation kernels (corr3d_tc.cu + corr3d.cu stage 2) for an A/B comparison."""
+For an A/B comparison, run it once per build with B200FLOW_LIB pointing at the other library (profiles/build_variant.sh)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import torch
@@ -28,4 +28,4 @@ for C, N in LEVELS:
         flush.zero_(); a.record(); fn(); b.record(); b.synchronize(); ms.append(a.elapsed_time(b))
     ms.sort(); tot += ms[3]
     print(f"C={C:3d} N={N:4d} B={B}: {ms[3]*1e3:8.1f} us", flush=True)
-print(f"total {tot:.3f} ms  ({'v1' if os.environ.get('B200_CORR3D_V1') else 'v2'})")
+print(f"total {tot:.3f} ms")

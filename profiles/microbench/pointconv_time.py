@@ -1,5 +1,6 @@
 """PointConv forward (b200_pointconv_fwd) at the 20 call shapes of one RPEFlow forward (config 1), batch 74 by default:
-time per call for precision 2 (3xTF32) and 1 (TF32).  B200_POINTCONV_V1=1 times the first-generation kernel."""
+time per call for precision 2 (3xTF32) and 1 (TF32).  For an A/B comparison, run it once per build with B200FLOW_LIB
+pointing at the other library (profiles/build_variant.sh)."""
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import rpeflow_b200 as b200

@@ -13,8 +13,6 @@
 //     warp hit 8 different 16-byte bank groups (conflict-free LDS.128).
 //   * every in2 value loaded is used by up to 6 pixels x 2 packed lanes; every in1 value by 9 shifts.
 //   * stores: each thread writes 6 consecutive floats per displacement channel, the 4 strips of a row are contiguous.
-#include <stdlib.h>
-
 #include <algorithm>
 
 #include "common.cuh"
@@ -374,8 +372,7 @@ extern "C" int b200_corr2d_bwd(const float* gout, const float* in1, const float*
         B200_LAUNCH_CHECK("b200_corr2d_bwd(any md)");
         return B200_OK;
     }
-    const char* old_kernel = getenv("B200_CORR2D_BWD_SIMPLE");          // measurement knob: "1" = the first, untiled kernel
-    if (!(old_kernel && old_kernel[0] == '1') && corr2d_bwd_tiled_eligible(gout, in1, in2, gin1, gin2, B, C, H, W, md)) {
+    if (corr2d_bwd_tiled_eligible(gout, in1, in2, gin1, gin2, B, C, H, W, md)) {
         e = corr2d_bwd_tiled(gout, in1, in2, gin1, gin2, B, C, H, W, as_stream(stream));
         if (e != cudaSuccess) return cuda_fail(e, "b200_corr2d_bwd(tiled)");
         return B200_OK;

@@ -18,8 +18,6 @@
 //     reference's padding, correlation_forward_kernel.cu:36-41).
 //   * epilogue: 6 px = 24 bytes per (row, column shift): one 16-byte and one 8-byte streaming store, order chosen by
 //     the strip's parity so both are naturally aligned; the 8 strips of a row fill 192 contiguous bytes.
-#include <stdlib.h>
-
 #include "sm100_async.cuh"
 
 namespace b200 {
@@ -226,9 +224,6 @@ static bool make_diag_map(CUtensorMap* m, const float* ptr, int B, int C, int H,
 // Columns computed per useful column for the two tilings; the diagonal kernel is taken unless its 48-px tiles waste
 // clearly more of a narrow map than the 32-px tiles of corr2d_nchw.cu do.
 bool corr2d_diag_preferred(int W) {
-    const char* force = getenv("B200_CORR2D_TILING");            // "32" / "48": measurement knob (profiles/microbench)
-    if (force && force[0] == '3') return false;
-    if (force && force[0] == '4') return true;
     const double w48 = (double)ceil_div(W, D_TW) * D_TW / W, w32 = (double)ceil_div(W, 32) * 32 / W;
     return w48 <= 1.2 * w32;
 }

@@ -16,8 +16,6 @@
 //   pass 3  corr3d_stage2       : out[b,:,i] = sum_{j in knn11(i)} weight_net1(xyz1_j - xyz1_i) * P[b,j,:]
 //
 // precision 0 = fp32 FFMA throughout (this file).  Tensor-core variants of pass 2 live in corr3d_tc.cu.
-#include <stdlib.h>
-
 #include "corr3d_common.cuh"
 
 namespace b200 {
@@ -332,8 +330,7 @@ extern "C" int b200_corr3d_fwd(const float* xyz1, const float* feat1, const floa
     const Corr3dScratch s = carve(scratch, B, Cout, N1, N2);
     const int Kin = 2 * Cin + 3;
 
-    static const bool use_v1 = getenv("B200_CORR3D_V1") != nullptr;      // A/B switch for profiling: first-generation kernels
-    if (!use_v1 && Cin == Cout && corr3d_v2_eligible(Cout, k, precision)) {
+    if (Cin == Cout && corr3d_v2_eligible(Cout, k, precision)) {
         // second generation (corr3d_v2.cu): all three passes on tcgen05; needs W1cT from the common prep kernel
         corr3d_prep_weights<<<ceil_div(Cout * (Cout + 19), 256), 256, 0, st>>>(w->W1, w->W2, w->n1_Wc, w->n2_Wc, s.W2T, s.W1cT,
                                                                              s.n1WcT, s.n2WcT, Cin, Cout);

@@ -21,8 +21,6 @@
 // The accumulators are double-buffered in tensor memory when 4*C <= 512 columns, so the epilogue of tile t overlaps
 // the MMAs of tile t+1; produce(t+1) is issued before epilogue(t).
 #include <algorithm>
-#include <stdio.h>
-#include <stdlib.h>
 
 #include "corr3d_common.cuh"
 #include "sm100_async.cuh"
@@ -41,15 +39,6 @@ extern "C" __attribute__((visibility("default"))) int b200_debug_read_v2_trace(l
 namespace b200 {
 
 constexpr int V2_ROWS = 128, V2_KB = 32, V2_K = 16;
-#ifndef V2_GROUP
-#define V2_GROUP 4
-#endif
-#ifndef V2_MINB
-#define V2_MINB 4
-#endif
-#ifndef V2_PREJ
-#define V2_PREJ 0
-#endif
 constexpr int V2_TILE = V2_ROWS * 128;                  // one 128-row operand tile: 16 KB
 
 // ---- weight images (once per call) ---------------------------------------------------------------------------------
@@ -168,7 +157,7 @@ __device__ __forceinline__ void v2_hidden_full(const float* s_wn, float dx, floa
 // DEPTH = stages of the operand ring / HID buffers (2 also double-buffers the accumulators when 4*C <= 512 columns).
 // =====================================================================================================================
 template <int NW, int DEPTH>
-__global__ void __launch_bounds__(NW * 32 + 32, NW == 4 ? V2_MINB : 1)
+__global__ void __launch_bounds__(NW * 32 + 32, NW == 4 ? 4 : 1)
 corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict__ xyz2, const int64_t* __restrict__ knn12,
                         const float* __restrict__ A1, const float* __restrict__ G2, const float* __restrict__ W2img,
                         const float* __restrict__ wcimg, const float* __restrict__ W1cT, const float* __restrict__ Wa,
@@ -297,7 +286,7 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
             jpre = __ldg(knn12 + ((size_t)b * N1 + i) * V2_K + (row & 15));
             jpre_item = item;
         };
-        constexpr int STEPS = 1024 / NWT, GROUP = V2_GROUP;
+        constexpr int STEPS = 1024 / NWT, GROUP = 4;
         auto convert = [&](const float4& a, const float4& g, int r, int q, const float4& wx, const float4& wy, const float4& wz,
                            uint8_t* a_hi, uint8_t* a_lo) {
             const float4 d = s_d[r];
@@ -325,7 +314,7 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
                             z2 = __ldg(xyz2 + ((size_t)b * 3 + 2) * N2 + j);
                 const float x1 = __ldg(xyz1 + ((size_t)b * 3 + 0) * N1 + i), y1 = __ldg(xyz1 + ((size_t)b * 3 + 1) * N1 + i),
                             z1 = __ldg(xyz1 + ((size_t)b * 3 + 2) * N1 + i);
-                if ((DEEP || V2_PREJ) && item + gridDim.x < items) fetch_j(item + gridDim.x);   // in flight until the next produce()
+                if (DEEP && item + gridDim.x < items) fetch_j(item + gridDim.x);   // in flight until the next produce()
                 const float dx = x2 - x1, dy = y2 - y1, dz = z2 - z1;
 #ifdef V2_TRACE
                 if (dx == 123456.0f) s_d[row].w = dx;     // make the stamp below wait for the loads
@@ -492,21 +481,20 @@ corr3d_v2_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict_
 // =====================================================================================================================
 // pass 3: out[b,:,i] = sum_{j in knn11(i)} relu(weight_net1(xyz1_j - xyz1_i)) * P[b,j,:]
 // An item = 32 consecutive points of one sample (4 tiles of 128 rows); results go through a [C][33] shared-memory tile
-// so that the channel-first output is written as 128-byte runs.
+// so that the channel-first output is written as 128-byte runs.  4 worker warps (one thread per row) and one HID buffer /
+// accumulator: thin CTAs, up to 4 of which overlap each other on an SM.
 // =====================================================================================================================
-template <int NW, int DEPTH>
-__global__ void __launch_bounds__(NW * 32 + 32, NW == 4 ? 4 : 2)
+__global__ void __launch_bounds__(160, 4)
 corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restrict__ knn11, const float* __restrict__ P,
                         const float* __restrict__ wcimg, const float* __restrict__ Wa, const float* __restrict__ ba,
                         const float* __restrict__ Wb, const float* __restrict__ bb, float* __restrict__ out, int C, int N1, int B,
                         uint32_t tmem_cols) {
-    constexpr int NWT = NW * 32;
+    constexpr int NW = 4, NWT = 128;
     extern __shared__ uint8_t v2_smem_raw[];
     const uint32_t sbase = (smem_u32(v2_smem_raw) + 1023u) & ~1023u;
     uint8_t* gbase = v2_smem_raw + (sbase - smem_u32(v2_smem_raw));
-    const V2Smem L = v2_layout(C, false, true, DEPTH);
+    const V2Smem L = v2_layout(C, false, true, 1);
     float* s_wn = reinterpret_cast<float*>(gbase + L.wn);
-    int* s_j = reinterpret_cast<int*>(gbase + L.meta_j);    // [2][256]: slot = (tile parity, thread) — private to a thread
     float* s_out = reinterpret_cast<float*>(gbase + L.stagebuf);
     const uint32_t bars = sbase + L.bars;
     const uint32_t tmem_slot = bars + 72;
@@ -529,9 +517,9 @@ corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restric
     }
     if (tid < NWT) {
         weight_net_stage(s_wn, Wa, ba, Wb, bb, tid, NWT);
-        for (int e = tid; e < DEPTH * V2_ROWS * 8; e += NWT) {
-            const int buf = e / (V2_ROWS * 8), r = (e >> 3) & (V2_ROWS - 1), q = e & 7;
-            *reinterpret_cast<float4*>(gbase + HID_OFF(buf) + sw128(r, q)) = q == 4 ? make_float4(1.0f, 1.0f, 0.0f, 0.0f) : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+        for (int e = tid; e < V2_ROWS * 8; e += NWT) {
+            const int r = e >> 3, q = e & 7;
+            *reinterpret_cast<float4*>(gbase + HID_OFF(0) + sw128(r, q)) = q == 4 ? make_float4(1.0f, 1.0f, 0.0f, 0.0f) : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
         }
         for (int e = tid; e < C * 8; e += NWT)
             reinterpret_cast<float4*>(gbase + L.wc)[e] = __ldg(reinterpret_cast<const float4*>(wcimg) + e);
@@ -543,31 +531,31 @@ corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restric
     const uint32_t tmem = *tmem_slot_ptr;
     const uint32_t idesc = umma_idesc_tf32(V2_ROWS, C);
 
-    // tiles are numbered consecutively over this CTA's items: tile lt uses HID buffer / accumulator lt % DEPTH
+    // tiles are numbered consecutively over this CTA's items: tile lt is the lt-th use of the one HID buffer / accumulator
     if (warp == NW) {
         if (lane == 0) {
             uint32_t lt = 0;
             for (uint32_t item = blockIdx.x; item < items; item += gridDim.x) {
                 for (int t4 = 0; t4 < 4; ++t4, ++lt) {
-                    const uint32_t buf = lt % DEPTH, use = lt / DEPTH;
-                    mbar_wait(bar_full(buf), use & 1u);
+                    mbar_wait(bar_full(0), lt & 1u);
                     tcgen05_fence_after();
-                    if (use >= 1) {
-                        mbar_wait(bar_acce(buf), (use - 1) & 1u);
+                    if (lt >= 1) {
+                        mbar_wait(bar_acce(0), (lt - 1) & 1u);
                         tcgen05_fence_after();
                     }
-                    const uint32_t accw = tmem + buf * (uint32_t)C, wc = sbase + L.wc, hid = sbase + HID_OFF(buf);
+                    const uint32_t accw = tmem, wc = sbase + L.wc, hid = sbase + HID_OFF(0);
                     umma_tf32(accw, umma_desc_sw128(hid), umma_desc_sw128(wc), idesc, 0u);
                     umma_tf32(accw, umma_desc_sw128(hid), umma_desc_sw128(wc + 32), idesc, 1u);
                     umma_tf32(accw, umma_desc_sw128(hid + 32), umma_desc_sw128(wc), idesc, 1u);
                     umma_tf32(accw, umma_desc_sw128(hid + 64), umma_desc_sw128(wc + 64), idesc, 1u);
-                    umma_commit(bar_accf(buf));
+                    umma_commit(bar_accf(0));
                 }
             }
         }
         __syncwarp();
     } else {
-        const int row = tid & (V2_ROWS - 1), half = tid >> 7;
+        const int row = tid & (V2_ROWS - 1);
+        // ch is 0 in every worker warp; the kernel's register allocation (12 bytes of spill instead of 16) depends on it
         const int lq = warp & 3, ch = warp >> 2, m = lane & 15;
 
         // The tile sequence of this CTA: tile g = (item = blockIdx.x + (g / 4) * gridDim.x, quarter g % 4).
@@ -588,54 +576,43 @@ corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restric
             const int i = min(i0 + (row >> 4), N1 - 1);
             return __ldg(knn11 + ((size_t)b * N1 + i) * V2_K + (row & 15));
         };
-        // HID(g) may be overwritten once the MMAs of the tile that used the buffer last are complete: they are, because
-        // that tile's epilogue (which waited for bar_accf) precedes this call in program order of every worker.
-        auto meta = [&](uint32_t g, int b, int i0, int64_t jraw) -> int {
-            const uint32_t buf = g % DEPTH;
+        // The HID buffer may be overwritten once the MMAs of the previous tile are complete: they are, because that
+        // tile's epilogue (which waited for bar_accf) precedes this call in program order of every worker.
+        auto meta = [&](int b, int i0, int64_t jraw) -> int {
             const int i = min(i0 + (row >> 4), N1 - 1);
             int64_t j = jraw;
             j = j < 0 ? 0 : (j >= N1 ? N1 - 1 : j);
             const float dx = __ldg(xyz1 + ((size_t)b * 3 + 0) * N1 + j) - __ldg(xyz1 + ((size_t)b * 3 + 0) * N1 + i);
             const float dy = __ldg(xyz1 + ((size_t)b * 3 + 1) * N1 + j) - __ldg(xyz1 + ((size_t)b * 3 + 1) * N1 + i);
             const float dz = __ldg(xyz1 + ((size_t)b * 3 + 2) * N1 + j) - __ldg(xyz1 + ((size_t)b * 3 + 2) * N1 + i);
-            uint8_t* hid = gbase + HID_OFF(buf);
-            if (NW == 8) {
-                float hd[4];
-                v2_hidden_half(s_wn, dx, dy, dz, half, hd);
-                const float4 hi = make_float4(tf32_hi(hd[0]), tf32_hi(hd[1]), tf32_hi(hd[2]), tf32_hi(hd[3]));
-                *reinterpret_cast<float4*>(hid + sw128(row, half)) = hi;
-                *reinterpret_cast<float4*>(hid + sw128(row, 2 + half)) = make_float4(hd[0] - hi.x, hd[1] - hi.y, hd[2] - hi.z, hd[3] - hi.w);
-            } else {
-                float hd[8];
-                v2_hidden_full(s_wn, dx, dy, dz, hd);
+            uint8_t* hid = gbase + HID_OFF(0);
+            float hd[8];
+            v2_hidden_full(s_wn, dx, dy, dz, hd);
 #pragma unroll
-                for (int u = 0; u < 2; ++u) {
-                    const float4 hi = make_float4(tf32_hi(hd[4 * u]), tf32_hi(hd[4 * u + 1]), tf32_hi(hd[4 * u + 2]), tf32_hi(hd[4 * u + 3]));
-                    *reinterpret_cast<float4*>(hid + sw128(row, u)) = hi;
-                    *reinterpret_cast<float4*>(hid + sw128(row, 2 + u)) =
-                        make_float4(hd[4 * u] - hi.x, hd[4 * u + 1] - hi.y, hd[4 * u + 2] - hi.z, hd[4 * u + 3] - hi.w);
-                }
+            for (int u = 0; u < 2; ++u) {
+                const float4 hi = make_float4(tf32_hi(hd[4 * u]), tf32_hi(hd[4 * u + 1]), tf32_hi(hd[4 * u + 2]), tf32_hi(hd[4 * u + 3]));
+                *reinterpret_cast<float4*>(hid + sw128(row, u)) = hi;
+                *reinterpret_cast<float4*>(hid + sw128(row, 2 + u)) =
+                    make_float4(hd[4 * u] - hi.x, hd[4 * u + 1] - hi.y, hd[4 * u + 2] - hi.z, hd[4 * u + 3] - hi.w);
             }
             fence_proxy_async();
-            mbar_arrive(bar_full(buf));
+            mbar_arrive(bar_full(0));
             return (int)j;
         };
-        constexpr int CSTEP = 16 * (NW / 4);                // the warps of a lane quarter take alternate 16-column chunks
         auto load_p = [&](const float* prow, int cb, float4 (&p4)[4]) {
 #pragma unroll
             for (int u = 0; u < 4; ++u) p4[u] = __ldg(reinterpret_cast<const float4*>(prow + cb) + u);
         };
         auto epilogue = [&](uint32_t g, const float* prow, float4 (&p4)[4]) {
-            const uint32_t buf = g % DEPTH, use = g / DEPTH;
-            mbar_wait(bar_accf(buf), use & 1u);
+            mbar_wait(bar_accf(0), g & 1u);
             tcgen05_fence_after();
-            const uint32_t accw = tmem + buf * (uint32_t)C + ((uint32_t)(lq * 32) << 16);
+            const uint32_t accw = tmem + ((uint32_t)(lq * 32) << 16);
             const int ptl = (int)(g & 3u) * 8 + lq * 2 + (lane >> 4);   // point index inside the 32-point item
-            for (int cb = ch * 16; cb < C; cb += CSTEP) {
+            for (int cb = ch * 16; cb < C; cb += 16) {
                 uint32_t rw[16];
                 tmem_ld(accw + (uint32_t)cb, rw);
                 float4 pn[4];
-                if (cb + CSTEP < C) load_p(prow, cb + CSTEP, pn);
+                if (cb + 16 < C) load_p(prow, cb + 16, pn);
                 tmem_ld_wait();
                 float v[16];
 #pragma unroll
@@ -647,13 +624,13 @@ corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restric
                 }
                 const float tot = v2_reduce16(v, m);
                 s_out[(cb + m) * 33 + ptl] = tot;
-                if (cb + CSTEP < C) {
+                if (cb + 16 < C) {
 #pragma unroll
                     for (int u = 0; u < 4; ++u) p4[u] = pn[u];
                 }
             }
             tcgen05_fence_before();
-            mbar_arrive(bar_acce(buf));
+            mbar_arrive(bar_acce(0));
         };
 
         const uint32_t ntiles = blockIdx.x < items ? ((items - 1u - blockIdx.x) / gridDim.x + 1u) * 4u : 0u;
@@ -662,7 +639,7 @@ corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restric
             int b = 0, i0 = 0, bn = 0, in0 = 0;
             tile_pos(0, b, i0);
             int64_t jraw1 = fetch_j(1);
-            int jcur = meta(0, b, i0, fetch_j(0));
+            int jcur = meta(b, i0, fetch_j(0));
             int64_t jraw2 = fetch_j(2);
             for (uint32_t g = 0; g < ntiles; ++g) {
                 const bool more = g + 1 < ntiles;
@@ -670,15 +647,10 @@ corr3d_v2_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restric
                 const float* prow = P + ((size_t)b * N1 + jcur) * C;
                 float4 p4[4];
                 load_p(prow, ch * 16, p4);                  // requested before the accumulator wait
-                int jnext = 0;
-                if (DEPTH == 2 && more) {                   // with one buffer the next tile's HID can only be written after this epilogue
-                    jnext = meta(g + 1, bn, in0, jraw1);
-                    jraw1 = jraw2;
-                    jraw2 = fetch_j(g + 3);
-                }
                 epilogue(g, prow, p4);
-                if (DEPTH == 1 && more) {
-                    jnext = meta(g + 1, bn, in0, jraw1);
+                int jnext = 0;
+                if (more) {                                 // with one buffer the next tile's HID can only be written after this epilogue
+                    jnext = meta(bn, in0, jraw1);
                     jraw1 = jraw2;
                     jraw2 = fetch_j(g + 3);
                 }
@@ -877,26 +849,17 @@ __global__ void corr3d_v2_prep_w1_kernel(const float* __restrict__ W1, float* __
 
 // ---- host side -----------------------------------------------------------------------------------------------------
 struct V2Config { int nw, depth; };
-static V2Config v2_config(int C, int pass) {
-    // Thin CTAs (4 worker warps, one stage; 2-4 of them overlap each other on an SM) or fat ones (8 worker warps, 2-deep ring,
-    // hoisted loads; the overlap is inside the one CTA an SM can hold).  Measured at batch 74 (profiles/r2_corr3d.md): thin
-    // wins while >= 2 CTAs fit (C <= 128), fat wins pass 2 at C = 192.  B200_CORR3D_CFG="nw1,depth1,nw2,depth2" overrides.
-    static int ov[4] = {0, 0, 0, 0};
-    static bool parsed = false;
-    if (!parsed) {
-        parsed = true;
-        if (const char* e = getenv("B200_CORR3D_CFG")) sscanf(e, "%d,%d,%d,%d", &ov[0], &ov[1], &ov[2], &ov[3]);
-    }
-    V2Config c = (pass == 1 && C > 128) ? V2Config{8, 2} : V2Config{4, 1};
-    if (ov[2 * (pass - 1)]) c = V2Config{ov[2 * (pass - 1)], ov[2 * (pass - 1) + 1]};
-    return c;
+static V2Config v2_config(int C) {
+    // Pass 2: thin CTAs (4 worker warps, one stage; 2-4 of them overlap each other on an SM) or fat ones (8 worker warps,
+    // 2-deep ring, hoisted loads; the overlap is inside the one CTA an SM can hold).  Measured at batch 74
+    // (profiles/r2_notes.md): thin wins while >= 2 CTAs fit (C <= 128), fat wins pass 2 at C = 192.  Pass 3 is always thin.
+    return C > 128 ? V2Config{8, 2} : V2Config{4, 1};
 }
 
 bool corr3d_v2_eligible(int C, int k, int precision) {
     if (precision != 2) return false;                      // 3xTF32 only (the default; precision 1 keeps the first-generation kernel)
     if (k != V2_K || C % 32 != 0 || C < 32 || C > 192) return false;
-    const V2Config c1 = v2_config(C, 1), c2 = v2_config(C, 2);
-    return v2_layout(C, true, false, c1.depth).total + 1024 <= 227 * 1024 && v2_layout(C, false, true, c2.depth).total + 1024 <= 227 * 1024;
+    return v2_layout(C, true, false, v2_config(C).depth).total + 1024 <= 227 * 1024 && v2_layout(C, false, true, 1).total + 1024 <= 227 * 1024;
 }
 
 static uint32_t pow2_cols(int need) {
@@ -914,18 +877,13 @@ static cudaError_t v2_prepare(K kern, int threads, size_t smem, uint32_t cols, i
     if (e != cudaSuccess) return e;
     // CTAs per SM from first principles (registers are allocated per warp in units of 256; 1 KB of shared memory is
     // reserved per CTA; 228 KB per SM).  cudaOccupancyMaxActiveBlocksPerMultiprocessor answered 1 for every variant
-    // of these kernels on the r2 box while ncu reported 2-4 resident CTAs, so it is only printed for comparison.
+    // of these kernels on the r2 box while ncu reported 2-4 resident CTAs, so it is not used.
     cudaFuncAttributes fa;
     e = cudaFuncGetAttributes(&fa, kern);
     if (e != cudaSuccess) return e;
     const int warps = (threads + 31) / 32;
     const int regs_per_warp = ((fa.numRegs * 32 + 255) / 256) * 256;
     int n = std::min(std::min(65536 / (regs_per_warp * warps), (int)((228 * 1024) / (smem + fa.sharedSizeBytes + 1024))), 2048 / threads);
-    int api = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&api, kern, threads, smem);
-    static const bool debug = getenv("B200_DEBUG") != nullptr;
-    if (debug) fprintf(stderr, "corr3d_v2: threads %d regs %d smem %zu+%zu tmem cols %u -> %d CTAs/SM (api %d), tmem limit %u\n", threads,
-                       fa.numRegs, smem, (size_t)fa.sharedSizeBytes, cols, n, api, 512 / cols);
     n = std::min(n, (int)(512 / cols));                    // tensor memory: 512 columns per SM
     *ctas_per_sm = std::max(n, 1);
     return cudaSuccess;
@@ -960,7 +918,7 @@ cudaError_t corr3d_v2_run(const float* xyz1, const float* feat1, const float* xy
     }
     // ---- pass 2
     {
-        const V2Config c = v2_config(C, 1);
+        const V2Config c = v2_config(C);
         const int nbuf = (c.depth == 2 && 4 * C <= 512) ? 2 : 1;
         const size_t smem = (size_t)v2_layout(C, true, false, c.depth).total + 1024;
         const uint32_t cols = pow2_cols(nbuf * 2 * C);
@@ -975,8 +933,7 @@ cudaError_t corr3d_v2_run(const float* xyz1, const float* feat1, const float* xy
         corr3d_v2_stage1_kernel<NW, DEPTH><<<grid, threads, smem, st>>>(xyz1, xyz2, knn12, s.A1, s.G2, W2img, wc2, s.W1cT, w->n2_Wa, \
                                                                        w->n2_ba, w->n2_Wb, w->n2_bb, s.P, C, N1, N2, B, cols, nbuf); \
     } while (0)
-        if (c.nw == 8 && c.depth == 2) V2_LAUNCH1(8, 2);
-        else if (c.nw == 8) V2_LAUNCH1(8, 1);
+        if (c.nw == 8) V2_LAUNCH1(8, 2);
         else V2_LAUNCH1(4, 1);
 #undef V2_LAUNCH1
         e = cudaGetLastError();
@@ -984,24 +941,15 @@ cudaError_t corr3d_v2_run(const float* xyz1, const float* feat1, const float* xy
     }
     // ---- pass 3
     {
-        const V2Config c = v2_config(C, 2);
-        const size_t smem = (size_t)v2_layout(C, false, true, c.depth).total + 1024;
-        const uint32_t cols = pow2_cols(c.depth * C);
-        const int threads = c.nw * 32 + 32;
+        const size_t smem = (size_t)v2_layout(C, false, true, 1).total + 1024;
+        const uint32_t cols = pow2_cols(C);
         const long long items = (long long)B * ((N1 + 31) / 32);
         int per_sm = 1;
-#define V2_LAUNCH2(NW, DEPTH)                                                                                                       \
-    do {                                                                                                                            \
-        e = v2_prepare(corr3d_v2_stage2_kernel<NW, DEPTH>, threads, smem, cols, &per_sm);                                           \
-        if (e != cudaSuccess) return e;                                                                                             \
-        const int grid = (int)std::min<long long>(items, (long long)sm_count() * per_sm);                                           \
-        corr3d_v2_stage2_kernel<NW, DEPTH><<<grid, threads, smem, st>>>(xyz1, knn11, s.P, wc1, w->n1_Wa, w->n1_ba, w->n1_Wb, w->n1_bb, \
-                                                                       out, C, N1, B, cols);                                        \
-    } while (0)
-        if (c.nw == 8 && c.depth == 2) V2_LAUNCH2(8, 2);
-        else if (c.nw == 8) V2_LAUNCH2(8, 1);
-        else V2_LAUNCH2(4, 1);
-#undef V2_LAUNCH2
+        e = v2_prepare(corr3d_v2_stage2_kernel, 160, smem, cols, &per_sm);
+        if (e != cudaSuccess) return e;
+        const int grid = (int)std::min<long long>(items, (long long)sm_count() * per_sm);
+        corr3d_v2_stage2_kernel<<<grid, 160, smem, st>>>(xyz1, knn11, s.P, wc1, w->n1_Wa, w->n1_ba, w->n1_Wb, w->n1_bb, out, C, N1, B,
+                                                         cols);
     }
     return cudaGetLastError();
 }

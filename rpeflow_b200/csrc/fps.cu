@@ -18,7 +18,6 @@
 // Exactness (SURVEY §8a): start at index 0, distances start at 1e10, ties -> LOWEST index.  Equal to the
 // reference torch fallback models/csrc/wrapper.py:83-96 bit for bit.
 #include <cooperative_groups.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -31,20 +30,18 @@ struct FpsSlot {               // what a CTA publishes to its cluster peers each
     float x, y, z, pad;
 };
 
-template <int PPT, int T, int CS>
-__global__ void __launch_bounds__(T, 1)
+constexpr int FPS_PPT = 16, FPS_T = 512;               // points per thread, threads per CTA: 8192 points per CTA
+
+template <int CS>
+__global__ void __launch_bounds__(FPS_T, 1)
 fps_kernel(const float* __restrict__ xyz, int64_t* __restrict__ out, int N, int S, float negzero) {
-    constexpr int NW = T / 32;
+    constexpr int PPT = FPS_PPT, T = FPS_T, NW = T / 32;
     __shared__ unsigned s_d[2][32], s_i[2][32];
-    __shared__ __align__(16) FpsSlot s_slot[2][CS > 1 ? CS : 1];
-    extern __shared__ float s_pts[];                     // CS > 1: xyz of this CTA's chunk
+    __shared__ __align__(16) FpsSlot s_slot[2][CS];
+    extern __shared__ float s_pts[];                     // xyz of this CTA's chunk
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    int cloud = blockIdx.x, rank = 0;
-    if (CS > 1) {
-        rank = (int)cg::this_cluster().block_rank();
-        cloud = blockIdx.x / CS;
-    }
+    const int rank = (int)cg::this_cluster().block_rank(), cloud = blockIdx.x / CS;
     const int chunk = (N + CS - 1) / CS;
     const int lo = rank * chunk, hi = min(N, lo + chunk);
     const float* P = xyz + (size_t)cloud * N * 3;
@@ -58,13 +55,13 @@ fps_kernel(const float* __restrict__ xyz, int64_t* __restrict__ out, int N, int 
         py[i] = ok ? __ldg(P + (size_t)gi * 3 + 1) : 0.0f;
         pz[i] = ok ? __ldg(P + (size_t)gi * 3 + 2) : 0.0f;
         dist[i] = ok ? 1e10f : 0.0f;                     // padding never beats a real point (index tie-break below)
-        if (CS > 1 && ok) {
+        if (ok) {
             s_pts[(i * T + tid) * 3 + 0] = px[i];
             s_pts[(i * T + tid) * 3 + 1] = py[i];
             s_pts[(i * T + tid) * 3 + 2] = pz[i];
         }
     }
-    if (CS > 1) cg::this_cluster().sync();
+    cg::this_cluster().sync();
 
     unsigned cur = 0;
     float cx = __ldg(P + 0), cy = __ldg(P + 1), cz = __ldg(P + 2);
@@ -76,28 +73,20 @@ fps_kernel(const float* __restrict__ xyz, int64_t* __restrict__ out, int N, int 
 
         // Running argmax over this thread's points.  Only the slot number is tracked in the loop (SEL with an
         // immediate); padding slots hold distance 0 and an index >= hi, so they lose every tie to a real point.
+        // Two points per FADD2/FFMA2 (non-fused rule kept, see sqr2).
         float bd = -1.0f;
         int bslot = 0;
-        if (PPT >= 2) {                                  // two points per FADD2/FFMA2 (non-fused rule kept, see sqr2)
-            const u64 nz = pack2(negzero, negzero);
-            const u64 c2x = pack2(cx, cx), c2y = pack2(cy, cy), c2z = pack2(cz, cz);
+        const u64 nz = pack2(negzero, negzero);
+        const u64 c2x = pack2(cx, cx), c2y = pack2(cy, cy), c2z = pack2(cz, cz);
 #pragma unroll
-            for (int i = 0; i + 1 < PPT; i += 2) {
-                float d0, d1;
-                unpack2(sqdist_pair<3>(pack2(px[i], px[i + 1]), pack2(py[i], py[i + 1]), pack2(pz[i], pz[i + 1]),
-                                       c2x, c2y, c2z, nz), d0, d1);
-                dist[i] = fminf(dist[i], d0);
-                dist[i + 1] = fminf(dist[i + 1], d1);
-                if (dist[i] > bd) { bd = dist[i]; bslot = i; }                  // increasing index, strict '>': lowest index wins
-                if (dist[i + 1] > bd) { bd = dist[i + 1]; bslot = i + 1; }
-            }
-        } else {
-#pragma unroll
-            for (int i = 0; i < PPT; ++i) {
-                const float d = sqdist3_rule(px[i], py[i], pz[i], cx, cy, cz);
-                dist[i] = fminf(dist[i], d);
-                if (dist[i] > bd) { bd = dist[i]; bslot = i; }
-            }
+        for (int i = 0; i < PPT; i += 2) {
+            float d0, d1;
+            unpack2(sqdist_pair<3>(pack2(px[i], px[i + 1]), pack2(py[i], py[i + 1]), pack2(pz[i], pz[i + 1]),
+                                   c2x, c2y, c2z, nz), d0, d1);
+            dist[i] = fminf(dist[i], d0);
+            dist[i + 1] = fminf(dist[i + 1], d1);
+            if (dist[i] > bd) { bd = dist[i]; bslot = i; }                      // increasing index, strict '>': lowest index wins
+            if (dist[i + 1] > bd) { bd = dist[i + 1]; bslot = i + 1; }
         }
         const unsigned bi = (unsigned)(lo + bslot * T + tid);
         const unsigned db = __float_as_uint(bd);         // distances are >= +0: the bit pattern orders like the value
@@ -107,42 +96,32 @@ fps_kernel(const float* __restrict__ xyz, int64_t* __restrict__ out, int N, int 
         if (lane == 0) { s_d[par][warp] = wmax; s_i[par][warp] = widx; }
         __syncthreads();
 
-        if (CS == 1) {
+        cg::cluster_group cluster = cg::this_cluster();
+        if (warp == 0) {
             const unsigned vd = lane < NW ? s_d[par][lane] : 0u;
             const unsigned vi = lane < NW ? s_i[par][lane] : 0xFFFFFFFFu;
             const unsigned gmax = __reduce_max_sync(FULL, vd);
-            cur = __reduce_min_sync(FULL, vd == gmax ? vi : 0xFFFFFFFFu);
-            cx = __ldg(P + (size_t)cur * 3 + 0);         // L1-resident after the first touch
-            cy = __ldg(P + (size_t)cur * 3 + 1);
-            cz = __ldg(P + (size_t)cur * 3 + 2);
-        } else {
-            cg::cluster_group cluster = cg::this_cluster();
-            if (warp == 0) {
-                const unsigned vd = lane < NW ? s_d[par][lane] : 0u;
-                const unsigned vi = lane < NW ? s_i[par][lane] : 0xFFFFFFFFu;
-                const unsigned gmax = __reduce_max_sync(FULL, vd);
-                const unsigned gidx = __reduce_min_sync(FULL, vd == gmax ? vi : 0xFFFFFFFFu);
-                if (lane < CS) {                         // lane r writes this CTA's winner into peer r's slot
-                    FpsSlot v;
-                    v.key = ((unsigned long long)gmax << 32) | (unsigned long long)(0xFFFFFFFFu - gidx);
-                    const int li = (int)gidx - lo;          // < PPT*T even for a padding slot (never the global winner)
-                    v.x = s_pts[li * 3 + 0]; v.y = s_pts[li * 3 + 1]; v.z = s_pts[li * 3 + 2]; v.pad = 0.0f;
-                    FpsSlot* dst = cluster.map_shared_rank(&s_slot[par][rank], lane);
-                    *dst = v;
-                }
+            const unsigned gidx = __reduce_min_sync(FULL, vd == gmax ? vi : 0xFFFFFFFFu);
+            if (lane < CS) {                             // lane r writes this CTA's winner into peer r's slot
+                FpsSlot v;
+                v.key = ((unsigned long long)gmax << 32) | (unsigned long long)(0xFFFFFFFFu - gidx);
+                const int li = (int)gidx - lo;              // < PPT*T even for a padding slot (never the global winner)
+                v.x = s_pts[li * 3 + 0]; v.y = s_pts[li * 3 + 1]; v.z = s_pts[li * 3 + 2]; v.pad = 0.0f;
+                FpsSlot* dst = cluster.map_shared_rank(&s_slot[par][rank], lane);
+                *dst = v;
             }
-            cluster.sync();                              // release our DSMEM stores / acquire the peers'
-            FpsSlot w = s_slot[par][0];
-#pragma unroll
-            for (int r = 1; r < CS; ++r) {
-                const FpsSlot c = s_slot[par][r];
-                if (c.key > w.key) w = c;
-            }
-            cur = 0xFFFFFFFFu - (unsigned)(w.key & 0xFFFFFFFFull);
-            cx = w.x; cy = w.y; cz = w.z;
         }
+        cluster.sync();                                  // release our DSMEM stores / acquire the peers'
+        FpsSlot w = s_slot[par][0];
+#pragma unroll
+        for (int r = 1; r < CS; ++r) {
+            const FpsSlot c = s_slot[par][r];
+            if (c.key > w.key) w = c;
+        }
+        cur = 0xFFFFFFFFu - (unsigned)(w.key & 0xFFFFFFFFull);
+        cx = w.x; cy = w.y; cz = w.z;
     }
-    if (CS > 1) cg::this_cluster().sync();               // no CTA may exit while peers can still write its smem
+    cg::this_cluster().sync();                           // no CTA may exit while peers can still write its smem
 }
 
 // ---- pruned variant (one CTA per cloud, N <= 8192) --------------------------------------------------------------------
@@ -158,7 +137,7 @@ fps_kernel(const float* __restrict__ xyz, int64_t* __restrict__ out, int N, int 
 // box, and d_box >= the row's cached max proves that no dist[] of the row changes: the row is skipped, its cache
 // stays valid.  Rows that fail the test are updated exactly as in the full scan and their cache is recomputed with
 // two redux.  The running distances are therefore bit-identical to the full scan's at every iteration, and with the
-// (max distance, lowest original index) argmax so is every output index (tests: vs oracle, vs the full-scan kernel).
+// (max distance, lowest original index) argmax so is every output index (tests: vs the oracle).
 
 __device__ __forceinline__ unsigned fps_orderable(float v) {          // monotone float -> uint map (for redux min/max)
     const unsigned b = __float_as_uint(v);
@@ -365,28 +344,20 @@ static cudaError_t dispatch_pruned(const float* xyz, int64_t* idx, int B, int N,
     if (N <= 1024) return launch_fps_pruned<4, 256>(xyz, idx, B, N, S, st);
     if (N <= 2048) return launch_fps_pruned<4, 512>(xyz, idx, B, N, S, st);
     if (N <= 4096) return launch_fps_pruned<8, 512>(xyz, idx, B, N, S, st);
-    const char* t = getenv("B200_FPS_T");                // measurement / test knob: 1, 2 = other shapes, 3 / 0 = force / forbid the shared variant
-    if (t && t[0] == '2') return launch_fps_pruned<32, 256>(xyz, idx, B, N, S, st);
-    if (t && t[0] == '1') return launch_fps_pruned<8, 1024>(xyz, idx, B, N, S, st);
-    if (t && t[0] == '4') return launch_fps_pruned<32, 256, true>(xyz, idx, B, N, S, st);
     // more clouds than SMs: two clouds per SM (coordinates in shared memory) instead of a second wave
-    if ((B > sm_count() && !(t && t[0] == '0')) || (t && t[0] == '3')) return launch_fps_pruned<16, 512, true>(xyz, idx, B, N, S, st);
+    if (B > sm_count()) return launch_fps_pruned<16, 512, true>(xyz, idx, B, N, S, st);
     return launch_fps_pruned<16, 512>(xyz, idx, B, N, S, st);
 }
 
-template <int PPT, int T, int CS>
+template <int CS>
 static cudaError_t launch_fps(const float* xyz, int64_t* idx, int B, int N, int S, cudaStream_t st) {
-    auto kern = fps_kernel<PPT, T, CS>;
-    if (CS == 1) {
-        kern<<<B, T, 0, st>>>(xyz, idx, N, S, -0.0f);
-        return cudaGetLastError();
-    }
-    const size_t smem = (size_t)PPT * T * 3 * sizeof(float);
+    auto kern = fps_kernel<CS>;
+    const size_t smem = (size_t)FPS_PPT * FPS_T * 3 * sizeof(float);
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(B * CS);
-    cfg.blockDim = dim3(T);
+    cfg.blockDim = dim3(FPS_T);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
@@ -397,16 +368,6 @@ static cudaError_t launch_fps(const float* xyz, int64_t* idx, int B, int N, int 
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kern, xyz, idx, N, S, -0.0f);
-}
-
-template <int CS>
-static cudaError_t dispatch_ppt(const float* xyz, int64_t* idx, int B, int N, int S, cudaStream_t st) {
-    const int per_cta = (N + CS - 1) / CS;
-    if (per_cta <= 512) return launch_fps<1, 512, CS>(xyz, idx, B, N, S, st);
-    if (per_cta <= 1024) return launch_fps<2, 512, CS>(xyz, idx, B, N, S, st);
-    if (per_cta <= 2048) return launch_fps<4, 512, CS>(xyz, idx, B, N, S, st);
-    if (per_cta <= 4096) return launch_fps<8, 512, CS>(xyz, idx, B, N, S, st);
-    return launch_fps<16, 512, CS>(xyz, idx, B, N, S, st);
 }
 
 }  // namespace b200
@@ -421,27 +382,13 @@ extern "C" int b200_fps(const float* xyz, int64_t* idx, int B, int N, int n_samp
         return B200_ENOSUP;
     }
     if (B == 0) return B200_OK;
-    // Cluster size: the smallest that fits the cloud in registers; B200_FPS_CLUSTER=2|4|8 forces a larger one
-    // (shorter scan per iteration, one cluster barrier more) for small batches.
-    int cs = N <= 8192 ? 1 : N <= 16384 ? 2 : N <= 32768 ? 4 : 8;
-    if (const char* env = getenv("B200_FPS_CLUSTER")) {
-        const int want = atoi(env);
-        if ((want == 1 || want == 2 || want == 4 || want == 8) && want > cs) cs = want;
-    }
     cudaStream_t st = as_stream(stream);
+    // one CTA per cloud up to 8192 points; above, the smallest cluster whose CTAs hold the cloud in registers
     cudaError_t e;
-    const char* full = getenv("B200_FPS_FULL_SCAN");                 // measurement knob: "1" = the unpruned kernel
-    if (cs == 1 && !(full && full[0] == '1')) {
-        e = dispatch_pruned(xyz, idx, B, N, n_samples, st);
-        if (e != cudaSuccess) return cuda_fail(e, "b200_fps");
-        return B200_OK;
-    }
-    switch (cs) {
-        case 1: e = dispatch_ppt<1>(xyz, idx, B, N, n_samples, st); break;
-        case 2: e = dispatch_ppt<2>(xyz, idx, B, N, n_samples, st); break;
-        case 4: e = dispatch_ppt<4>(xyz, idx, B, N, n_samples, st); break;
-        default: e = dispatch_ppt<8>(xyz, idx, B, N, n_samples, st); break;
-    }
+    if (N <= 8192) e = dispatch_pruned(xyz, idx, B, N, n_samples, st);
+    else if (N <= 16384) e = launch_fps<2>(xyz, idx, B, N, n_samples, st);
+    else if (N <= 32768) e = launch_fps<4>(xyz, idx, B, N, n_samples, st);
+    else e = launch_fps<8>(xyz, idx, B, N, n_samples, st);
     if (e != cudaSuccess) return cuda_fail(e, "b200_fps");
     return B200_OK;
 }

@@ -26,8 +26,6 @@
 // which cells (and the atomically scattered points inside a cell) are visited does not matter.
 #include <math_constants.h>
 
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace b200 {
@@ -36,10 +34,7 @@ constexpr int KG_CELLS_MAX = 16384;     // cells per cloud (64 KB shared-memory 
 constexpr int KG_GMAX = 1024;           // cells per axis
 constexpr int KG_BUILD_THREADS = 1024;
 constexpr int KG_QUERY_THREADS = 128;
-#ifndef KG_STEP_N
-#define KG_STEP_N 4
-#endif
-constexpr int KG_STEP = KG_STEP_N;          // candidates per lane per lock-step iteration of the batched query (votes amortised)
+constexpr int KG_STEP = 4;              // candidates per lane per lock-step iteration of the batched query (votes amortised)
 
 struct KnnGridParams {                  // 48 bytes per cloud, written by the build kernel
     float lo[3];
@@ -510,7 +505,6 @@ static cudaError_t kg_run(const float* input, const float* query, int64_t* idx, 
     if (e != cudaSuccess) return e;
     int ctarget = k / 2 < 2 ? 2 : (k / 2 > 16 ? 16 : k / 2);
     if (k >= 16 && M <= 2048) ctarget = M <= 1024 ? 16 : 12;    // small clouds: coarser cells (self search 1024 pts, k = 16: 122 -> 89 us; 2048 pts: 202 -> 183 us)
-    if (const char* e = getenv("B200_KNN_CTARGET")) { const int v = atoi(e); if (v >= 1 && v <= 64 && k >= 16) ctarget = v; }   // measurement knob
     knn_grid_build_kernel<D><<<B, KG_BUILD_THREADS, smem, st>>>(input, M, isp, isd, ctarget, 1, s.params, s.cell_start, s.sorted_pts);
     KnnGridScratch q = s;
     if (s.sorted_q) {

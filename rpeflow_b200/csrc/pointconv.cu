@@ -17,8 +17,6 @@
 //                                   x N=out x K8) into a TMEM accumulator that lives across the whole K loop.
 //                                   epilogue: tcgen05.ld, + bias, LeakyReLU(0.1), channel-first coalesced stores.
 // precision 1 = TF32 operands, 2 = 3xTF32 (hi/lo split of both operands, three MMAs: fp32-level accuracy).
-#include <stdlib.h>
-
 #include "sm100_async.cuh"
 
 namespace b200 {
@@ -262,15 +260,11 @@ pointconv_tc_kernel(const float* __restrict__ xyz, const float* __restrict__ sam
 }
 
 // second generation (pointconv_v2.cu): 128 points per CTA, warp-specialised; this file's kernel stays as the route for
-// clouds of more than 65536 points and for A/B timing (B200_POINTCONV_V1=1)
+// clouds of more than 65536 points
 int pointconv_v2_run(const float* xyz, const float* feat, const float* sampled_xyz, const int64_t* knn,
                      const b200_pointconv_weights* w, float* out, float* scratch, int B, int C, int Cout, int N, int S,
                      int precision, int act, cudaStream_t st);
 int64_t pointconv_v2_scratch_floats(int B, int C, int Cout, int N);
-static bool pc_force_v1() {
-    static const bool v = [] { const char* e = getenv("B200_POINTCONV_V1"); return e && e[0] == '1'; }();
-    return v;
-}
 
 static inline int pc_cp(int C) { return (C + 3 + 31) / 32 * 32; }
 static inline int pc_npad(int Cout) { return (Cout + 31) / 32 * 32; }      // 32: the epilogue reads 32 TMEM columns at a time
@@ -322,7 +316,7 @@ extern "C" int b200_pointconv_fwd(const float* xyz, const float* feat, const flo
     }
     if (B == 0 || S == 0) return B200_OK;
     cudaStream_t st = as_stream(stream);
-    if (N <= 65536 && !pc_force_v1())
+    if (N <= 65536)
         return pointconv_v2_run(xyz, feat, sampled_xyz, knn, w, out, scratch, B, C, Cout, N, S, precision, 1, st);
     const int Cp = pc_cp(C), Npad = pc_npad(Cout);
     float* Fpm = scratch;

@@ -63,10 +63,10 @@ class CostVolumeStack:
             self.corr3d[lvl] = {n: v.to(self.device) for n, v in pwc3d.pack_weights(mod).items()}
         self._grids = {}
         self.concurrent = True        # independent op groups on side streams (parallel branches under graph capture)
-        self.max_streams = int(os.environ.get("B200_MAX_STREAMS", "3"))    # batch 148: 1 / 2 / 3 / 6 / 10 = 27.23 / 26.76 / 26.12 / 26.82 / 27.11 ms per step
+        self.max_streams = 3          # batch 148: 1 / 2 / 3 / 6 / 10 = 27.23 / 26.76 / 26.12 / 26.82 / 27.11 ms per step
         # streams the per-sample voxelisations are dealt onto: 2 pays for the RED-issue-bound tri-linear voxeliser (dsec step
         # 28.66 -> 27.83 ms at batch 148), not for the integer one (things: 26.77 -> 27.04 ms with 2, 27.7 with 3)
-        self.voxel_lanes = int(os.environ.get("B200_VOXEL_LANES", "2" if cfg.name == "dsec" else "1"))
+        self.voxel_lanes = 2 if cfg.name == "dsec" else 1
 
     def pixel_grid(self, batch, h, w):
         key = (batch, h, w)

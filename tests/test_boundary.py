@@ -99,6 +99,28 @@ def test_kernels_call_the_async_ptx_helpers():
     assert not found, "inline async PTX outside sm100_async.cuh:\n" + "\n".join(found)
 
 
+ENVIRONMENT = {"B200FLOW_LIB", "B200_CHECK_INDICES", "B200_PROJECT_ROUTE"}
+
+
+def test_environment_selects_no_kernel():
+    """The inputs choose every kernel, not the process's environment.  The library reads only B200FLOW_LIB (load another
+    build of libb200flow.so), B200_CHECK_INDICES (validate indices that come from outside the library) and
+    B200_PROJECT_ROUTE (run the two-pass projection on a map the tiled route takes, so that both can be compared on one
+    input); the native code reads only the last."""
+    native = set()
+    for path in sorted(glob.glob(os.path.join(ROOT, "rpeflow_b200", "csrc", "*.cu*"))):
+        code = re.sub(r"/\*.*?\*/|//[^\n]*", "", open(path).read(), flags=re.S)
+        for m in re.finditer(r"\bgetenv\b\s*(?:\(\s*\"(\w+)\")?", code):
+            native.add(m.group(1) or f"{os.path.basename(path)}: {code[m.start():m.start() + 40]}")
+    assert native <= {"B200_PROJECT_ROUTE"}, sorted(native)
+    python = set()
+    for path in sorted(glob.glob(os.path.join(ROOT, "rpeflow_b200", "**", "*.py"), recursive=True)):
+        code = re.sub(r"#[^\n]*", "", open(path).read())
+        for m in re.finditer(r"\b(?:environ|getenv)\b(?:(?:\.get\s*\(|\s*\[|\s*\()\s*([\"'])(\w+)\1)?", code):
+            python.add(m.group(2) or f"{os.path.relpath(path, ROOT)}: {code[m.start():m.start() + 40]}")
+    assert python <= ENVIRONMENT, sorted(python)
+
+
 def test_same_names_as_the_reference_wrapper():
     import rpeflow_b200.ops as ops
     for n in ("correlation2d", "furthest_point_sampling", "k_nearest_neighbor", "squared_distance",

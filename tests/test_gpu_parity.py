@@ -226,9 +226,9 @@ def _fps_adversarial_clouds():
             "lattice": np.ascontiguousarray(lattice), "ft3d": ft3d, "large": big}
 
 
-def test_fps_pruned_scan_exact(monkeypatch):
-    """The bounding-box pruned kernel (default for N <= 8192) returns the full scan's indices on every cloud: vs the
-    oracle and vs the unpruned kernel (B200_FPS_FULL_SCAN=1)."""
+def test_fps_pruned_scan_exact():
+    """The bounding-box pruned kernel (N <= 8192) returns the full scan's indices on every cloud, as the oracle computes
+    them."""
     clouds = _fps_adversarial_clouds()
     xyz = np.stack(list(clouds.values()))
     S = 1500
@@ -236,43 +236,43 @@ def test_fps_pruned_scan_exact(monkeypatch):
     got = b200.ops._furthest_point_sampling_cuda(cu(xyz), S).cpu().numpy()
     for i, name in enumerate(clouds):
         np.testing.assert_array_equal(got[i], want[i], err_msg=name)
-    monkeypatch.setenv("B200_FPS_FULL_SCAN", "1")
-    full = b200.ops._furthest_point_sampling_cuda(cu(xyz), S).cpu().numpy()
-    np.testing.assert_array_equal(full, want)
-    monkeypatch.delenv("B200_FPS_FULL_SCAN")
-    # full-size cloud (config 1), both kernels agree on all 4096 picks
+    # full-size clouds (config 1): all 4096 picks
     g = torch.Generator().manual_seed(12)
-    big = (torch.rand(6, 8192, 3, generator=g) * torch.tensor([30.0, 17.0, 90.0])).to(DEV)
-    a = b200.ops._furthest_point_sampling_cuda(big, 4096)
-    monkeypatch.setenv("B200_FPS_FULL_SCAN", "1")
-    assert torch.equal(a, b200.ops._furthest_point_sampling_cuda(big, 4096))
+    big = torch.rand(6, 8192, 3, generator=g) * torch.tensor([30.0, 17.0, 90.0])
+    got = b200.ops._furthest_point_sampling_cuda(big.to(DEV), 4096).cpu().numpy()
+    np.testing.assert_array_equal(got, spec.fps(big.numpy(), 4096))
 
 
-def test_fps_forced_cluster(monkeypatch):
-    rng = np.random.default_rng(9)
-    xyz = rng.random((3, 8192, 3), dtype=np.float32)
-    want = spec.fps(xyz, 512)
-    for cs in ("2", "4", "8"):
-        monkeypatch.setenv("B200_FPS_CLUSTER", cs)
-        np.testing.assert_array_equal(b200.ops._furthest_point_sampling_cuda(cu(xyz), 512).cpu().numpy(), want)
+def test_fps_forced_cluster():
+    """The cloud size forces a cluster of 2, 4 or 8 CTAs on clouds of more than 8192 points: both sides of each size
+    boundary, a ragged last CTA, and duplicates of the first CTA's points in the last one (ties between CTAs go to the
+    lowest index)."""
+    for N in (8193, 16384, 16385, 32768, 32769, 50001, 65536):
+        rng = np.random.default_rng(N)
+        xyz = rng.random((2, N, 3), dtype=np.float32) * np.array([30.0, 17.0, 90.0], dtype=np.float32)
+        xyz[:, 50:60] = xyz[:, 0:10]
+        xyz[:, -10:] = xyz[:, 0:10]
+        want = spec.fps(xyz, 600)
+        got = b200.ops._furthest_point_sampling_cuda(cu(xyz), 600).cpu().numpy()
+        np.testing.assert_array_equal(got, want, err_msg=f"N={N}")
 
 
-def test_fps_two_clouds_per_sm_variant(monkeypatch):
-    """Coordinates in shared memory, two clouds per SM (taken when a call has more clouds than SMs; B200_FPS_T=3 forces it,
-    =0 forbids it): same picks as the oracle and as the register-resident kernel, with and without padding slots."""
+def test_fps_two_clouds_per_sm_variant():
+    """Coordinates in shared memory, two clouds per SM (taken above 4096 points when a call has more clouds than SMs):
+    same picks as the oracle, with and without padding slots, and as the register-resident kernel that calls of at
+    most one cloud per SM take."""
+    sms = torch.cuda.get_device_properties(DEV).multi_processor_count
     rng = np.random.default_rng(31)
     for n in (8192, 5003):
-        xyz = (rng.random((3, n, 3), dtype=np.float32) * np.array([40.0, 25.0, 80.0], dtype=np.float32)).astype(np.float32)
+        xyz = (rng.random((sms + 1, n, 3), dtype=np.float32) * np.array([40.0, 25.0, 80.0], dtype=np.float32)).astype(np.float32)
         xyz[1, 100:400] = xyz[1, 7]                                     # duplicates: index tie-breaks
         want = spec.fps(xyz, 700)
-        monkeypatch.setenv("B200_FPS_T", "3")
         np.testing.assert_array_equal(b200.ops._furthest_point_sampling_cuda(cu(xyz), 700).cpu().numpy(), want)
-        monkeypatch.delenv("B200_FPS_T")
     g = torch.Generator().manual_seed(5)
-    many = (torch.rand(300, 8192, 3, generator=g) * torch.tensor([30.0, 17.0, 90.0])).to(DEV)      # > 148 clouds: the natural dispatch
+    many = (torch.rand(300, 8192, 3, generator=g) * torch.tensor([30.0, 17.0, 90.0])).to(DEV)
     a = b200.ops._furthest_point_sampling_cuda(many, 4096)
-    monkeypatch.setenv("B200_FPS_T", "0")
-    assert torch.equal(a, b200.ops._furthest_point_sampling_cuda(many, 4096))
+    parts = [b200.ops._furthest_point_sampling_cuda(c, 4096) for c in many.split(sms)]
+    assert torch.equal(a, torch.cat(parts))
 
 
 def test_fps_pyramid_prefix_property():
@@ -330,10 +330,11 @@ def test_corr2d_pyramid_levels_vs_oracle(C, H, W):
 
 
 @pytest.mark.parametrize("C,H,W", [(32, 144, 240), (64, 72, 120), (96, 36, 60), (128, 18, 28), (36, 11, 44), (8, 9, 12),
-                                   (20, 13, 50), (7, 5, 3)])
-def test_corr2d_backward_levels_vs_oracle(C, H, W, monkeypatch):
-    """a2 at the pyramid shapes: the register-tiled kernel (md = 4, C % 4 == 0, W % 4 == 0) and the simple one (other
-    shapes, or B200_CORR2D_BWD_SIMPLE=1) against the CPU oracle; ragged tiles and tiles larger than the map included."""
+                                   (20, 13, 50), (7, 5, 3), (30, 9, 20)])
+def test_corr2d_backward_levels_vs_oracle(C, H, W):
+    """a2 at the pyramid shapes: the register-tiled kernel (md = 4, C % 4 == 0, W % 4 == 0) and the simple one (the other
+    shapes: (20, 13, 50), (7, 5, 3), (30, 9, 20)) against the CPU oracle; ragged tiles and tiles larger than the map
+    included."""
     rng = np.random.default_rng(C * H + W)
     f1 = rng.standard_normal((2, H, W, C), dtype=np.float32)
     f2 = rng.standard_normal((2, H, W, C), dtype=np.float32)
@@ -342,10 +343,6 @@ def test_corr2d_backward_levels_vs_oracle(C, H, W, monkeypatch):
     g1, g2 = b200.ops._correlation_backward_cuda(cu(go), cu(f1), cu(f2), 4)
     np.testing.assert_allclose(g1.cpu().numpy(), w1, rtol=1e-5, atol=1e-5)
     np.testing.assert_allclose(g2.cpu().numpy(), w2, rtol=1e-5, atol=1e-5)
-    monkeypatch.setenv("B200_CORR2D_BWD_SIMPLE", "1")
-    s1, s2 = b200.ops._correlation_backward_cuda(cu(go), cu(f1), cu(f2), 4)
-    torch.testing.assert_close(g1, s1, rtol=1e-5, atol=1e-5)
-    torch.testing.assert_close(g2, s2, rtol=1e-5, atol=1e-5)
 
 
 @pytest.mark.parametrize("B,C,H,W,md", [(2, 19, 11, 14, 5), (1, 40, 20, 16, 7)])
