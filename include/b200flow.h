@@ -128,8 +128,22 @@ B200_API int b200_corr2d_bwd(const float* grad_out_nchw, const float* in1_nhwc, 
  * Rule (SURVEY §8a): idx[0]=0; dist_i = min(dist_i, ((dx*dx+dy*dy)+dz*dz)) in non-fused fp32, init 1e10;
  * next = argmax(dist), LOWEST index on ties  == the reference torch fallback (wrapper.py:83-96) bit for bit.
  * Requires N > n_samples >= 1 (wrapper.py:98 asserts it).  No scratch needed (distances live in registers).
+ * Limits: N <= 65536 (B200_ENOSUP otherwise: call b200_fps_large, which takes any N).
  */
 B200_API int b200_fps(const float* xyz, int64_t* idx, int B, int N, int n_samples, b200_stream_t stream);
+
+/* a3 for clouds of any size (the reference's kernel, furthest_point_sampling_kernel.cu:34-85, keeps its running
+ * distances in the global `dists_temp` and takes any N; b200_fps stops at 65536 points).  Same rule, same result as
+ * b200_fps bit for bit: a pruned scan over one 8-CTA thread-block cluster per cloud, on a Morton-sorted copy of the
+ * cloud in the caller's scratch (fps_large.cu).
+ *   xyz : [B,N,3] fp32 contiguous        idx : [B,n_samples] int64
+ *   scratch : >= b200_fps_scratch_bytes(B,N) bytes, 256-byte aligned; its contents on entry do not matter.
+ * Requires N > n_samples >= 1; short or misaligned scratch -> B200_EINVAL.  B = 0 is a no-op (NULL pointers allowed).
+ * No host synchronisation and no allocation: capturable in a CUDA graph.
+ */
+B200_API int64_t b200_fps_scratch_bytes(int B, int N);                 /* -1 for B < 0 or N < 1 */
+B200_API int b200_fps_large(const float* xyz, int64_t* idx, void* scratch, int64_t scratch_bytes, int B, int N,
+                            int n_samples, b200_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------------
  * a4  k nearest neighbours (brute-force exact).

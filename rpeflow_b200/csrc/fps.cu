@@ -19,7 +19,7 @@
 // reference torch fallback models/csrc/wrapper.py:83-96 bit for bit.
 #include <cooperative_groups.h>
 
-#include "common.cuh"
+#include "fps_common.cuh"
 
 namespace cg = cooperative_groups;
 
@@ -137,15 +137,9 @@ fps_kernel(const float* __restrict__ xyz, int64_t* __restrict__ out, int N, int 
 // box, and d_box >= the row's cached max proves that no dist[] of the row changes: the row is skipped, its cache
 // stays valid.  Rows that fail the test are updated exactly as in the full scan and their cache is recomputed with
 // two redux.  The running distances are therefore bit-identical to the full scan's at every iteration, and with the
-// (max distance, lowest original index) argmax so is every output index (tests: vs the oracle).
+// (max distance, lowest original index) argmax so is every output index (tests: vs the oracle).  The box test is
+// fps_common.cuh::fps_box_dist, shared with the cluster scan of fps_large.cu.
 
-__device__ __forceinline__ unsigned fps_orderable(float v) {          // monotone float -> uint map (for redux min/max)
-    const unsigned b = __float_as_uint(v);
-    return b ^ ((b >> 31) ? 0xFFFFFFFFu : 0x80000000u);
-}
-__device__ __forceinline__ float fps_unorder(unsigned u) {
-    return __uint_as_float(u ^ ((u >> 31) ? 0x80000000u : 0xFFFFFFFFu));
-}
 __device__ __forceinline__ unsigned fps_spread5(unsigned v) {         // 5 bits -> every third bit
     return (v & 1u) | ((v & 2u) << 2) | ((v & 4u) << 4) | ((v & 8u) << 6) | ((v & 16u) << 8);
 }
@@ -278,11 +272,8 @@ fps_pruned_kernel(const float* __restrict__ xyz, int64_t* __restrict__ out, int 
         if (s == S - 1) break;
 
         // which rows can change?  lane i answers for row i
-        const float gx = fmaxf(fmaxf(__fsub_rn(lox, cx), __fsub_rn(cx, hix)), 0.0f);
-        const float gy = fmaxf(fmaxf(__fsub_rn(loy, cy), __fsub_rn(cy, hiy)), 0.0f);
-        const float gz = fmaxf(fmaxf(__fsub_rn(loz, cz), __fsub_rn(cz, hiz)), 0.0f);
-        const float dbox = __fadd_rn(__fadd_rn(__fmul_rn(gx, gx), __fmul_rn(gy, gy)), __fmul_rn(gz, gz));
-        const unsigned mask = __ballot_sync(FULL, lane < PPT && !(dbox >= rmax_d));
+        const float dbox = fps_box_dist(lox, loy, loz, hix, hiy, hiz, cx, cy, cz);
+        const unsigned mask = __ballot_sync(FULL, lane < PPT && fps_box_may_change(dbox, rmax_d));
 #pragma unroll
         for (int g4 = 0; g4 < PPT; g4 += 4) {
             if (((mask >> g4) & 0xFu) == 0u) continue;   // warp-uniform
@@ -372,13 +363,22 @@ static cudaError_t launch_fps(const float* xyz, int64_t* idx, int B, int N, int 
 
 }  // namespace b200
 
+// Largest cloud b200_fps takes (the 8-CTA cluster holds 8 x 8192 points in registers); above it b200_fps returns
+// B200_ENOSUP and the host layer calls b200_fps_large.  A variant build may lower it to 8192 to time the pruned cluster
+// scan against fps_kernel<CS> on the same clouds (profiles/build_variant.sh; DESIGN §4).
+#ifndef B200_FPS_CLUSTER_MAX_N
+#define B200_FPS_CLUSTER_MAX_N 65536
+#endif
+static_assert(B200_FPS_CLUSTER_MAX_N >= 8192 && B200_FPS_CLUSTER_MAX_N <= 65536, "b200_fps: 8192 <= cluster limit <= 65536");
+
 extern "C" int b200_fps(const float* xyz, int64_t* idx, int B, int N, int n_samples, b200_stream_t stream) {
     using namespace b200;
     B200_REQUIRE((B == 0) || (xyz && idx), "b200_fps: null pointer");   // empty calls carry null pointers
     B200_REQUIRE(B >= 0 && n_samples >= 1, "b200_fps: bad sizes B=%d n_samples=%d", B, n_samples);
     B200_REQUIRE(N > n_samples, "b200_fps: need N > n_samples (N=%d, n_samples=%d) as models/csrc/wrapper.py:98", N, n_samples);
-    if (N > 8 * 8192) {
-        set_error("b200_fps: N=%d exceeds 65536 points per cloud (8-CTA cluster x 8192)", N);
+    if (N > B200_FPS_CLUSTER_MAX_N) {
+        set_error("b200_fps: N=%d exceeds %d points per cloud (8-CTA cluster x 8192); b200_fps_large takes any N",
+                  N, B200_FPS_CLUSTER_MAX_N);
         return B200_ENOSUP;
     }
     if (B == 0) return B200_OK;

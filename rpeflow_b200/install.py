@@ -335,7 +335,7 @@ def patch_python_ops(patch_events=True, only=None):
         return ops.furthest_point_sampling(xyz, n_samples)
 
     def furthest_point_sampling_ok(xyz, n_samples, cpp_impl=True):
-        return cpp_impl and xyz.dim() == 3 and xyz.shape[2] == 3 and n_samples < xyz.shape[1] <= 65536
+        return cpp_impl and xyz.dim() == 3 and xyz.shape[2] == 3 and n_samples < xyz.shape[1]
 
     def knn_interpolation(input_xyz, input_features, query_xyz, k=3):
         """models/utils.py:140-156: the k-nearest search, then gathers + inverse-distance weights + weighted sum in one kernel."""

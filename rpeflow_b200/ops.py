@@ -73,15 +73,26 @@ def _correlation_backward_cuda(grad_output, input1, input2, max_displacement):
     return g1, g2
 
 
+FPS_CLUSTER_MAX_N = 65536     # b200_fps holds a cloud of up to 8 x 8192 points in a cluster's registers
+
+
 def _furthest_point_sampling_cuda(points_xyz, n_samples):
-    """points_xyz [B,N,3] -> [B,n_samples] int64 (replaces furthest_point_sampling.cpp:5-16)."""
+    """points_xyz [B,N,3] -> [B,n_samples] int64 (replaces furthest_point_sampling.cpp:5-16).  Clouds of more than 65536
+    points (or whatever b200_fps of this build declines with B200_ENOSUP) take b200_fps_large with a scratch buffer."""
     _cuda_f32(points_xyz, "points_xyz")
     _require(points_xyz.dim() == 3 and points_xyz.shape[2] == 3, "points_xyz must be [B,N,3]")
     B, N, _ = points_xyz.shape
     out = torch.empty((B, int(n_samples)), dtype=torch.int64, device=points_xyz.device)
     with torch.cuda.device(points_xyz.device):
-        check(lib.b200_fps(points_xyz.data_ptr(), out.data_ptr(), B, N, int(n_samples), _stream(points_xyz)),
-              "b200_fps")
+        if N <= FPS_CLUSTER_MAX_N:
+            rc = lib.b200_fps(points_xyz.data_ptr(), out.data_ptr(), B, N, int(n_samples), _stream(points_xyz))
+            if rc != _lib.B200_ENOSUP:
+                check(rc, "b200_fps")
+                return out
+        nbytes = lib.b200_fps_scratch_bytes(B, N)
+        scratch = torch.empty((max(nbytes, 256),), dtype=torch.uint8, device=points_xyz.device)  # torch blocks are 512-B aligned
+        check(lib.b200_fps_large(points_xyz.data_ptr(), out.data_ptr(), scratch.data_ptr(), nbytes, B, N, int(n_samples),
+                                 _stream(points_xyz)), "b200_fps_large")
     return out
 
 
