@@ -120,6 +120,19 @@ B200_API int b200_corr2d_bwd(const float* grad_out_nchw, const float* in1_nhwc, 
                     float* gin1_nchw, float* gin2_nchw,
                     int B, int C, int H, int W, int md, b200_stream_t stream);
 
+/* a2 on NCHW maps: the backward of b200_corr2d_fwd_nchw with no permutes on either side.
+ *   grad_out : [B,81,H,W];  in1, in2 : [B,C,H,W] NCHW contiguous;  gin1, gin2 : [B,C,H,W] NCHW.  Any alignment, any W.
+ *   - a gradient passed as NULL is neither computed nor written; every element of a requested one is written;
+ *   - B = 0, or both gradients NULL, is a no-op that accepts NULL pointers; bad sizes, null inputs and grids beyond
+ *     2^31 - 1 tiles return B200_EINVAL before anything touches a device;
+ *   - no atomics (bit-reproducible), no allocation and no host synchronisation (the call can be captured in a graph).
+ * Limits: md == 4; any other displacement returns B200_ENOSUP (permute the inputs and call b200_corr2d_bwd).  Sums in
+ * the order of b200_corr2d_bwd's md = 4 tiled kernel, so where that one runs (C % 4 == 0, W % 4 == 0, 16-byte aligned
+ * pointers) both entries return the same bits.
+ */
+B200_API int b200_corr2d_bwd_nchw(const float* grad_out_nchw, const float* in1_nchw, const float* in2_nchw,
+                         float* gin1_nchw, float* gin2_nchw, int B, int C, int H, int W, int md, b200_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------------
  * a3  furthest point sampling.
  * Replaces: furthest_point_sampling.cpp:5-16 + furthest_point_sampling_kernel.cu:34-85; binding

@@ -3,6 +3,7 @@
 Public surface (same names as the reference, danqu130/RPEFlow):
   ops         correlation2d, furthest_point_sampling, k_nearest_neighbor      (models/csrc/wrapper.py)
               correlation2d_leaky, warp_correlate                             (RPEFlow_core.py:351,362 fused)
+              Correlation2dNCHWFunction — correlation2d's backward on NCHW maps (b200_corr2d_bwd_nchw)
   projection  batch_indexing_channel_{first,last}, grid_sample_wrapper, project_feat_with_nn_corr,
               knn_interpolation, backwarp_3d, backwarp_2d, convex_upsample    (models/utils.py)
               KnnInterpolationFunction, Backwarp2dFunction, ConvexUpsampleFunction — their backwards
@@ -17,7 +18,7 @@ Importing the package loads rpeflow_b200/libb200flow.so and fails loudly if it i
 """
 from . import _lib  # noqa: F401  (raises ImportError when the CUDA library is missing)
 from .ops import (correlation2d, correlation2d_leaky, warp_correlate, furthest_point_sampling,  # noqa: F401
-                  k_nearest_neighbor, squared_distance, CorrelationFunction)
+                  k_nearest_neighbor, squared_distance, CorrelationFunction, Correlation2dNCHWFunction)
 from .projection import (batch_indexing_channel_first, batch_indexing_channel_last, grid_sample_wrapper,  # noqa: F401
                          project_feat_with_nn_corr, knn_interpolation, backwarp_3d, backwarp_2d, convex_upsample,
                          KnnInterpolationFunction, Backwarp2dFunction, ConvexUpsampleFunction)

@@ -54,6 +54,7 @@ SIGNATURES = {
     "b200_convex_upsample_bwd_scratch_floats": (c_i64, [c_i, c_i, c_i, c_i]),
     "b200_convex_upsample_bwd": (c_i, [c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_p]),
     "b200_corr2d_bwd": (c_i, [c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_p]),
+    "b200_corr2d_bwd_nchw": (c_i, [c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_p]),
     "b200_fps": (c_i, [c_p, c_p, c_i, c_i, c_i, c_p]),
     "b200_fps_scratch_bytes": (c_i64, [c_i, c_i]),
     "b200_fps_large": (c_i, [c_p, c_p, c_p, c_i64, c_i, c_i, c_i, c_p]),
@@ -110,7 +111,7 @@ B200_ENOSUP = -3        # include/b200flow.h
 lib = _load()
 LAUNCHES = 0          # kernels of this library launched by this process (bench.py reports it as gpu_launches)
 KERNELS_PER_CALL = {"b200_knn_grid": 3, "b200_knn_grid_cf": 3, "b200_pointconv_fwd": 2, "b200_pointconv_fwd_linear": 2, "b200_pointconv_bwd": 6, "b200_corr2d_bwd": 2, "b200_project_nn_corr": 2, "b200_corr3d_fwd": 5, "b200_corr3d_bwd": 10, "b200_event_voxel_trilinear": 3,
-                    "b200_knn_interpolate_bwd": 1, "b200_backwarp2d_bwd": 1, "b200_convex_upsample_bwd": 2, "b200_fps_large": 5}
+                    "b200_knn_interpolate_bwd": 1, "b200_backwarp2d_bwd": 1, "b200_corr2d_bwd_nchw": 2, "b200_convex_upsample_bwd": 2, "b200_fps_large": 5}
 
 
 class B200Error(RuntimeError):

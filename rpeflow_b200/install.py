@@ -34,7 +34,10 @@ reference.  ``train`` is a collection of op names from ``TRAINABLE``:
   b200_knn_interpolate / b200_knn_interpolate_bwd;
 - "backwarp_2d": ``projection.Backwarp2dFunction``, b200_backwarp2d / b200_backwarp2d_bwd;
 - "convex_upsample": ``projection.ConvexUpsampleFunction``, b200_convex_upsample / b200_convex_upsample_bwd.  Its
-  backward has no atomics, so this one also trains here under deterministic mode.
+  backward has no atomics, so this one also trains here under deterministic mode;
+- "correlation2d" (lowercase, like the function): ``ops.Correlation2dNCHWFunction``, b200_corr2d_fwd_nchw / b200_corr2d_bwd_nchw on the model's NCHW maps
+  with no permutes (other displacements: b200_corr2d_fwd / b200_corr2d_bwd).  No atomics either: it also trains under
+  deterministic mode.
 A call takes the train route when it needs a graph, its op is in ``train``, every floating tensor is CUDA fp32 and its
 arguments are inside what the kernels were built for; ``stats()`` counts it as "b200".  ``train=True`` means
 {"Correlation3D"}.
@@ -58,7 +61,7 @@ _ADDED_MODULES = []    # sys.modules keys registered by install()
 _STATS = {}
 _OBSERVER = None
 _TRAIN = frozenset()   # ops whose calls that need a graph run this library's autograd Functions (install(train=...))
-TRAINABLE = ("Correlation3D", "PointConv", "knn_interpolation", "backwarp_2d", "convex_upsample")
+TRAINABLE = ("Correlation3D", "PointConv", "knn_interpolation", "backwarp_2d", "convex_upsample", "correlation2d")
 
 
 def stats(reset=False):
@@ -352,7 +355,8 @@ def patch_python_ops(patch_events=True, only=None):
         return batched_data.element_size() == 4 and not batched_indices.is_floating_point()
 
     replaced = {
-        "correlation2d": _dispatch("correlation2d", correlation2d, ref["correlation2d"], correlation2d_ok),
+        "correlation2d": _dispatch("correlation2d", correlation2d, ref["correlation2d"], correlation2d_ok, train="correlation2d",
+                                   atomics=False),
         "k_nearest_neighbor": _dispatch("k_nearest_neighbor", k_nearest_neighbor, ref["k_nearest_neighbor"], k_nearest_neighbor_ok),
         "furthest_point_sampling": _dispatch("furthest_point_sampling", furthest_point_sampling, ref["furthest_point_sampling"],
                                              furthest_point_sampling_ok),
@@ -414,7 +418,8 @@ def install(patch_python=True, patch_events=False, only=None, extensions=True, t
     """train: the ops whose calls that need an autograd graph run this library's forward and backward instead of the
     reference's torch code — a collection of names from TRAINABLE ("Correlation3D": pwc3d.Correlation3DFunction;
     "PointConv": pointconv.PointConvFunction under the module's own norm and activation; "knn_interpolation" (with
-    backwarp_3d), "backwarp_2d", "convex_upsample": the projection module's autograd Functions).  True means
+    backwarp_3d), "backwarp_2d", "convex_upsample": the projection module's autograd Functions; "correlation2d":
+    ops.Correlation2dNCHWFunction).  True means
     {"Correlation3D"}; False (the default) routes every such call to the reference."""
     global _TRAIN
     if isinstance(train, bool):

@@ -21,6 +21,7 @@ from ._lib import check, lib
 
 __all__ = [
     "correlation2d", "furthest_point_sampling", "k_nearest_neighbor", "squared_distance", "CorrelationFunction",
+    "Correlation2dNCHWFunction",
     "_correlation_forward_cuda", "_correlation_backward_cuda", "_furthest_point_sampling_cuda",
     "_k_nearest_neighbor_cuda", "knn_bruteforce",
 ]
@@ -161,13 +162,8 @@ def _no_fallback(name, *tensors):
             raise RuntimeError(f"rpeflow_b200.{name}: CUDA tensors required — this build has no CPU/torch fallback")
 
 
-def _correlation2d_nchw(input1, input2, max_displacement, negative_slope):
-    """The single-pass NCHW route (b200_corr2d_fwd_nchw[_leaky]); None when the call is outside its limits."""
-    needs_grad = torch.is_grad_enabled() and (input1.requires_grad or input2.requires_grad)
-    md = int(max_displacement)
-    if needs_grad or not 1 <= md <= 4 or input1.dim() != 4 or input1.shape != input2.shape:
-        return None
-    a, b = input1.contiguous().float(), input2.contiguous().float()
+def _corr2d_fwd_nchw(a, b, md, negative_slope):
+    """b200_corr2d_fwd_nchw[_leaky] on contiguous fp32 NCHW maps; None when the call is outside its limits."""
     B, C, H, W = a.shape
     out = torch.empty((B, (2 * md + 1) ** 2, H, W), dtype=torch.float32, device=a.device)
     with torch.cuda.device(a.device):
@@ -184,16 +180,72 @@ def _correlation2d_nchw(input1, input2, max_displacement, negative_slope):
     return out
 
 
+def _correlation2d_nchw(input1, input2, max_displacement, negative_slope):
+    """The single-pass NCHW route (b200_corr2d_fwd_nchw[_leaky]); None when the call is outside its limits."""
+    needs_grad = torch.is_grad_enabled() and (input1.requires_grad or input2.requires_grad)
+    md = int(max_displacement)
+    if needs_grad or not 1 <= md <= 4 or input1.dim() != 4 or input1.shape != input2.shape:
+        return None
+    return _corr2d_fwd_nchw(input1.contiguous().float(), input2.contiguous().float(), md, negative_slope)
+
+
+class Correlation2dNCHWFunction(torch.autograd.Function):
+    """correlation2d with a graph: NCHW in, NCHW out, gradients in the inputs' dtypes.
+
+    The forward runs the kernels of the no-grad call (b200_corr2d_fwd_nchw inside its limits, else permute +
+    b200_corr2d_fwd), so both forwards are bit-identical.  It saves the caller's NCHW inputs, no copies.  At md = 4 the
+    backward reads them as they are (b200_corr2d_bwd_nchw, no permutes); other displacements permute the saved inputs
+    for b200_corr2d_bwd, which writes NCHW gradients."""
+
+    @staticmethod
+    def forward(ctx, input1, input2, max_displacement):
+        _no_fallback("Correlation2dNCHWFunction", input1, input2)
+        md = int(max_displacement)
+        _require(input1.dim() == 4 and input1.shape == input2.shape, "input1/input2 must both be [B,C,H,W]")
+        a, b = input1.contiguous().float(), input2.contiguous().float()
+        out = _corr2d_fwd_nchw(a, b, md, None) if 1 <= md <= 4 else None
+        if out is None:
+            out = _correlation_forward_cuda(a.permute(0, 2, 3, 1).contiguous(), b.permute(0, 2, 3, 1).contiguous(), md)
+        ctx.save_for_backward(input1, input2)
+        ctx.max_displacement = md
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_output):
+        input1, input2 = ctx.saved_tensors
+        md = ctx.max_displacement
+        need1, need2 = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+        a, b = input1.contiguous().float(), input2.contiguous().float()
+        grad_output = grad_output.contiguous().float()
+        if md == 4:
+            B, C, H, W = a.shape
+            _require(tuple(grad_output.shape) == (B, 81, H, W), "grad_output has the wrong shape")
+            g1 = torch.empty_like(a) if need1 else None
+            g2 = torch.empty_like(b) if need2 else None
+            with torch.cuda.device(a.device):
+                check(lib.b200_corr2d_bwd_nchw(grad_output.data_ptr(), a.data_ptr(), b.data_ptr(),
+                                               g1.data_ptr() if need1 else None, g2.data_ptr() if need2 else None,
+                                               B, C, H, W, md, _stream(a)), "b200_corr2d_bwd_nchw")
+        else:
+            g1, g2 = _correlation_backward_cuda(grad_output, a.permute(0, 2, 3, 1).contiguous(),
+                                                b.permute(0, 2, 3, 1).contiguous(), md)
+        return (g1.to(input1.dtype) if need1 else None), (g2.to(input2.dtype) if need2 else None), None
+
+
 def correlation2d(input1, input2, max_displacement, cpp_impl=True):
     """input1, input2 [B,C,H,W] -> [B,(2md+1)^2,H,W] (wrapper.py:55-72). cpp_impl is accepted and ignored.
 
     Without autograd (inference; the reference evaluates under torch.no_grad) and for md = 4, W % 4 == 0 the cost
-    volume is computed straight from the NCHW maps (b200_corr2d_fwd_nchw): the wrapper's two permutes are gone.
+    volume is computed straight from the NCHW maps (b200_corr2d_fwd_nchw): the wrapper's two permutes are gone.  When
+    autograd needs a graph, Correlation2dNCHWFunction runs the same forward and a backward without permutes.
     Otherwise: permute to NHWC and go through CorrelationFunction exactly as wrapper.py:68-70 does."""
     _no_fallback("correlation2d", input1, input2)
     out = _correlation2d_nchw(input1, input2, max_displacement, None)
     if out is not None:
         return out
+    needs_grad = torch.is_grad_enabled() and (input1.requires_grad or input2.requires_grad)
+    if needs_grad and input1.dim() == 4 and input1.shape == input2.shape:
+        return Correlation2dNCHWFunction.apply(input1, input2, max_displacement)
     input1 = input1.permute(0, 2, 3, 1).contiguous().float()
     input2 = input2.permute(0, 2, 3, 1).contiguous().float()
     return CorrelationFunction.apply(input1, input2, max_displacement)
