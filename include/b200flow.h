@@ -239,6 +239,9 @@ B200_API int b200_project_nn_corr_sampled(const float* xy, const float* feat2d_n
  *   weights (row-major [out,in]): weight_net Wa [8,3], ba [8], Wb [16,8], bb [16]; linear L [Cout, 16*(C+3)], bias [Cout]
  *   scratch : >= b200_pointconv_scratch_floats(B,C,Cout,N) floats, 16-byte aligned.
  *   precision: 1 = TF32 tensor cores (tcgen05), 2 (and 0) = 3xTF32 (fp32-level accuracy).
+ *   knn indices are local to each sample.  A negative index wraps once (j + N, as torch indexing does) and whatever is
+ *   still outside [0, N-1] is clamped to it: -1 reads point N-1, -N-3 reads point 0, N or more reads point N-1.  No
+ *   error is reported for such indices.
  * Limits: k == 16, Cout <= 256 (B200_ENOSUP otherwise).
  */
 typedef struct b200_pointconv_weights {
@@ -319,6 +322,8 @@ B200_API int b200_knn_interpolate_bwd(const float* input_xyz, const float* input
  *     weight_net{1,2}: Wa[8,3],ba[8], Wb[8,8],bb[8], Wc[Cout,8],bc[Cout]    ReLU after each (incl. last)
  *   packed as struct b200_corr3d_weights (device pointers).
  *   scratch : >= b200_corr3d_scratch_floats(B,Cin,Cout,N1,N2,k) floats.
+ *   knn indices are local to each sample and are clamped to [0, N-1] of the cloud they index (N2 for knn12, N1 for
+ *   knn11): a negative index reads point 0 (it does not wrap), N or more reads point N-1.  No error is reported.
  *   precision: 0 = fp32 FFMA everywhere; 1 = TF32 tensor cores (tcgen05) for the Cout x Cout layer,
  *              fp32 accumulate (what cuDNN does for the reference's 1x1 convs under torch's default
  *              allow_tf32); 2 = 3xTF32 split (tensor cores, ~fp32 accuracy).
