@@ -375,6 +375,8 @@ B200_API int b200_corr3d_bwd(const float* xyz1, const float* feat1, const float*
  *   (the reference raises IndexError there; negative pixels in [-W,-1]/[-H,-1] wrap like torch indexing).
  *   polarity=1: channels [0,bins) count p>0 events, [bins,2*bins) count p<=0 events (both weight +1).
  *   polarity=0: one grid, weight = p (event_utils.py:247).
+ *   A zero-length window (first and last timestamps equal) makes the reference's normalised time 0/0 = NaN, which its
+ *   clamp keeps: every event then puts NaN into all channels at its pixel (with polarity=1, in both grids).
  */
 B200_API int b200_event_voxel_int(const float* events, int64_t n, float* vox, int bins, int H, int W,
                          int polarity, int* status, b200_stream_t stream);

@@ -468,6 +468,10 @@ ORC_API int64_t orc_event_voxel_int(const float* ev, int64_t n, float* vox, int 
         if (y < 0) y += H;
         volatile float ts = (e[2] - t_first) / den;
         volatile float tn = (ts - ts0) / dt * (float)(bins - 1);      /* event_utils.py:242 */
+        if (tn != tn) {                   /* zero-length window: tn = 0/0, clamp keeps NaN, NaN in every bin of every grid */
+            for (int b = 0; b < bins * (polarity ? 2 : 1); ++b) vox[(size_t)b * HW + (size_t)y * W + x] += NAN;
+            continue;
+        }
         float wgt; size_t base;
         if (polarity) { wgt = 1.0f; base = p > 0 ? 0 : (size_t)bins * HW; }
         else          { wgt = (float)p; base = 0; }

@@ -45,8 +45,16 @@ event_voxel_int_kernel(const float4* __restrict__ ev, int64_t n, float* __restri
     if (polarity) { wgt = 1.0f; base = p > 0 ? 0 : (size_t)bins * HW; }             // :293-296: both polarities weigh +1
     else          { wgt = (float)p; base = 0; }
     float* cell = vox + base + (size_t)y * W + x;
+    if (tn != tn) {
+        // Zero-length window (t_last == t_first): tn = 0/0.  torch.clamp keeps the NaN, so every bin of the event's pixel
+        // gets a NaN weight, in the other polarity's grid too (its weight-0 pass adds 0 * NaN).
+        const float qnan = __int_as_float(0x7fffffff);
+        float* pix = vox + (size_t)y * W + x;
+        for (int b = 0; b < bins * (polarity ? 2 : 1); ++b) atomicAdd(pix + (size_t)b * HW, qnan);
+        return;
+    }
     const float fl = floorf(tn);
-    if (!(fabsf(fl) < 1e9f)) return;                                                // NaN/Inf time: every bin weight is <= 0 or NaN
+    if (!(fabsf(fl) < 1e9f)) return;                                                // +-inf or huge tn: every clamped bin weight is 0
     const int b0 = (int)fl;
 #pragma unroll
     for (int k = 0; k < 2; ++k) {                                                   // only bins floor(tn), floor(tn)+1 can be > 0

@@ -42,6 +42,12 @@ def test_graph_replay_and_feeder_match_eager_run():
     stack.concurrent = False
     want, _ = stack.run(x)                                   # kernel by kernel, one stream
     want = {k: v for k, v in want.items() if k != "event_voxel"}      # atomics: order-dependent last ulp
+    from test_event_voxel_reference import check_cells, ref_int
+    refs = [ref_int(host["events"][i].numpy(), cfg.event_bins, cfg.height, cfg.width, True) for i in range(2)]
+
+    def voxels_match(out):                                   # instead, every sample cell by cell against the reference
+        for i, R in enumerate(refs):
+            check_cells(out["event_voxel"][i].cpu().numpy(), R, "stack tiny graph", f"sample {i}")
     stack.concurrent = True
     ints_w, flts_w = stack.checksum(stack.run(x)[0])
 
@@ -50,6 +56,7 @@ def test_graph_replay_and_feeder_match_eager_run():
         out = fused.replay()
     torch.cuda.synchronize()
     assert _same({k: v for k, v in out.items() if k != "event_voxel"}, want)
+    voxels_match(out)
     assert torch.equal(fused.checksum[0], ints_w)
     torch.testing.assert_close(fused.checksum[1], flts_w, rtol=1e-6, atol=1e-3)
 
@@ -62,6 +69,7 @@ def test_graph_replay_and_feeder_match_eager_run():
         out = runners[slot].replay(wait=lambda g, evs=evs: main.wait_event(evs[g]))
         main.synchronize()
         assert _same({k: v for k, v in out.items() if k != "event_voxel"}, want)
+        voxels_match(out)
         assert torch.equal(runners[slot].checksum[0], ints_w)
 
     # external inputs only (point clouds + raw events) streamed per step, the feature maps shared from the resident set
@@ -78,6 +86,7 @@ def test_graph_replay_and_feeder_match_eager_run():
         out = runners[slot].replay(wait=lambda g, evs=evs: main.wait_event(evs[g]))
         main.synchronize()
         assert _same({k: v for k, v in out.items() if k != "event_voxel"}, want)
+        voxels_match(out)
         assert torch.equal(runners[slot].checksum[0], ints_w)
 
 
@@ -86,7 +95,8 @@ def test_graph_replay_and_feeder_match_eager_run():
 def test_other_baseline_configs_run_and_index_ops_stay_exact(name):
     """BASELINE.json configs[3] (DSEC-shaped: 640x480, tri-linear voxels) and configs[4] (1920x1080, 32768 points: FPS
     over a 4-CTA cluster, KNN over 32768 inputs): one frame pair through the whole stack; FPS and a sample of the KNN
-    results are compared with the CPU oracle, float outputs must be finite and the voxel grid must hold every event."""
+    results are compared with the CPU oracle, float outputs must be finite and the voxel grid is held cell by cell to the
+    float64 reference of test_event_voxel_reference.py."""
     import numpy as np
     from oracle import spec
     dev = torch.device("cuda", 0)
@@ -107,9 +117,13 @@ def test_other_baseline_configs_run_and_index_ops_stay_exact(name):
     for lvl in range(1, 6):
         for t in [out["corr2d"][lvl], out["corr3d"][lvl]] + out["proj"][lvl] + out["sample"][lvl]:
             assert bool(torch.isfinite(t).all())
-    n_ev = cfg.n_events
-    total = float(out["event_voxel"].double().sum())
-    assert abs(total - n_ev) <= 1e-4 * n_ev if name.startswith("hd") else total > 0     # integer-pixel voxels conserve the event count
+    from test_event_voxel_reference import check_cells, ref_int, ref_trilinear
+    if name == "dsec":
+        R = ref_trilinear(host["ev_x"][0].numpy(), host["ev_y"][0].numpy(), host["ev_t"][0].numpy(), host["ev_p"][0].numpy(),
+                          cfg.event_bins, cfg.height, cfg.width, True)
+    else:
+        R = ref_int(host["events"][0].numpy(), cfg.event_bins, cfg.height, cfg.width, True)
+    check_cells(out["event_voxel"][0].cpu().numpy(), R, "stack " + name, name)
 
 
 @pytest.mark.gpu
