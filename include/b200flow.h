@@ -208,6 +208,32 @@ B200_API int b200_gather_cl(const void* data, const int64_t* idx, void* out,
 B200_API int b200_grid_sample_pts(const float* feat_nchw, const float* xy, float* out,
                          int B, int C, int H, int W, int N, b200_stream_t stream);
 
+/* a6 / a7 backwards (decoder_bwd.cu): the gradients of grid_sample_wrapper (F.grid_sample, models/utils.py:288-294) and
+ * of batch_indexing_channel_first / _last (torch.gather / advanced indexing, models/utils.py:119-137, :101-116).
+ * Rules as for the f3 / f4 backwards above: inputs and sizes exactly as given to the matching forward, grad_out has the
+ * forward output's shape; every gradient is overwritten (zero-filled with cudaMemsetAsync on `stream`, then accumulated);
+ * empty calls accept NULL pointers; bad arguments return B200_EINVAL before anything touches a device; no host
+ * synchronisation and no allocation (capturable in a CUDA graph).  Scattered gradients are summed with float atomics:
+ * not bit-reproducible.
+ *
+ * grid_sample_pts: dfeat [B,C,H,W], dxy [B,2,N]; either may be NULL (not computed, not written).  Taps are recomputed
+ * with the forward's own fp32 operations.  dxy follows ATen's grid_sampler_2d backward with zero padding (out-of-image
+ * taps read 0, nothing is clipped), reduced over the channels in a fixed order.  Where the forward finds no tap inside
+ * the image — the point lies outside it, or a coordinate is huge (|.| >= 1e9 after the round trip) or not finite, or
+ * W = 1 / H = 1 makes the round trip 0/0 — dxy is 0 (ATen gives 0 or NaN there).
+ */
+B200_API int b200_grid_sample_pts_bwd(const float* feat_nchw, const float* xy, const float* grad_out, float* dfeat_nchw,
+                             float* dxy, int B, int C, int H, int W, int N, b200_stream_t stream);
+
+/* gathers: fp32 only.  ddata [B,C,N] (cf) / [B,N,C] (cl) receives grad_out [B,C,I] / [B,I,C] at the element the forward
+ * read: negative indices wrap once, out-of-range ones clamp (the forward's rule; nothing is counted here).  The
+ * channel-last entry adds whole 16-byte rows (red.global.add.v4.f32) when C % 4 == 0 and both pointers are 16-byte
+ * aligned. */
+B200_API int b200_gather_cf_bwd(const float* grad_out, const int64_t* idx, float* ddata,
+                       int B, int C, int N, int64_t I, b200_stream_t stream);
+B200_API int b200_gather_cl_bwd(const float* grad_out, const int64_t* idx, float* ddata,
+                       int B, int C, int N, int64_t I, b200_stream_t stream);
+
 /* a8  point -> image projection with nearest-neighbour correlation.
  * Replaces: models/utils.py:297-317 (project_feat_with_nn_corr) with nn_indices supplied
  *           (models/RPEFlow_core.py:329-330 always supplies them).

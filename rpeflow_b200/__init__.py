@@ -6,7 +6,8 @@ Public surface (same names as the reference, danqu130/RPEFlow):
               Correlation2dNCHWFunction — correlation2d's backward on NCHW maps (b200_corr2d_bwd_nchw)
   projection  batch_indexing_channel_{first,last}, grid_sample_wrapper, project_feat_with_nn_corr,
               knn_interpolation, backwarp_3d, backwarp_2d, convex_upsample    (models/utils.py)
-              KnnInterpolationFunction, Backwarp2dFunction, ConvexUpsampleFunction — their backwards
+              KnnInterpolationFunction, Backwarp2dFunction, ConvexUpsampleFunction, GridSampleFunction,
+              BatchIndexingChannelFirstFunction, BatchIndexingChannelLastFunction — their backwards
   pwc3d       Correlation3D, build_pc_pyramid                                 (models/pwc3d_core.py)
               correlation3d, Correlation3DFunction — the same op with a backward (b200_corr3d_bwd)
   pointconv   PointConvDownSampling, PointConvNoSampling                      (models/pointconv.py)
@@ -21,7 +22,8 @@ from .ops import (correlation2d, correlation2d_leaky, warp_correlate, furthest_p
                   k_nearest_neighbor, squared_distance, CorrelationFunction, Correlation2dNCHWFunction)
 from .projection import (batch_indexing_channel_first, batch_indexing_channel_last, grid_sample_wrapper,  # noqa: F401
                          project_feat_with_nn_corr, knn_interpolation, backwarp_3d, backwarp_2d, convex_upsample,
-                         KnnInterpolationFunction, Backwarp2dFunction, ConvexUpsampleFunction)
+                         KnnInterpolationFunction, Backwarp2dFunction, ConvexUpsampleFunction, GridSampleFunction,
+                         BatchIndexingChannelFirstFunction, BatchIndexingChannelLastFunction)
 from .pwc3d import (Correlation3D, Correlation3DFunction, build_pc_pyramid, correlation3d,  # noqa: F401
                     correlation3d_forward)
 from .pointconv import PointConvDownSampling, PointConvNoSampling, pointconv_forward  # noqa: F401

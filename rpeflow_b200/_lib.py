@@ -65,6 +65,9 @@ SIGNATURES = {
     "b200_gather_cf": (c_i, [c_p, c_p, c_p, c_i, c_i, c_i, c_i64, c_p, c_p]),
     "b200_gather_cl": (c_i, [c_p, c_p, c_p, c_i, c_i, c_i, c_i64, c_p, c_p]),
     "b200_grid_sample_pts": (c_i, [c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_p]),
+    "b200_grid_sample_pts_bwd": (c_i, [c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_p]),
+    "b200_gather_cf_bwd": (c_i, [c_p, c_p, c_p, c_i, c_i, c_i, c_i64, c_p]),
+    "b200_gather_cl_bwd": (c_i, [c_p, c_p, c_p, c_i, c_i, c_i, c_i64, c_p]),
     "b200_project_nn_corr": (c_i, [c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_p]),
     "b200_project_nn_corr_scratch_floats": (c_i64, [c_i, c_i, c_i, c_i]),
     "b200_project_nn_corr_sampled": (c_i, [c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_p]),
@@ -111,7 +114,8 @@ B200_ENOSUP = -3        # include/b200flow.h
 lib = _load()
 LAUNCHES = 0          # kernels of this library launched by this process (bench.py reports it as gpu_launches)
 KERNELS_PER_CALL = {"b200_knn_grid": 3, "b200_knn_grid_cf": 3, "b200_pointconv_fwd": 2, "b200_pointconv_fwd_linear": 2, "b200_pointconv_bwd": 6, "b200_corr2d_bwd": 2, "b200_project_nn_corr": 2, "b200_corr3d_fwd": 5, "b200_corr3d_bwd": 10, "b200_event_voxel_trilinear": 3,
-                    "b200_knn_interpolate_bwd": 1, "b200_backwarp2d_bwd": 1, "b200_corr2d_bwd_nchw": 2, "b200_convex_upsample_bwd": 2, "b200_fps_large": 5}
+                    "b200_knn_interpolate_bwd": 1, "b200_backwarp2d_bwd": 1, "b200_corr2d_bwd_nchw": 2, "b200_convex_upsample_bwd": 2, "b200_fps_large": 5,
+                    "b200_grid_sample_pts_bwd": 1, "b200_gather_cf_bwd": 1, "b200_gather_cl_bwd": 1}
 
 
 class B200Error(RuntimeError):
@@ -128,10 +132,10 @@ def check(rc, what):
 
 def require_dense(what, **tensors):
     """Raise unless every tensor is a contiguous CUDA tensor of the dtype the kernels read (int64 for names starting
-    with "knn", fp32 otherwise): the entry points pass raw data pointers and would read any other layout wrongly."""
+    with "knn" or "idx", fp32 otherwise): the entry points pass raw data pointers and would read any other layout wrongly."""
     import torch
     for name, t in tensors.items():
-        want = torch.int64 if name.startswith("knn") else torch.float32
+        want = torch.int64 if name.startswith(("knn", "idx")) else torch.float32
         if not (t.is_cuda and t.dtype == want and t.is_contiguous()):
             raise ValueError(f"{what}: {name} must be a contiguous CUDA {want} tensor, got {t.dtype} on {t.device}"
                              f"{'' if t.is_contiguous() else ', not contiguous'} (the functional form converts it)")

@@ -1,22 +1,24 @@
-// decoder_bwd.cu — backwards of the decoder's f2 / f3 / f4 forwards in gather.cu:
+// decoder_bwd.cu — backwards of the decoder's f2 / f3 / f4 and the projection gathers' a6 / a7 forwards in gather.cu:
 //   f2 knn_interpolation (models/utils.py:140-156; backwarp_3d :159-169 is the same op on (xyz1+flow, -flow)),
 //   f3 backwarp_2d with padding_mode='border' (:186-198),
-//   f4 convex_upsample (:201-214).
+//   f4 convex_upsample (:201-214),
+//   a6 batch_indexing_channel_first / _last (:119-137 torch.gather, :101-116 advanced indexing),
+//   a7 grid_sample_wrapper (:288-294, F.grid_sample bilinear, align_corners=True, zero padding).
 //
-// Nothing of the forward is saved beyond its inputs and indices: every kernel recomputes the taps, weights and softmax
-// with the forward's own fp32 operations (decoder_common.cuh), so the gradient belongs to exactly the output the
-// forward produced.  All of them are HBM / L2-atomic bound; there is no tensor-core work here.
+// Nothing of the forward is saved beyond its inputs and indices: every kernel recomputes the taps, weights, softmax and
+// gather indices with the forward's own fp32 operations (decoder_common.cuh), so the gradient belongs to exactly the
+// output the forward produced.  All of them are HBM / L2-atomic bound; there is no tensor-core work here.
 //
-// f2 and f3 scatter into the gradient of the gathered tensor with float atomics (not bit-reproducible); their other
-// gradients are reduced in a fixed order and written once.  f4 uses no atomics at all: a per-pixel pass writes the mask
-// gradient and 18 per-tap partials, a second pass gathers the flow gradient from them in tap order.
+// f2, f3, a6 and a7 scatter into the gradient of the gathered tensor with float atomics (not bit-reproducible); their
+// other gradients are reduced in a fixed order and written once.  f4 uses no atomics at all: a per-pixel pass writes the
+// mask gradient and 18 per-tap partials, a second pass gathers the flow gradient from them in tap order.
 #include "common.cuh"
 #include "decoder_common.cuh"
 
 namespace b200 {
 
-constexpr int DB_PTS = 32;       // f2 / f3: queries (pixels) per CTA on threadIdx.x
-constexpr int DB_LANES = 8;      // f2 / f3: at most this many channel lanes per query on threadIdx.y
+constexpr int DB_PTS = 32;       // f2 / f3 / a6 cf / a7: queries (pixels, points, columns) per CTA on threadIdx.x
+constexpr int DB_LANES = 8;      // f2 / f3 / a6 cf / a7: at most this many channel lanes per query on threadIdx.y
 
 static int channel_lanes(int C) { return C < DB_LANES ? (C < 1 ? 1 : C) : DB_LANES; }
 
@@ -172,6 +174,100 @@ backwarp2d_border_bwd_kernel(const float* __restrict__ x, const float* __restric
     }
     dflow[((size_t)b * 2 + 0) * HW + p] = mx ? tx_sum : 0.0f;
     dflow[((size_t)b * 2 + 1) * HW + p] = my ? ty_sum : 0.0f;
+}
+
+// a7 backward.  CTA = 32 points x blockDim.y channel lanes, the forward's taps (zero_sample / zero_taps) per point:
+//   dfeat[b,c,tap] += w_tap g_c for every in-image tap                (atomics)
+//   dxy[b,0,n] = sum_c g_c ((v01 - v00) wy0 + (v11 - v10) wy1),  dxy[b,1,n] = sum_c g_c ((v10 - v00) wx0 + (v11 - v01) wx1)
+// with out-of-image taps reading 0 and nothing clipped (ATen's grid_sampler_2d backward with zero padding); lane
+// partials summed in lane order and written once.  The normalise / un-normalise factors 2/(W-1) and (W-1)/2 cancel.
+// A point with no tap inside the image (far outside it, or a huge / non-finite coordinate) skips the channel loop and
+// gets dxy = 0.
+__global__ void __launch_bounds__(DB_PTS * DB_LANES)
+grid_sample_pts_bwd_kernel(const float* __restrict__ feat, const float* __restrict__ xy, const float* __restrict__ grad_out,
+                           float* __restrict__ dfeat, float* __restrict__ dxy, int C, int H, int W, int N) {
+    __shared__ float part[2][DB_LANES][DB_PTS];
+    const int b = blockIdx.y;
+    const int tx = threadIdx.x, lane = threadIdx.y, lanes = blockDim.y;
+    const int n = blockIdx.x * DB_PTS + tx;
+    const size_t plane = (size_t)H * W;
+    float sx = 0.0f, sy = 0.0f;
+    if (n < N) {
+        const ZeroSample s = zero_sample(__ldg(xy + ((size_t)b * 2 + 0) * N + n), __ldg(xy + ((size_t)b * 2 + 1) * N + n), H, W);
+        const Taps t = zero_taps(s, H, W);
+        if (t.o00 >= 0 || t.o01 >= 0 || t.o10 >= 0 || t.o11 >= 0) {
+            const float* fb = feat + (size_t)b * C * plane;
+            const float* g = grad_out + (size_t)b * C * N + n;
+            float* dfb = dfeat != nullptr ? dfeat + (size_t)b * C * plane : nullptr;
+            for (int c = lane; c < C; c += lanes) {
+                const float gc = __ldg(g + (size_t)c * N);
+                if (dfb != nullptr) {
+                    float* d = dfb + (size_t)c * plane;
+                    if (t.o00 >= 0) atomicAdd(d + t.o00, t.w00 * gc);
+                    if (t.o01 >= 0) atomicAdd(d + t.o01, t.w01 * gc);
+                    if (t.o10 >= 0) atomicAdd(d + t.o10, t.w10 * gc);
+                    if (t.o11 >= 0) atomicAdd(d + t.o11, t.w11 * gc);
+                }
+                if (dxy != nullptr) {
+                    const float* f = fb + (size_t)c * plane;
+                    const float v00 = t.o00 >= 0 ? __ldg(f + t.o00) : 0.0f;
+                    const float v01 = t.o01 >= 0 ? __ldg(f + t.o01) : 0.0f;
+                    const float v10 = t.o10 >= 0 ? __ldg(f + t.o10) : 0.0f;
+                    const float v11 = t.o11 >= 0 ? __ldg(f + t.o11) : 0.0f;
+                    sx += gc * ((v01 - v00) * s.wy0 + (v11 - v10) * s.wy1);
+                    sy += gc * ((v10 - v00) * s.wx0 + (v11 - v01) * s.wx1);
+                }
+            }
+        }
+    }
+    if (dxy == nullptr) return;                                           // uniform over the grid
+    part[0][lane][tx] = sx;
+    part[1][lane][tx] = sy;
+    __syncthreads();
+    if (lane != 0 || n >= N) return;
+    float tx_sum = 0.0f, ty_sum = 0.0f;
+    for (int l = 0; l < lanes; ++l) {
+        tx_sum += part[0][l][tx];
+        ty_sum += part[1][l][tx];
+    }
+    dxy[((size_t)b * 2 + 0) * N + n] = tx_sum;
+    dxy[((size_t)b * 2 + 1) * N + n] = ty_sum;
+}
+
+// a6 channel-first backward: ddata[b,c,j(i)] += grad_out[b,c,i], j = the forward's wrap_index of idx[b,i].  CTA = 32
+// output columns x blockDim.y channel lanes: the index is read once per column, grad_out rows are read coalesced.
+__global__ void __launch_bounds__(DB_PTS * DB_LANES)
+gather_cf_bwd_kernel(const float* __restrict__ grad_out, const int64_t* __restrict__ idx, float* __restrict__ ddata,
+                     int C, int N, int64_t I) {
+    const int b = blockIdx.y;
+    const int64_t i = (int64_t)blockIdx.x * DB_PTS + threadIdx.x;
+    if (i >= I) return;
+    const int64_t j = wrap_index(__ldg(idx + (size_t)b * I + i), N, nullptr);
+    const float* g = grad_out + (size_t)b * C * I + i;
+    float* d = ddata + (size_t)b * C * N + j;
+    for (int c = threadIdx.y; c < C; c += blockDim.y) atomicAdd(d + (size_t)c * N, __ldg(g + (size_t)c * I));
+}
+
+// a6 channel-last backward: ddata[b,j(i),:] += grad_out[b,i,:].  One thread per 16-byte (VEC: one red.global.add.v4.f32)
+// or 4-byte element of a grad_out row, as in the forward.
+template <bool VEC>
+__global__ void __launch_bounds__(256)
+gather_cl_bwd_kernel(const float* __restrict__ grad_out, const int64_t* __restrict__ idx, float* __restrict__ ddata,
+                     int C, int N, int64_t I) {
+    const int b = blockIdx.y;
+    const int per_row = VEC ? C / 4 : C;
+    const int64_t e = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (e >= I * per_row) return;
+    const int64_t i = e / per_row;
+    const int c = (int)(e - i * per_row);
+    const int64_t j = wrap_index(__ldg(idx + (size_t)b * I + i), N, nullptr);
+    if (VEC) {
+        const float4 v = __ldg(reinterpret_cast<const float4*>(grad_out + ((size_t)b * I + i) * C) + c);
+        float* dst = ddata + ((size_t)b * N + j) * C + 4 * c;
+        asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
+    } else {
+        atomicAdd(ddata + ((size_t)b * N + j) * C + c, __ldg(grad_out + ((size_t)b * I + i) * C + c));
+    }
 }
 
 // f4 backward, pass 1: thread = low-res pixel (y, x), all s*s sub-pixels (i, j) in order.  With p_k the forward's softmax
@@ -358,5 +454,60 @@ extern "C" int b200_convex_upsample_bwd(const float* flow, const float* mask, co
         convex_upsample_bwd_pass2_kernel<<<grid, 256, 0, st>>>(P, dflow, H, W);
         B200_LAUNCH_CHECK("b200_convex_upsample_bwd(pass 2)");
     }
+    return B200_OK;
+}
+
+extern "C" int b200_grid_sample_pts_bwd(const float* feat, const float* xy, const float* grad_out, float* dfeat, float* dxy,
+                                        int B, int C, int H, int W, int N, b200_stream_t stream) {
+    using namespace b200;
+    const bool empty = B == 0 || C == 0 || N == 0;
+    B200_REQUIRE(empty || (feat && xy && grad_out), "b200_grid_sample_pts_bwd: null pointer");   // empty calls carry null pointers
+    B200_REQUIRE(B >= 0 && C >= 0 && H >= 1 && W >= 1 && N >= 0, "b200_grid_sample_pts_bwd: bad sizes");
+    B200_REQUIRE((int64_t)H * W < (1ll << 31) && B <= 65535, "b200_grid_sample_pts_bwd: plane or batch too large");
+    cudaStream_t st = as_stream(stream);
+    int rc;
+    if ((rc = zero_fill(dfeat, (size_t)B * C * H * W, st)) != B200_OK) return rc;
+    if (empty || !(dfeat || dxy)) return zero_fill(dxy, (size_t)B * 2 * N, st);      // C = 0: the point gradient is zero
+    const dim3 grid(ceil_div(N, DB_PTS), B), block(DB_PTS, channel_lanes(C));
+    grid_sample_pts_bwd_kernel<<<grid, block, 0, st>>>(feat, xy, grad_out, dfeat, dxy, C, H, W, N);
+    B200_LAUNCH_CHECK("b200_grid_sample_pts_bwd");
+    return B200_OK;
+}
+
+extern "C" int b200_gather_cf_bwd(const float* grad_out, const int64_t* idx, float* ddata, int B, int C, int N, int64_t I,
+                                  b200_stream_t stream) {
+    using namespace b200;
+    const bool empty = B == 0 || C == 0 || I == 0;
+    B200_REQUIRE(B == 0 || C == 0 || (ddata && (I == 0 || (grad_out && idx))), "b200_gather_cf_bwd: null pointer");
+    B200_REQUIRE(B >= 0 && C >= 0 && N >= 1 && I >= 0, "b200_gather_cf_bwd: bad sizes");
+    B200_REQUIRE(B <= 65535 && I <= ((1ll << 31) - 1) * DB_PTS, "b200_gather_cf_bwd: batch or index count exceeds the grid limit");
+    cudaStream_t st = as_stream(stream);
+    int rc;
+    if ((rc = zero_fill(ddata, (size_t)B * C * N, st)) != B200_OK) return rc;
+    if (empty) return B200_OK;
+    const dim3 grid(ceil_div(I, DB_PTS), B), block(DB_PTS, channel_lanes(C));
+    gather_cf_bwd_kernel<<<grid, block, 0, st>>>(grad_out, idx, ddata, C, N, I);
+    B200_LAUNCH_CHECK("b200_gather_cf_bwd");
+    return B200_OK;
+}
+
+extern "C" int b200_gather_cl_bwd(const float* grad_out, const int64_t* idx, float* ddata, int B, int C, int N, int64_t I,
+                                  b200_stream_t stream) {
+    using namespace b200;
+    const bool empty = B == 0 || C == 0 || I == 0;
+    B200_REQUIRE(B == 0 || C == 0 || (ddata && (I == 0 || (grad_out && idx))), "b200_gather_cl_bwd: null pointer");
+    B200_REQUIRE(B >= 0 && C >= 0 && N >= 1 && I >= 0, "b200_gather_cl_bwd: bad sizes");
+    B200_REQUIRE(B <= 65535 && (C == 0 || I <= ((1ll << 31) - 1) * 256 / C),
+                 "b200_gather_cl_bwd: batch or index count exceeds the grid limit");
+    cudaStream_t st = as_stream(stream);
+    int rc;
+    if ((rc = zero_fill(ddata, (size_t)B * N * C, st)) != B200_OK) return rc;
+    if (empty) return B200_OK;
+    const bool vec = (C % 4 == 0) && ((reinterpret_cast<uintptr_t>(grad_out) & 15) == 0) &&
+                     ((reinterpret_cast<uintptr_t>(ddata) & 15) == 0);
+    const dim3 grid(ceil_div(I * (vec ? C / 4 : C), 256), B);
+    if (vec) gather_cl_bwd_kernel<true><<<grid, 256, 0, st>>>(grad_out, idx, ddata, C, N, I);
+    else     gather_cl_bwd_kernel<false><<<grid, 256, 0, st>>>(grad_out, idx, ddata, C, N, I);
+    B200_LAUNCH_CHECK("b200_gather_cl_bwd");
     return B200_OK;
 }

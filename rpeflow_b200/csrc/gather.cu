@@ -19,15 +19,7 @@
 
 namespace b200 {
 
-__device__ __forceinline__ int64_t wrap_index(int64_t j, int N, int* bad) {
-    if (j < 0) j += N;                                   // python-style wrap of negative indices (torch.gather itself raises on them)
-    if (j < 0 || j >= N) {                               // torch would raise; we clamp and count (deliberate: see projection.py)
-        if (bad) atomicAdd(bad, 1);
-        j = j < 0 ? 0 : N - 1;
-    }
-    return j;
-}
-
+// wrap_index: decoder_common.cuh
 // out[b,c,i] = data[b,c,idx[b,i]]     grid: (ceil(I/256), csplit, B)
 __global__ void __launch_bounds__(256)
 gather_cf_kernel(const uint32_t* __restrict__ data, const int64_t* __restrict__ idx, uint32_t* __restrict__ out,
@@ -69,22 +61,7 @@ gather_cl_kernel(const uint32_t* __restrict__ data, const int64_t* __restrict__ 
     }
 }
 
-// zero-padding taps (Taps, renorm_coord: decoder_common.cuh)
-__device__ __forceinline__ Taps make_taps(float x, float y, int H, int W) {
-    const float ix = renorm_coord(x, W), iy = renorm_coord(y, H);
-    const float fx = floorf(ix), fy = floorf(iy);
-    const float wx1 = ix - fx, wy1 = iy - fy, wx0 = (fx + 1.0f) - ix, wy0 = (fy + 1.0f) - iy;
-    // guard the float->int conversion against huge / non-finite coordinates (all taps invalid then)
-    const bool finite = fabsf(ix) < 1e9f && fabsf(iy) < 1e9f;
-    const int x0 = finite ? (int)fx : -2, y0 = finite ? (int)fy : -2, x1 = x0 + 1, y1 = y0 + 1;
-    const bool vx0 = x0 >= 0 && x0 < W, vx1 = x1 >= 0 && x1 < W, vy0 = y0 >= 0 && y0 < H, vy1 = y1 >= 0 && y1 < H;
-    Taps t;
-    t.o00 = (vy0 && vx0) ? y0 * W + x0 : -1; t.w00 = wx0 * wy0;
-    t.o01 = (vy0 && vx1) ? y0 * W + x1 : -1; t.w01 = wx1 * wy0;
-    t.o10 = (vy1 && vx0) ? y1 * W + x0 : -1; t.w10 = wx0 * wy1;
-    t.o11 = (vy1 && vx1) ? y1 * W + x1 : -1; t.w11 = wx1 * wy1;
-    return t;
-}
+// zero-padding taps: make_taps (decoder_common.cuh)
 __device__ __forceinline__ float blend(const float* __restrict__ plane, const Taps& t) {
     // same accumulation order as ATen's grid_sampler_2d (nw, ne, sw, se), out-of-image taps skipped
     float v = 0.0f;

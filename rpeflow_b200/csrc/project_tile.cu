@@ -48,7 +48,7 @@ constexpr int PT_MAX_TILES = 4095;                                             /
 static_assert(PT_STAGE % 128 == 0, "TMA destinations stay 128-byte aligned");
 static_assert(PT_QX * PT_TH == PT_CONSUMERS, "one quad per consumer thread");
 
-// ---- bilinear taps as (x0, y0) + weights: the arithmetic of gather.cu::make_taps -----------------------------------
+// ---- bilinear taps as (x0, y0) + weights: the arithmetic of decoder_common.cuh::make_taps-------------------------------
 struct TapXY {
     int x0, y0;                  // top-left tap; -2^30 when the coordinate is not finite (all taps invalid)
     float w00, w01, w10, w11;

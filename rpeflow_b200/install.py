@@ -37,7 +37,11 @@ reference.  ``train`` is a collection of op names from ``TRAINABLE``:
   backward has no atomics, so this one also trains here under deterministic mode;
 - "correlation2d" (lowercase, like the function): ``ops.Correlation2dNCHWFunction``, b200_corr2d_fwd_nchw / b200_corr2d_bwd_nchw on the model's NCHW maps
   with no permutes (other displacements: b200_corr2d_fwd / b200_corr2d_bwd).  No atomics either: it also trains under
-  deterministic mode.
+  deterministic mode;
+- "grid_sample_wrapper": ``projection.GridSampleFunction``, b200_grid_sample_pts / b200_grid_sample_pts_bwd;
+- "batch_indexing_channel_first" / "batch_indexing_channel_last": ``projection.BatchIndexingChannelFirstFunction`` /
+  ``BatchIndexingChannelLastFunction``, b200_gather_cf / b200_gather_cf_bwd and b200_gather_cl / b200_gather_cl_bwd
+  (4-byte data only: gathers of 2-byte data keep going to the reference).
 A call takes the train route when it needs a graph, its op is in ``train``, every floating tensor is CUDA fp32 and its
 arguments are inside what the kernels were built for; ``stats()`` counts it as "b200".  ``train=True`` means
 {"Correlation3D"}.
@@ -61,7 +65,8 @@ _ADDED_MODULES = []    # sys.modules keys registered by install()
 _STATS = {}
 _OBSERVER = None
 _TRAIN = frozenset()   # ops whose calls that need a graph run this library's autograd Functions (install(train=...))
-TRAINABLE = ("Correlation3D", "PointConv", "knn_interpolation", "backwarp_2d", "convex_upsample", "correlation2d")
+TRAINABLE = ("Correlation3D", "PointConv", "knn_interpolation", "backwarp_2d", "convex_upsample", "correlation2d",
+             "grid_sample_wrapper", "batch_indexing_channel_first", "batch_indexing_channel_last")
 
 
 def stats(reset=False):
@@ -362,11 +367,14 @@ def patch_python_ops(patch_events=True, only=None):
                                              furthest_point_sampling_ok),
         "batch_indexing_channel_first": _dispatch(
             "batch_indexing_channel_first", projection.batch_indexing_channel_first, ref["batch_indexing_channel_first"],
-            lambda batched_data, batched_indices: batched_data.dim() == 3 and four_byte(batched_data, batched_indices)),
+            lambda batched_data, batched_indices: batched_data.dim() == 3 and four_byte(batched_data, batched_indices),
+            train="batch_indexing_channel_first"),
         "batch_indexing_channel_last": _dispatch(
             "batch_indexing_channel_last", projection.batch_indexing_channel_last, ref["batch_indexing_channel_last"],
-            lambda batched_data, batched_indices: batched_data.dim() in (2, 3) and four_byte(batched_data, batched_indices)),
-        "grid_sample_wrapper": _dispatch("grid_sample_wrapper", projection.grid_sample_wrapper, ref["grid_sample_wrapper"]),
+            lambda batched_data, batched_indices: batched_data.dim() in (2, 3) and four_byte(batched_data, batched_indices),
+            train="batch_indexing_channel_last"),
+        "grid_sample_wrapper": _dispatch("grid_sample_wrapper", projection.grid_sample_wrapper, ref["grid_sample_wrapper"],
+                                         train="grid_sample_wrapper"),
         "project_feat_with_nn_corr": _dispatch("project_feat_with_nn_corr", projection.project_feat_with_nn_corr,
                                                ref["project_feat_with_nn_corr"]),
         "knn_interpolation": _dispatch("knn_interpolation", knn_interpolation, ref["knn_interpolation"],
@@ -418,7 +426,8 @@ def install(patch_python=True, patch_events=False, only=None, extensions=True, t
     """train: the ops whose calls that need an autograd graph run this library's forward and backward instead of the
     reference's torch code — a collection of names from TRAINABLE ("Correlation3D": pwc3d.Correlation3DFunction;
     "PointConv": pointconv.PointConvFunction under the module's own norm and activation; "knn_interpolation" (with
-    backwarp_3d), "backwarp_2d", "convex_upsample": the projection module's autograd Functions; "correlation2d":
+    backwarp_3d), "backwarp_2d", "convex_upsample", "grid_sample_wrapper", "batch_indexing_channel_first",
+    "batch_indexing_channel_last": the projection module's autograd Functions; "correlation2d":
     ops.Correlation2dNCHWFunction).  True means
     {"Correlation3D"}; False (the default) routes every such call to the reference."""
     global _TRAIN

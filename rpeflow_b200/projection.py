@@ -2,9 +2,13 @@
 
 Same signatures and return shapes as ``batch_indexing_channel_first`` (:119-137), ``batch_indexing_channel_last``
 (:101-116), ``grid_sample_wrapper`` (:288-294) and ``project_feat_with_nn_corr`` (:297-317); each is one or two
-sm_100a kernels behind include/b200flow.h.  Those are forward only: the reference calls the last two under
-``torch.no_grad()`` everywhere (RPEFlow_core.py:52,105,156; models/utils.py:297), and the gathers are used on
-index/geometry tensors.  When autograd needs a gradient through a gather, keep the torch version.
+sm_100a kernels behind include/b200flow.h.  The first three are differentiable like the reference's ``torch.gather``,
+advanced indexing and ``F.grid_sample``: when autograd needs a graph they go through
+``BatchIndexingChannelFirstFunction``, ``BatchIndexingChannelLastFunction`` and ``GridSampleFunction`` (the same
+forward kernel, bit for bit, and b200_gather_cf_bwd / b200_gather_cl_bwd / b200_grid_sample_pts_bwd); otherwise they
+run the forward kernel alone.  Their backwards scatter with float atomics and raise under
+``torch.use_deterministic_algorithms(True)``.  ``project_feat_with_nn_corr`` is forward only: the reference defines
+it under ``torch.no_grad()`` (models/utils.py:297).
 
 The decoder ops ``knn_interpolation`` / ``backwarp_3d`` (:140-169), ``backwarp_2d`` (:186-198) and ``convex_upsample``
 (:201-214) also have backwards.  Under ``torch.no_grad()``, or when no input requires grad, they run their forward
@@ -20,7 +24,8 @@ from ._lib import check, lib, require_dense
 
 __all__ = ["batch_indexing_channel_first", "batch_indexing_channel_last", "grid_sample_wrapper", "backwarp_2d", "convex_upsample",
            "project_feat_with_nn_corr", "knn_interpolation", "backwarp_3d", "KnnInterpolationFunction",
-           "Backwarp2dFunction", "ConvexUpsampleFunction"]
+           "Backwarp2dFunction", "ConvexUpsampleFunction", "BatchIndexingChannelFirstFunction",
+           "BatchIndexingChannelLastFunction", "GridSampleFunction"]
 
 
 def _stream(t):
@@ -73,26 +78,107 @@ def _raise_if_bad(counter, what, n):
             raise IndexError(f"rpeflow_b200.{what}: {bad} indices are out of range for a dimension of size {n}")
 
 
+def _gather_run(data, idx, channel_last):
+    """data [B,C,N] (or [B,N,C] when channel_last), idx [B,I] int64 -> [B,C,I] (or [B,I,C])."""
+    B, I = idx.shape
+    if channel_last:
+        _, N, C = data.shape
+        out, fn, what = torch.empty((B, I, C), dtype=data.dtype, device=data.device), lib.b200_gather_cl, "b200_gather_cl"
+    else:
+        _, C, N = data.shape
+        out, fn, what = torch.empty((B, C, I), dtype=data.dtype, device=data.device), lib.b200_gather_cf, "b200_gather_cf"
+    bad = _bad_counter(data.device)
+    with torch.cuda.device(data.device):
+        check(fn(data.data_ptr(), idx.data_ptr(), out.data_ptr(), B, C, N, I, bad.data_ptr() if bad is not None else None,
+                 _stream(data)), what)
+    _raise_if_bad(bad, "batch_indexing_channel_last" if channel_last else "batch_indexing_channel_first", N)
+    return out
+
+
+def _gather_forward(ctx, data, idx, channel_last):
+    what = "BatchIndexingChannelLastFunction" if channel_last else "BatchIndexingChannelFirstFunction"
+    _require_cuda(what, data, idx)
+    _refuse_nondeterministic("batch_indexing_channel_last" if channel_last else "batch_indexing_channel_first")
+    require_dense(what, data=data, idx=idx)
+    if data.dim() != 3 or idx.dim() != 2 or idx.shape[0] != data.shape[0]:
+        raise ValueError(f"{what}: needs data [B,{'N,C' if channel_last else 'C,N'}] and idx [B,I]")
+    ctx.save_for_backward(idx)
+    ctx.data_shape = data.shape
+    return _gather_run(data, idx, channel_last)
+
+
+def _gather_backward(ctx, grad_out, channel_last):
+    if not ctx.needs_input_grad[0]:
+        return None, None
+    idx, = ctx.saved_tensors
+    B, I = idx.shape
+    if channel_last:
+        _, N, C = ctx.data_shape
+        fn, what = lib.b200_gather_cl_bwd, "b200_gather_cl_bwd"
+    else:
+        _, C, N = ctx.data_shape
+        fn, what = lib.b200_gather_cf_bwd, "b200_gather_cf_bwd"
+    g = grad_out.contiguous().float()
+    ddata = torch.empty(ctx.data_shape, dtype=torch.float32, device=idx.device)
+    with torch.cuda.device(idx.device):
+        check(fn(g.data_ptr(), idx.data_ptr(), ddata.data_ptr(), B, C, N, I, _stream(idx)), what)
+    return ddata, None
+
+
+class BatchIndexingChannelFirstFunction(torch.autograd.Function):
+    """apply(data [B,C,N], idx [B,I]) -> [B,C,I]; contiguous CUDA fp32 data, int64 indices.  Forward is b200_gather_cf,
+    backward b200_gather_cf_bwd: a scatter-add into a zero-filled [B,C,N] at the element each output read (the
+    forward's wrap-and-clamp rule).  Only the indices and the data's shape are saved, never the data.  The scatter sums
+    with float atomics, so this raises under torch.use_deterministic_algorithms(True)."""
+
+    @staticmethod
+    def forward(ctx, data, idx):
+        return _gather_forward(ctx, data, idx, False)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_out):
+        return _gather_backward(ctx, grad_out, False)
+
+
+class BatchIndexingChannelLastFunction(torch.autograd.Function):
+    """apply(data [B,N,C], idx [B,I]) -> [B,I,C]: b200_gather_cl, backward b200_gather_cl_bwd (scatter-add of whole
+    rows); otherwise as BatchIndexingChannelFirstFunction."""
+
+    @staticmethod
+    def forward(ctx, data, idx):
+        return _gather_forward(ctx, data, idx, True)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_out):
+        return _gather_backward(ctx, grad_out, True)
+
+
+def _batch_indexing(data, idx, channel_last):
+    B = data.shape[0]
+    flat_idx = idx.view(B, idx.numel() // max(B, 1))
+    if _needs_graph(data):
+        fn = BatchIndexingChannelLastFunction if channel_last else BatchIndexingChannelFirstFunction
+        return fn.apply(data, flat_idx)
+    return _gather_run(data, flat_idx, channel_last)
+
+
 def batch_indexing_channel_first(batched_data, batched_indices):
-    """[B,C,N], [B,I1..Im] -> [B,C,I1..Im] (bit-exact move of 4-byte elements)."""
+    """[B,C,N], [B,I1..Im] -> [B,C,I1..Im] (bit-exact move of 4-byte elements).  Differentiable in the data
+    (BatchIndexingChannelFirstFunction) when autograd needs a graph."""
     assert batched_data.shape[0] == batched_indices.shape[0]
     data = _prep_data(batched_data, "batch_indexing_channel_first")
     if data.dim() != 3:
         raise RuntimeError("batch_indexing_channel_first expects data of shape [B,C,N]")
     idx = _prep_idx(batched_indices, data.device)
-    B, C, N = data.shape
-    I = idx.numel() // max(B, 1)
-    out = torch.empty((B, C, I), dtype=data.dtype, device=data.device)
-    bad = _bad_counter(data.device)
-    with torch.cuda.device(data.device):
-        check(lib.b200_gather_cf(data.data_ptr(), idx.data_ptr(), out.data_ptr(), B, C, N, I,
-                                 bad.data_ptr() if bad is not None else None, _stream(data)), "b200_gather_cf")
-    _raise_if_bad(bad, "batch_indexing_channel_first", N)
-    return out.view([B, C] + list(idx.shape[1:]))
+    B, C, _ = data.shape
+    return _batch_indexing(data, idx, False).view([B, C] + list(idx.shape[1:]))
 
 
 def batch_indexing_channel_last(batched_data, batched_indices):
-    """[B,N,C] (or [B,N]), [B,I1..Im] -> [B,I1..Im,C] (or [B,I1..Im])."""
+    """[B,N,C] (or [B,N]), [B,I1..Im] -> [B,I1..Im,C] (or [B,I1..Im]).  Differentiable in the data
+    (BatchIndexingChannelLastFunction) when autograd needs a graph."""
     assert batched_data.shape[0] == batched_indices.shape[0]
     data = _prep_data(batched_data, "batch_indexing_channel_last")
     flat = data.dim() == 2
@@ -101,14 +187,8 @@ def batch_indexing_channel_last(batched_data, batched_indices):
     if data.dim() != 3:
         raise RuntimeError("batch_indexing_channel_last expects data of shape [B,N,C] or [B,N]")
     idx = _prep_idx(batched_indices, data.device)
-    B, N, C = data.shape
-    I = idx.numel() // max(B, 1)
-    out = torch.empty((B, I, C), dtype=data.dtype, device=data.device)
-    bad = _bad_counter(data.device)
-    with torch.cuda.device(data.device):
-        check(lib.b200_gather_cl(data.data_ptr(), idx.data_ptr(), out.data_ptr(), B, C, N, I,
-                                 bad.data_ptr() if bad is not None else None, _stream(data)), "b200_gather_cl")
-    _raise_if_bad(bad, "batch_indexing_channel_last", N)
+    B, _, C = data.shape
+    out = _batch_indexing(data, idx, True)
     shape = [B] + list(idx.shape[1:])
     return out.view(shape) if flat else out.view(shape + [C])
 
@@ -155,17 +235,7 @@ class _SampleMemo:
 SAMPLE_MEMO = _SampleMemo()
 
 
-def grid_sample_wrapper(feat_2d, xy):
-    """feat_2d [B,C,H,W], xy [B,2,N] (pixels) -> [B,C,N]; bilinear, align_corners=True, zero padding.
-    If project_feat_with_nn_corr has just sampled this very map at these very points, its result is returned
-    (see _SampleMemo) and no kernel runs."""
-    if not (feat_2d.is_cuda and xy.is_cuda):
-        raise RuntimeError("rpeflow_b200.grid_sample_wrapper: CUDA tensors required — no CPU/torch fallback")
-    parked = SAMPLE_MEMO.take(feat_2d, xy)
-    if parked is not None:
-        return parked
-    feat = feat_2d.contiguous().float()
-    pts = xy.contiguous().float()
+def _grid_sample_run(feat, pts):
     B, C, H, W = feat.shape
     N = pts.shape[2]
     out = torch.empty((B, C, N), dtype=torch.float32, device=feat.device)
@@ -173,6 +243,54 @@ def grid_sample_wrapper(feat_2d, xy):
         check(lib.b200_grid_sample_pts(feat.data_ptr(), pts.data_ptr(), out.data_ptr(), B, C, H, W, N,
                                        _stream(feat)), "b200_grid_sample_pts")
     return out
+
+
+class GridSampleFunction(torch.autograd.Function):
+    """apply(feat_2d [B,C,H,W], xy [B,2,N]), contiguous CUDA fp32.  Forward is b200_grid_sample_pts, backward
+    b200_grid_sample_pts_bwd (ATen's zero-padding gradients; a point with no tap inside the image gets a zero xy
+    gradient); gradients autograd does not ask for are not computed.  The map gradient is summed with float atomics,
+    so this raises under torch.use_deterministic_algorithms(True)."""
+
+    @staticmethod
+    def forward(ctx, feat_2d, xy):
+        _require_cuda("GridSampleFunction", feat_2d, xy)
+        _refuse_nondeterministic("grid_sample_wrapper")
+        require_dense("GridSampleFunction", feat_2d=feat_2d, xy=xy)
+        ctx.save_for_backward(feat_2d, xy)
+        return _grid_sample_run(feat_2d, xy)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_out):
+        feat, xy = ctx.saved_tensors
+        dfeat = torch.empty_like(feat) if ctx.needs_input_grad[0] else None
+        dxy = torch.empty_like(xy) if ctx.needs_input_grad[1] else None
+        if dfeat is None and dxy is None:
+            return None, None
+        B, C, H, W = feat.shape
+        N = xy.shape[2]
+        g = grad_out.contiguous().float()
+        with torch.cuda.device(feat.device):
+            check(lib.b200_grid_sample_pts_bwd(feat.data_ptr(), xy.data_ptr(), g.data_ptr(),
+                                               dfeat.data_ptr() if dfeat is not None else None,
+                                               dxy.data_ptr() if dxy is not None else None, B, C, H, W, N, _stream(feat)),
+                  "b200_grid_sample_pts_bwd")
+        return dfeat, dxy
+
+
+def grid_sample_wrapper(feat_2d, xy):
+    """feat_2d [B,C,H,W], xy [B,2,N] (pixels) -> [B,C,N]; bilinear, align_corners=True, zero padding.
+    Differentiable in both (GridSampleFunction) when autograd needs a graph.  Otherwise, if project_feat_with_nn_corr
+    has just sampled this very map at these very points, its result is returned (see _SampleMemo) and no kernel runs;
+    a call that needs a graph runs the kernel and leaves that parked result in place."""
+    if not (feat_2d.is_cuda and xy.is_cuda):
+        raise RuntimeError("rpeflow_b200.grid_sample_wrapper: CUDA tensors required — no CPU/torch fallback")
+    if _needs_graph(feat_2d, xy):
+        return GridSampleFunction.apply(feat_2d.contiguous().float(), xy.contiguous().float())
+    parked = SAMPLE_MEMO.take(feat_2d, xy)
+    if parked is not None:
+        return parked
+    return _grid_sample_run(feat_2d.contiguous().float(), xy.contiguous().float())
 
 
 def _backwarp2d_run(feat, flow):
