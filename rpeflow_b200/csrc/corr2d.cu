@@ -135,7 +135,7 @@ corr2d_fwd_kernel(const float* __restrict__ in1, const float* __restrict__ in2, 
         __syncthreads();                                 // everyone done with `cur` before it is refilled
     }
 
-    // epilogue: out[b, dyw*ND + d, y, x0 + lx*8 .. +7]
+    // epilogue: out[b, dyw*ND + d, y, x0 + lx*6 .. +5]
     const int y = y0 + ly, xs = x0 + lx * C2_PX;
     if (y >= H || xs >= W) return;
     const float fc = (float)C;
