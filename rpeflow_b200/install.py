@@ -211,14 +211,13 @@ def _pointconv_train(self, xyz, tensors):
 
 
 def _pointconv_weights(self):
-    """Weights for b200_pointconv_fwd, or None when the module is outside what the kernel was built for.  An eval-mode
-    BatchNorm1d after the Linear layer (the feature pyramid's norm, conf/test/things.yaml: pwc3d.norm.feature_pyramid) is
-    an affine map per output channel and is folded into the Linear weights."""
+    """Weights for b200_pointconv_fwd, or None when the module is outside what the kernel was built for: the body of
+    _pointconv_body_ok, then the module's own LeakyReLU(0.1), which the kernel applies.  An eval-mode BatchNorm1d after
+    the Linear layer (the feature pyramid's norm, conf/test/things.yaml: pwc3d.norm.feature_pyramid) is an affine map per
+    output channel and is folded into the Linear weights."""
     import torch.nn as nn
-    if self.k != 16 or self.linear.out_features > 256 or not isinstance(self.activation_fn, nn.LeakyReLU) \
+    if not _pointconv_body_ok(self) or not isinstance(self.activation_fn, nn.LeakyReLU) \
             or abs(self.activation_fn.negative_slope - 0.1) > 1e-12:
-        return None
-    if any(not isinstance(c.norm_fn, nn.Identity) or not isinstance(c.relu_fn, nn.LeakyReLU) for c in self.weight_net.convs):
         return None
     w = pointconv.pack_pointconv_weights(self)
     bn = self.norm_fn

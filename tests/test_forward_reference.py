@@ -8,9 +8,10 @@ below names the route it is meant to reach, read from the eligibility code of th
   and C % 32 == 0 with 32 <= C <= 192 (corr3d_v2_eligible; NW,DEPTH = 4,1 up to C = 128, 8,2 above); otherwise
   "tc<SPLIT>" = corr3d_stage1_tc_kernel at precision 1 (SPLIT 0) or 2 (SPLIT 1) when k = 16 and Cout % 32 == 0 with
   Cout <= 256 (corr3d_stage1_tc_eligible); otherwise "fp32<KMAX>" = corr3d_stage1_kernel<4/8/16/32> by k (launch_stage1).
-- PointConv (pointconv.cu b200_pointconv_fwd): "v2<MODE>" = pointconv_v2_kernel for N <= 65536: MODE 0 at precision 1
+- PointConv (pointconv.cu b200_pointconv_fwd): "v2<MODE,WIDE>" = pointconv_v2_kernel<MODE,WIDE>: MODE 0 at precision 1
   (TF32), MODE 1 at precisions 0 and 2 when roundup32(Cout) <= 128 (3xTF32, B halves stacked along N), MODE 2 above
-  (three MMAs, shallower ring); "legacy<SPLIT>" = pointconv_tc_kernel for N > 65536 (SPLIT = precision != 1).
+  (three MMAs, shallower ring); WIDE = N > 65536 (uint32 neighbour indices instead of uint16, which leave room for one
+  ring stage fewer at some widths: a single stage at MODE 2 with Cout = 256).
 test_every_case_reaches_its_route checks each claim against the kernels torch.profiler sees launched.
 
 Comparison.  Per sample b: max|got - ref| <= bar * max|ref| over that sample's outputs (normwise: fp32 sums of terms of
@@ -48,8 +49,9 @@ The bar is 2^-8, about 1.8 times that, and still 15 times below one lost neighbo
 
 Measured on a B200 at its 1000 W power limit (largest ratio per route and precision over every case of this file):
   Correlation3D  v2<4,1> p2 4.6e-6, v2<8,2> p2 5.3e-6, tc<1> p2 2.8e-6, tc<0> p1 2.3e-3, fp32<4/8/16/32> p0/p1/p2 9.3e-7
-  PointConv      v2<1> p0/p2 5.1e-5 (C = 509; 3.7e-6 up to C = 29), v2<2> p0/p2 7.3e-5 (C = 509; 6.7e-6 at C = 30),
-                 legacy<1> p0/p2 6.9e-6, v2<0> p1 1.0e-3, legacy<0> p1 8.6e-4
+  PointConv      v2<1,false> p0/p2 5.1e-5 (C = 509; 3.7e-6 up to C = 29), v2<2,false> p0/p2 7.3e-5 (C = 509; 6.7e-6 at
+                 C = 30), v2<1,true> p0/p2 4.6e-6 (C = 29), v2<2,true> p0/p2 7.1e-6 (C = 30), v2<0,false> p1 1.0e-3,
+                 v2<0,true> p1 9.0e-4
 
 Exact properties, bit for bit: a batched call equals the B single-sample calls (at the benchmark's batch of 148, where
 every persistent v2 CTA runs dozens of items); b200_pointconv_fwd equals LeakyReLU(0.1) of b200_pointconv_fwd_linear;
@@ -72,7 +74,7 @@ from test_backward_reference import DEV, _indices, _poison_allocator, _uniform, 
 
 FP32_BAR = 2e-5
 TF32_BAR = 2.0 ** -8
-TF32_ROUTES = {("corr3d", "tc<0>"), ("pointconv", "v2<0>"), ("pointconv", "legacy<0>")}
+TF32_ROUTES = {("corr3d", "tc<0>"), ("pointconv", "v2<0,false>"), ("pointconv", "v2<0,true>")}
 MEASURED = {}                                           # (op, route, precision) -> largest ratio seen
 
 
@@ -159,10 +161,11 @@ for _kind in ("same", "dups", "edges"):           # same: every neighbour is the
     C3_CASES[f"{_kind}_C32"] = ((3, 32, 32, 150, 200, 16), _kind, {0: "fp32<16>", 1: "tc<0>", 2: "v2<4,1>"})
     C3_CASES[f"{_kind}_k5_Cout5"] = ((3, 8, 5, 60, 40, 5), _kind, {0: "fp32<8>"})
 
-# PointConv, v2 route (N <= 65536).  name: ((B, C, Cout, N, S), neighbour kind, 3xTF32 MODE at precisions 0 and 2).
+# PointConv, uint16 neighbour indices (N <= 65536).  name: ((B, C, Cout, N, S), neighbour kind, 3xTF32 MODE at precisions
+# 0 and 2).
 # A CTA takes 120 sampled points (S = 119 / 120 / 121 / 241); channels are padded to Cp = roundup16(C+3) (C = 0 / 13 / 14 /
 # 29 / 30 / 195 / 509 -> Cp = 16 / 16 / 32 / 32 / 48 / 208 / 512), out_channels to Npad = roundup32(Cout) (MODE 2 and the
-# shallower ring above 128).  N = 65536 is the largest cloud of this route; its uint16 neighbour table holds 65535.
+# shallower ring above 128).  N = 65536 is the largest cloud of these; its uint16 neighbour table holds 65535.
 PC_CASES = {
     "S1_C0_Cout1": ((3, 0, 1, 50, 1), "random", 1),
     "S119_C13_Cout31": ((3, 13, 31, 300, 119), "random", 1),
@@ -179,19 +182,23 @@ for _kind in ("same", "dups", "edges"):
     PC_CASES[f"{_kind}_Cout129"] = ((3, 24, 129, 300, 241), _kind, 2)
     PC_CASES[f"{_kind}_Cout64"] = ((3, 24, 64, 300, 130), _kind, 1)
 
-# PointConv, legacy route (N > 65536, b200_pointconv_fwd only): 64 points per CTA.
-PC_LEGACY = {
-    "N65537_S63_C30": ((2, 30, 256, 65537, 63), "random"),
-    "N65537_S64_C13": ((2, 13, 256, 65537, 64), "edges"),
-    "N65537_S65_C0": ((2, 0, 256, 65537, 65), "dups"),
+# PointConv, uint32 neighbour indices (N > 65536, b200_pointconv_fwd only; "edges" reaches index 65536).  Cout = 256: MODE 2
+# on a one-stage ring, MODE 0 on three stages; Cout = 128: MODE 1 on two stages, MODE 0 on four.
+PC_WIDE = {
+    "N65537_S63_C30": ((2, 30, 256, 65537, 63), "random", 2),
+    "N65537_S64_C13": ((2, 13, 256, 65537, 64), "edges", 2),
+    "N65537_S65_C0": ((2, 0, 256, 65537, 65), "dups", 2),
+    "N65537_S121_C29_Cout128": ((2, 29, 128, 65537, 121), "edges", 1),
 }
 
 
-def _pc_routes(mode):
-    return {0: f"v2<{mode}>", 1: "v2<0>", 2: f"v2<{mode}>"}
+def _pc_routes(mode, wide=False):
+    w = "true" if wide else "false"
+    return {0: f"v2<{mode},{w}>", 1: f"v2<0,{w}>", 2: f"v2<{mode},{w}>"}
 
 
-LEGACY_ROUTES = {0: "legacy<1>", 1: "legacy<0>", 2: "legacy<1>"}
+def _pc_case_routes(name):
+    return _pc_routes(PC_CASES[name][2]) if name in PC_CASES else _pc_routes(PC_WIDE[name][2], wide=True)
 
 
 @functools.lru_cache(maxsize=None)
@@ -203,7 +210,7 @@ def c3_case(name):
 
 @functools.lru_cache(maxsize=None)
 def pc_case(name):
-    shape, kind = (PC_CASES[name][:2] if name in PC_CASES else PC_LEGACY[name])
+    shape, kind, _ = PC_CASES[name] if name in PC_CASES else PC_WIDE[name]
     inputs, w, knn = pc_inputs(*shape, kind, _seed(name))
     return (inputs, w, knn) + pc_reference(inputs, w, knn)
 
@@ -305,7 +312,7 @@ def test_pointconv_forward_vs_float64(name, precision):
     """b200_pointconv_fwd and b200_pointconv_fwd_linear against the reference; the first is LeakyReLU(0.1) of the
     second bit for bit, and precision 0 is precision 2 bit for bit."""
     inputs, w, knn, ref, ref_linear = pc_case(name)
-    route = _pc_routes(PC_CASES[name][2])[precision]
+    route = _pc_case_routes(name)[precision]
     got = run_pointconv(inputs, w, knn, precision)
     pc_check(route, precision, got, ref, name, inputs)
     linear = run_pointconv(inputs, w, knn, precision, "b200_pointconv_fwd_linear")
@@ -315,16 +322,16 @@ def test_pointconv_forward_vs_float64(name, precision):
         assert torch.equal(got, run_pointconv(inputs, w, knn, 2)), f"{name}: precision 0 != precision 2"
 
 
-LEGACY_IDS = [(n, p) for n in PC_LEGACY for p in (0, 1, 2)]
+WIDE_IDS = [(n, p) for n in PC_WIDE for p in (0, 1, 2)]
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("name,precision", LEGACY_IDS, ids=[f"{n}-p{p}" for n, p in LEGACY_IDS])
-def test_pointconv_legacy_kernel_vs_float64(name, precision):
+@pytest.mark.parametrize("name,precision", WIDE_IDS, ids=[f"{n}-p{p}" for n, p in WIDE_IDS])
+def test_pointconv_wide_index_vs_float64(name, precision):
     """Clouds of more than 65536 points: b200_pointconv_fwd only (the _linear entry refuses them)."""
     inputs, w, knn, ref, _ = pc_case(name)
     got = run_pointconv(inputs, w, knn, precision)
-    pc_check(LEGACY_ROUTES[precision], precision, got, ref, name, inputs)
+    pc_check(_pc_case_routes(name)[precision], precision, got, ref, name, inputs)
     if precision == 0:
         assert torch.equal(got, run_pointconv(inputs, w, knn, 2)), f"{name}: precision 0 != precision 2"
     with pytest.raises(B200Error, match="N <= 65536"):
@@ -354,28 +361,31 @@ C3_ROUTE_KERNELS.update({f"tc<{s}>": {"pointwise_linear_kernel", f"corr3d_stage1
 C3_ROUTE_KERNELS.update({f"v2<{c}>": {"corr3d_v2_linear_kernel", f"corr3d_v2_stage1_kernel<{c}>", "corr3d_v2_stage2_kernel"}
                          for c in ("4,1", "8,2")})
 C3_PREP_KERNELS = {"corr3d_prep_weights", "corr3d_v2_prep_kernel", "corr3d_v2_prep_w1_kernel"}
-PC_ROUTE_KERNELS = {f"v2<{m}>": {"pointconv_v2_prep_kernel", f"pointconv_v2_kernel<{m}>"} for m in (0, 1, 2)}
-PC_ROUTE_KERNELS.update({f"legacy<{s}>": {"pointconv_prep_kernel", f"pointconv_tc_kernel<{s}>"} for s in (0, 1)})
+PC_ROUTE_KERNELS = {f"v2<{m},{w}>": {"pointconv_v2_prep_kernel", f"pointconv_v2_kernel<{m},{w}>"}
+                    for m in (0, 1, 2) for w in ("false", "true")}
 
 
 @pytest.mark.gpu
 def test_every_case_reaches_its_route():
-    """Each (case, precision) of the tables above launches the kernels of the route it claims, and no other route's."""
-    wrong = []
+    """Each (case, precision) of the tables above launches the kernels of the route it claims, and no other route's; the
+    PointConv cases launch every PointConv forward kernel and nothing else."""
+    wrong, seen = [], set()
     for name, (_, _, routes) in C3_CASES.items():
         inputs, w, knn12, knn11, _ = c3_case(name)
         for p, route in routes.items():
             got = _kernel_names(lambda: run_corr3d(inputs, w, knn12, knn11, p)) - C3_PREP_KERNELS
             if got != C3_ROUTE_KERNELS[route]:
                 wrong.append(f"corr3d {name} p{p}: claims {route}, launched {sorted(got)}")
-    for name in list(PC_CASES) + list(PC_LEGACY):
+    for name in list(PC_CASES) + list(PC_WIDE):
         inputs, w, knn, _, _ = pc_case(name)
-        routes = _pc_routes(PC_CASES[name][2]) if name in PC_CASES else LEGACY_ROUTES
-        for p, route in routes.items():
+        for p, route in _pc_case_routes(name).items():
             got = _kernel_names(lambda: run_pointconv(inputs, w, knn, p))
+            seen |= got
             if got != PC_ROUTE_KERNELS[route]:
                 wrong.append(f"pointconv {name} p{p}: claims {route}, launched {sorted(got)}")
     assert not wrong, "\n".join(wrong)
+    every = set().union(*PC_ROUTE_KERNELS.values())
+    assert seen == every, sorted(seen ^ every)
 
 
 # ------------------------------------------------------------------------------------------------- batch invariance
@@ -439,8 +449,7 @@ def test_corr3d_neighbour_order_does_not_matter(name):
 @pytest.mark.parametrize("name", ["S241_C30_Cout129", "S121_C29_Cout128", "N65537_S63_C30"])
 def test_pointconv_neighbour_order_does_not_matter(name):
     inputs, w, knn, ref, _ = pc_case(name)
-    routes = _pc_routes(PC_CASES[name][2]) if name in PC_CASES else LEGACY_ROUTES
-    for p, route in routes.items():
+    for p, route in _pc_case_routes(name).items():
         pc_check(route, p, run_pointconv(inputs, w, _permute_neighbours(knn, 3), p), ref, name + " permuted", inputs)
 
 
@@ -477,5 +486,4 @@ def test_pointconv_out_of_range_indices_wrap_once_then_clamp(name, precision):
     N = inputs["xyz"].shape[2]
     bad = _out_of_range(knn, N)
     ref, _ = pc_reference(inputs, w, torch.where(bad < 0, bad + N, bad).clamp(0, N - 1))
-    routes = _pc_routes(PC_CASES[name][2]) if name in PC_CASES else LEGACY_ROUTES
-    pc_check(routes[precision], precision, run_pointconv(inputs, w, bad, precision), ref, name + " out-of-range", inputs)
+    pc_check(_pc_case_routes(name)[precision], precision, run_pointconv(inputs, w, bad, precision), ref, name + " out-of-range", inputs)

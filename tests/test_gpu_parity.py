@@ -869,7 +869,7 @@ def test_pointconv_golden(golden, tag, precision, tol):
 
 
 @pytest.mark.parametrize("C,cout,N,S", [(32, 32, 8192, 4096), (64, 64, 4096, 2048), (192, 192, 512, 256), (35, 64, 300, 300),
-                                         (0, 16, 100, 37), (32, 64, 70000, 512)])     # N > 65536: pointconv_tc_kernel
+                                         (0, 16, 100, 37), (32, 64, 70000, 512)])     # N > 65536: uint32 indices
 def test_pointconv_modules_vs_oracle(C, cout, N, S):
     gen = torch.Generator().manual_seed(C + N)
     B = 2

@@ -111,6 +111,33 @@ def test_install_train_rejects_unknown_op_names():
         inst.install(train={"PointConv", "Correlation2D"})
 
 
+class _UpstreamConv(torch.nn.Module):
+    def __init__(self, cin, cout, slope):
+        super().__init__()
+        self.conv_fn, self.norm_fn, self.relu_fn = torch.nn.Conv2d(cin, cout, 1), torch.nn.Identity(), torch.nn.LeakyReLU(slope)
+
+
+class _UpstreamPointConv(torch.nn.Module):
+    """The attributes install reads from models/pointconv.py's PointConvDownSampling / PointConvNoSampling."""
+    def __init__(self, C, Cout, weight_net_slope):
+        super().__init__()
+        self.k = 16
+        self.weight_net = torch.nn.Module()
+        self.weight_net.convs = torch.nn.ModuleList([_UpstreamConv(3, 8, weight_net_slope), _UpstreamConv(8, 16, weight_net_slope)])
+        self.linear = torch.nn.Linear(16 * (C + 3), Cout)
+        self.norm_fn, self.activation_fn = torch.nn.Identity(), torch.nn.LeakyReLU(0.1)
+
+
+@pytest.mark.parametrize("slope,accepted", [(0.1, True), (0.2, False)])
+def test_install_takes_only_the_kernels_weight_net_slope(slope, accepted):
+    """The kernels apply LeakyReLU(0.1) inside the weight net: a module whose weight net uses another slope is refused by
+    the inference route (_pointconv_weights) and the training route (_pointconv_body_ok) alike, so it runs the reference."""
+    import rpeflow_b200.install as inst
+    mod = _UpstreamPointConv(8, 32, slope)
+    assert inst._pointconv_body_ok(mod) is accepted
+    assert (inst._pointconv_weights(mod) is not None) is accepted
+
+
 # ------------------------------------------------------------------------------------------------- GPU helpers
 def _cloud(B, N, gen, dup):
     if not dup:
