@@ -378,7 +378,7 @@ B200_API int b200_corr3d_fwd(const float* xyz1, const float* feat1, const float*
  * Only the 3->8->8 part of weight_net1 (n1_Wa, n1_ba, n1_Wb, n1_bb) is bit-reproducible from run to run.  Every other
  * gradient depends on float-atomic sums whose order varies: dP, dG2, the clouds, the split-K dW1 / db1, and the
  * per-CTA shared-memory sums of the weight-net output layers, W1's xyz columns and b2.  No host synchronisation, no
- * allocation.
+ * allocation.  b200_corr3d_bwd_det below computes the same gradients without float atomics.
  */
 typedef struct b200_corr3d_grads {
     float *xyz1, *feat1, *xyz2, *feat2;
@@ -389,6 +389,33 @@ typedef struct b200_corr3d_grads {
 
 B200_API int64_t b200_corr3d_bwd_scratch_floats(int B, int Cin, int Cout, int N1, int N2, int k);
 B200_API int b200_corr3d_bwd(const float* xyz1, const float* feat1, const float* xyz2, const float* feat2,
+                    const int64_t* knn12, const int64_t* knn11, const b200_corr3d_weights* w,
+                    const float* grad_out, const float* fwd_scratch, const b200_corr3d_grads* grads, float* scratch,
+                    int B, int Cin, int Cout, int N1, int N2, int k, b200_stream_t stream);
+
+/* a5 backward without float atomics: the same arguments, checks and outputs as b200_corr3d_bwd, except
+ *   scratch : >= b200_corr3d_bwd_det_scratch_bytes(B,Cin,Cout,N1,N2,k) BYTES, 16-byte aligned, allocated by the caller.
+ *             It holds b200_corr3d_bwd's scratch, a row buffer of B*N1*k*((Cout+3)&~3) floats (dP rows, then dz1 rows),
+ *             B*N1*k float4 offset-gradient rows, the inverse index lists of knn11 and knn12 and the sort's workspace.
+ *             The size function needs a CUDA device (it asks cub for the sort's workspace); it returns a negative value
+ *             and sets b200_last_error() when that fails.  B*N1*k and B*N2 must be below 2^31.
+ * Sum-order contract.  Every output is the same, bit for bit, on every run, whatever the scheduling of the CTAs and
+ * whatever else runs on the device.  The four input gradients (xyz1, feat1, xyz2, feat2) of a sample do not depend on
+ * the other samples of the batch.  Indices are first clamped as the forward clamps them (m < 0 -> 0, m >= N -> N-1).
+ * Every gradient that b200_corr3d_bwd scatters over the knn rows (dP and dxyz1 over knn11; dG2, hence feat2 and W1's
+ * feat2 columns, and dxyz2 over knn12) is, for each element, a sum over the rows r = i*k + s that point at it, taken
+ * in ascending r and added in fp32 starting from +0.0.  Each dxyz1[i] is
+ *     ((sum of the pulled +de rows of knn11, ascending r) - (own de over s, ascending s)) - (own t over s, ascending s)
+ * with e = xyz1[m] - xyz1[i] (weight_net1) and t = dd + de the offset gradient of d = xyz2[j] - xyz1[i] (cost_mlp
+ * layer 1 and weight_net2).  Weight gradients are fixed-order sums of per-tile, per-warp and per-split partials, so
+ * they are reproducible but, like the atomic path's, depend on the whole batch.  No sum order depends on which
+ * gradients are requested: a call that asks for a subset returns the same bits as a call that asks for all of them.
+ * Sequence: knn11 / knn12 inverted (cub::DeviceRadixSort on key b*N + index, stable) -> pass 1 -> pull over knn11
+ * (dP, dxyz1) -> pass 2 -> pull over knn12 (dG2, dxyz2) -> per-CTA partial sums -> linear backward (split-K partials
+ * summed in ascending split order).  No host synchronisation, no allocation.
+ */
+B200_API int64_t b200_corr3d_bwd_det_scratch_bytes(int B, int Cin, int Cout, int N1, int N2, int k);
+B200_API int b200_corr3d_bwd_det(const float* xyz1, const float* feat1, const float* xyz2, const float* feat2,
                     const int64_t* knn12, const int64_t* knn11, const b200_corr3d_weights* w,
                     const float* grad_out, const float* fwd_scratch, const b200_corr3d_grads* grads, float* scratch,
                     int B, int Cin, int Cout, int N1, int N2, int k, b200_stream_t stream);

@@ -87,6 +87,9 @@ SIGNATURES = {
     "b200_corr3d_bwd_scratch_floats": (c_i64, [c_i, c_i, c_i, c_i, c_i, c_i]),
     "b200_corr3d_bwd": (c_i, [c_p, c_p, c_p, c_p, c_p, c_p, ctypes.POINTER(Corr3dWeights), c_p, c_p,
                               ctypes.POINTER(Corr3dGrads), c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_p]),
+    "b200_corr3d_bwd_det_scratch_bytes": (c_i64, [c_i, c_i, c_i, c_i, c_i, c_i]),
+    "b200_corr3d_bwd_det": (c_i, [c_p, c_p, c_p, c_p, c_p, c_p, ctypes.POINTER(Corr3dWeights), c_p, c_p,
+                                  ctypes.POINTER(Corr3dGrads), c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_p]),
     "b200_event_voxel_int": (c_i, [c_p, c_i64, c_p, c_i, c_i, c_i, c_i, c_p, c_p]),
     "b200_event_voxel_trilinear": (c_i, [c_p, c_p, c_p, c_p, c_i64, c_p, c_i, c_i, c_i, c_i, c_p, c_p]),
 }
@@ -113,7 +116,7 @@ def _load():
 B200_ENOSUP = -3        # include/b200flow.h
 lib = _load()
 LAUNCHES = 0          # kernels of this library launched by this process (bench.py reports it as gpu_launches)
-KERNELS_PER_CALL = {"b200_knn_grid": 3, "b200_knn_grid_cf": 3, "b200_pointconv_fwd": 2, "b200_pointconv_fwd_linear": 2, "b200_pointconv_bwd": 6, "b200_corr2d_bwd": 2, "b200_project_nn_corr": 2, "b200_corr3d_fwd": 5, "b200_corr3d_bwd": 10, "b200_event_voxel_trilinear": 3,
+KERNELS_PER_CALL = {"b200_knn_grid": 3, "b200_knn_grid_cf": 3, "b200_pointconv_fwd": 2, "b200_pointconv_fwd_linear": 2, "b200_pointconv_bwd": 6, "b200_corr2d_bwd": 2, "b200_project_nn_corr": 2, "b200_corr3d_fwd": 5, "b200_corr3d_bwd": 10, "b200_corr3d_bwd_det": 26, "b200_event_voxel_trilinear": 3,
                     "b200_knn_interpolate_bwd": 1, "b200_backwarp2d_bwd": 1, "b200_corr2d_bwd_nchw": 2, "b200_convex_upsample_bwd": 2, "b200_fps_large": 5,
                     "b200_grid_sample_pts_bwd": 1, "b200_gather_cf_bwd": 1, "b200_gather_cl_bwd": 1}
 

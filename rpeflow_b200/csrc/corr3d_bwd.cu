@@ -20,7 +20,22 @@
 // then one fixed-order sum over the CTAs' partials.  The partials themselves are not reproducible: dP, dG2, dxyz and the
 // split-K dW1a/dW1b/db1 use global float atomics, and the Wc/bc, W1c and b2 partials shared-memory float atomics; every
 // stage-1 gradient reads dP.  Only the weight_net1 3->8->8 gradients (thread-owned sums) are bit-reproducible.
+//
+// b200_corr3d_bwd_det runs the same passes with DET = true and no float atomics anywhere:
+//   - knn11 and knn12 are inverted first: rows r = (b*N1 + i)*k + s sorted by key b*N + clamp(idx) (cub radix sort,
+//     stable, so ascending r inside a destination) and segment offsets per destination (CSR);
+//   - pass 1 writes the dP rows relu(vpre)*g_i and the de rows to row buffers; its Wc / bc partials go to per-warp slices
+//     (CTA-owned scratch, read-modify-write) summed in warp order;
+//   - corr3d_det_pull_kernel sums, per destination, its rows in ascending r: dP and dxyz1 (minus the point's own de rows
+//     in ascending s) over knn11, then after pass 2 dG2 and dxyz2 over knn12;
+//   - pass 2 writes dz1 rows (into the buffer that held the dP rows) and t = dd + de rows; du2, the Wc / bc / b2 and W1c
+//     partials are per-tile reductions in ascending row order; the point's own -t, summed in ascending s, is subtracted
+//     from dxyz1 by the one CTA that owns the point;
+//   - pass 4 writes its split-K partials to scratch and linear_bwd_w_reduce_kernel sums them in ascending split order.
 #include <algorithm>
+#include <climits>
+
+#include <cub/device/device_radix_sort.cuh>
 
 #include "corr3d_common.cuh"
 
@@ -70,6 +85,13 @@ static inline BwdScratch carve_bwd(float* base, int B, int Cout, int N1, int N2)
     s.total = off;
     return s;
 }
+
+// Row buffers of the deterministic path (passed last, so the DET = false kernels keep their parameter layout).
+struct DetRows {
+    float* rows;        // [B*N1*k][c4of(C)]: pass 1 dP rows, pass 2 dz1 rows; NULL = not needed
+    float4* xrows;      // [B*N1*k]: pass 1 de, pass 2 t = dd + de (w = 0); NULL = not needed
+    float* wslice;      // pass 1: [CTA][warp][9][C] Wc (8 rows) and bc partials
+};
 
 // ---- device helpers -------------------------------------------------------------------------------------------
 __device__ __forceinline__ float lrelu_d(float pre) { return pre > 0.0f ? 1.0f : 0.1f; }     // torch: slope where x <= 0
@@ -155,13 +177,15 @@ __device__ __forceinline__ void wn_small_flush(float* part_small, float acc, flo
 // ---- pass 1: stage-2 backward --------------------------------------------------------------------------------
 // Tile = 16 points x k rows.  Warp w owns points w and w+8; its lanes walk the channels.
 // Dynamic smem: Gs[C][17] | u1[rows][8] | u2[rows][8] | e[rows][4] | du2[rows][8] | du1[rows][8] | jj[rows] | sWc[C][9]
+// DET: dP rows and de rows go to det.rows / det.xrows (dP, dxyz1 only flag what is needed), sWc is replaced by det.wslice.
 constexpr int S2_TP = 16;
+template <bool DET>
 __global__ void __launch_bounds__(BWD_THREADS)
 corr3d_bwd_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restrict__ knn11, const float* __restrict__ P,
                          const float* __restrict__ G, const float* __restrict__ Wa, const float* __restrict__ ba,
                          const float* __restrict__ Wb, const float* __restrict__ bb, const float* __restrict__ Wc,
                          const float* __restrict__ bc, float* __restrict__ dP, float* __restrict__ dxyz1,
-                         float* __restrict__ part, int64_t part_stride, int B, int C, int N1, int k, int small) {
+                         float* __restrict__ part, int64_t part_stride, int B, int C, int N1, int k, int small, DetRows det) {
     extern __shared__ float4 smem_f4[];
     float* Gs = reinterpret_cast<float*>(smem_f4);
     const int rows = S2_TP * k;
@@ -177,11 +201,18 @@ corr3d_bwd_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restri
     const PartLayout L = part_layout(C);
     float* mypart = part + (size_t)blockIdx.x * part_stride;
 
-    for (int e = tid; e < C * 9; e += BWD_THREADS) sWc[e] = 0.0f;
+    float* wslice = nullptr;                                          // DET: this warp's [9][C] Wc / bc slice
+    if constexpr (DET) {
+        wslice = det.wslice + ((size_t)blockIdx.x * (BWD_THREADS / 32) + warp) * 9 * C;
+        for (int e = lane; e < C * 9; e += 32) wslice[e] = 0.0f;
+    } else {
+        for (int e = tid; e < C * 9; e += BWD_THREADS) sWc[e] = 0.0f;
+    }
     float small_acc = 0.0f;
     const int tiles_per_b = (N1 + S2_TP - 1) / S2_TP;
     for (int tile = blockIdx.x; tile < B * tiles_per_b; tile += gridDim.x) {
         const int b = tile / tiles_per_b, i0 = (tile - b * tiles_per_b) * S2_TP;
+        const size_t row0 = ((size_t)b * N1 + i0) * k;                // global row of the tile's row 0
         __syncthreads();
         for (int e = tid; e < C * S2_TP; e += BWD_THREADS) {          // grad_out tile, coalesced over points
             const int o = e / S2_TP, pt = e - o * S2_TP;
@@ -219,7 +250,11 @@ corr3d_bwd_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restri
 #pragma unroll
                     for (int q = 0; q < 8; ++q) vpre = fmaf(wc[q], u2[q], vpre);
                     const float pm = ok ? __ldg(P + ((size_t)b * N1 + m) * C + o) : 0.0f;
-                    if (dP != nullptr && ok) atomicAdd(dP + ((size_t)b * N1 + m) * C + o, fmaxf(vpre, 0.0f) * g);
+                    if constexpr (DET) {
+                        if (dP != nullptr && ok) det.rows[(row0 + r) * c4of(C) + o] = fmaxf(vpre, 0.0f) * g;
+                    } else {
+                        if (dP != nullptr && ok) atomicAdd(dP + ((size_t)b * N1 + m) * C + o, fmaxf(vpre, 0.0f) * g);
+                    }
                     const float dvpre = vpre > 0.0f ? g * pm : 0.0f;
                     float du2[8];
 #pragma unroll
@@ -231,9 +266,15 @@ corr3d_bwd_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restri
                     }
                 }
                 if (ok) {
+                    if constexpr (DET) {
 #pragma unroll
-                    for (int q = 0; q < 8; ++q) atomicAdd(sWc + o * 9 + q, gw[q]);
-                    atomicAdd(sWc + o * 9 + 8, gb);
+                        for (int q = 0; q < 8; ++q) wslice[q * C + o] += gw[q];
+                        wslice[8 * C + o] += gb;
+                    } else {
+#pragma unroll
+                        for (int q = 0; q < 8; ++q) atomicAdd(sWc + o * 9 + q, gw[q]);
+                        atomicAdd(sWc + o * 9 + 8, gb);
+                    }
                 }
             }
         }
@@ -248,11 +289,15 @@ corr3d_bwd_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restri
 #pragma unroll
             for (int q = 0; q < 8; ++q) { du2s[r * 8 + q] = du2[q]; du1s[r * 8 + q] = du1[q]; }
             if (dxyz1 != nullptr && i < N1) {
-                const int m = jj[r];
+                if constexpr (DET) {
+                    det.xrows[row0 + r] = make_float4(de[0], de[1], de[2], 0.0f);
+                } else {
+                    const int m = jj[r];
 #pragma unroll
-                for (int x = 0; x < 3; ++x) {
-                    atomicAdd(dxyz1 + ((size_t)b * 3 + x) * N1 + m, de[x]);
-                    atomicAdd(dxyz1 + ((size_t)b * 3 + x) * N1 + i, -de[x]);
+                    for (int x = 0; x < 3; ++x) {
+                        atomicAdd(dxyz1 + ((size_t)b * 3 + x) * N1 + m, de[x]);
+                        atomicAdd(dxyz1 + ((size_t)b * 3 + x) * N1 + i, -de[x]);
+                    }
                 }
             }
         }
@@ -264,23 +309,36 @@ corr3d_bwd_stage2_kernel(const float* __restrict__ xyz1, const int64_t* __restri
         }
     }
     wn_small_flush(mypart + L.n1s, small_acc, s_tmp, tid);
-    for (int e = tid; e < C * 9; e += BWD_THREADS) {
-        const int o = e / 9, q = e - o * 9;
-        if (q < 8) mypart[L.n1Wc + o * 8 + q] = sWc[e];
-        else mypart[L.n1bc + o] = sWc[e];
+    if constexpr (DET) {
+        const float* cta = det.wslice + (size_t)blockIdx.x * (BWD_THREADS / 32) * 9 * C;
+        for (int e = tid; e < C * 9; e += BWD_THREADS) {
+            const int q = e / C, o = e - q * C;
+            float s = 0.0f;
+            for (int w = 0; w < BWD_THREADS / 32; ++w) s += cta[(size_t)w * 9 * C + e];
+            if (q < 8) mypart[L.n1Wc + o * 8 + q] = s;
+            else mypart[L.n1bc + o] = s;
+        }
+    } else {
+        for (int e = tid; e < C * 9; e += BWD_THREADS) {
+            const int o = e / 9, q = e - o * 9;
+            if (q < 8) mypart[L.n1Wc + o * 8 + q] = sWc[e];
+            else mypart[L.n1bc + o] = sWc[e];
+        }
     }
 }
 
 // ---- pass 2: stage-1 backward --------------------------------------------------------------------------------
 // Tile = TP points x k rows (TP*k <= 128).  Dynamic smem:
 //   h1[rows][LD] (later dz1) | dz2[rows][LD] | u1[rows][8] | u2[rows][8] | d[rows][4] | du2[rows][8] | du1[rows][8] |
-//   dd[rows][4] | jj[rows] | sWc[C][9] | sW1c[C][3] | sb2[C]
-static inline size_t s1_smem(int tp, int k, int C) {
+//   dd[rows][4] | jj[rows] | sWc[C][9] | sW1c[C][3] | sb2[C] | DET: dw[rows][LD] (dwpre, the weight_net2 output gradient)
+static inline size_t s1_smem(int tp, int k, int C, bool det) {
     const size_t r = (size_t)tp * k, LD = c4of(C) + 4;
-    return (2 * r * LD + r * (8 + 8 + 4 + 8 + 8 + 4 + 1) + (size_t)C * 13) * sizeof(float);
+    return ((det ? 3 : 2) * r * LD + r * (8 + 8 + 4 + 8 + 8 + 4 + 1) + (size_t)C * 13) * sizeof(float);
 }
 
-template <int KMAX>
+// DET: dz1 rows and t rows go to det.rows / det.xrows (dG2, dxyz2 only flag what is needed); du2 and the Wc / bc / b2 /
+// W1c partials are reduced per tile in ascending row order; dxyz1[i] -= (own t summed in ascending s), read-modify-write.
+template <int KMAX, bool DET>
 __global__ void __launch_bounds__(BWD_THREADS, 1)
 corr3d_bwd_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict__ xyz2, const int64_t* __restrict__ knn12,
                          const float* __restrict__ A1, const float* __restrict__ G2, const float* __restrict__ W2,
@@ -289,7 +347,7 @@ corr3d_bwd_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict
                          const float* __restrict__ bb, const float* __restrict__ WcT, const float* __restrict__ bc,
                          const float* __restrict__ dP, float* __restrict__ dA1, float* __restrict__ dG2,
                          float* __restrict__ dxyz1, float* __restrict__ dxyz2, float* __restrict__ part, int64_t part_stride,
-                         int B, int C, int N1, int N2, int k, int TP) {
+                         int B, int C, int N1, int N2, int k, int TP, DetRows det) {
     extern __shared__ float4 smem_f4[];
     float* smem = reinterpret_cast<float*>(smem_f4);
     const int rows = TP * k, C4 = c4of(C), LD = C4 + 4;
@@ -305,6 +363,7 @@ corr3d_bwd_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict
     float* sWc = reinterpret_cast<float*>(jj + rows);       // [C][9]
     float* sW1c = sWc + C * 9;                              // [C][3]
     float* sb2 = sW1c + C * 3;                              // [C]
+    float* dws = sb2 + C;                                   // DET only: [rows][LD]
     __shared__ float s_tmp[WN_SMALL];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const PartLayout L = part_layout(C);
@@ -323,6 +382,7 @@ corr3d_bwd_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict
     const int tiles_per_b = (N1 + TP - 1) / TP;
     for (int tile = blockIdx.x; tile < B * tiles_per_b; tile += gridDim.x) {
         const int b = tile / tiles_per_b, i0 = (tile - b * tiles_per_b) * TP;
+        const size_t row0 = ((size_t)b * N1 + i0) * k;      // global row of the tile's row 0
         __syncthreads();
         // (a) neighbour, offset, weight_net2 hidden layers per row
         for (int r = tid; r < rows; r += BWD_THREADS) {
@@ -390,6 +450,10 @@ corr3d_bwd_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict
                     const float z2 = acc[s];
                     const float d2 = dp * fmaxf(wpre, 0.0f) * lrelu_d(z2);
                     dz2[(size_t)r * LD + o] = d2;
+                    if constexpr (DET) {
+                        dws[(size_t)r * LD + o] = wpre > 0.0f ? dp * leaky01(z2) : 0.0f;
+                        continue;
+                    }
                     gb2 += d2;
                     const float dwpre = wpre > 0.0f ? dp * leaky01(z2) : 0.0f;
                     float du2[8];
@@ -405,12 +469,33 @@ corr3d_bwd_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict
                     }
                 }
             }
+            if constexpr (!DET) {
 #pragma unroll
-            for (int q = 0; q < 8; ++q) atomicAdd(sWc + o * 9 + q, gw[q]);
-            atomicAdd(sWc + o * 9 + 8, gb);
-            atomicAdd(sb2 + o, gb2);
+                for (int q = 0; q < 8; ++q) atomicAdd(sWc + o * 9 + q, gw[q]);
+                atomicAdd(sWc + o * 9 + 8, gb);
+                atomicAdd(sb2 + o, gb2);
+            }
         }
         __syncthreads();
+        if constexpr (DET) {
+            // (c') du2 = Wc^T dw per row (ascending o); Wc / bc / b2 partials += sums over the tile's rows (ascending r)
+            for (int e = tid; e < rows * 8; e += BWD_THREADS) {
+                const int r = e >> 3, q = e & 7;
+                float s = 0.0f;
+                for (int o = 0; o < C; ++o) s = fmaf(__ldg(WcT + (size_t)q * C + o), dws[(size_t)r * LD + o], s);
+                du2s[e] = s;
+            }
+            for (int e = tid; e < C * 10; e += BWD_THREADS) {
+                const int o = e / 10, q = e - o * 10;
+                float s = 0.0f;
+                if (q < 8)
+                    for (int r = 0; r < rows; ++r) s = fmaf(dws[(size_t)r * LD + o], u2s[r * 8 + q], s);
+                else
+                    for (int r = 0; r < rows; ++r) s += (q == 8 ? dws : dz2)[(size_t)r * LD + o];
+                if (q < 9) sWc[o * 9 + q] += s;
+                else sb2[o] += s;
+            }
+        }
         // (d) dW2 += dz2^T h1 over the tile's rows: 4x4 register blocks, read-modify-write of this CTA's partial
         for (int bi = tid; bi < nblk; bi += BWD_THREADS) {
             const int ob = bi / (C4 / 4), cb = bi - ob * (C4 / 4);
@@ -466,14 +551,29 @@ corr3d_bwd_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict
                     const float dz1 = acc[s] * lrelu_d(*hp);         // h1 > 0 exactly when z1 > 0
                     *hp = dz1;
                     da += dz1;
+                    if constexpr (DET) {
+                        if (dG2 != nullptr && i < N1) det.rows[(row0 + r) * C4 + c] = dz1;
+                        continue;
+                    }
                     if (dG2 != nullptr && i < N1) atomicAdd(dG2 + ((size_t)b * N2 + jj[r]) * C + c, dz1);
                     gx = fmaf(dz1, ds[r * 4 + 0], gx); gy = fmaf(dz1, ds[r * 4 + 1], gy); gz = fmaf(dz1, ds[r * 4 + 2], gz);
                 }
             }
             if (dA1 != nullptr && i < N1) dA1[((size_t)b * N1 + i) * C + c] = da;
-            atomicAdd(sW1c + c * 3 + 0, gx); atomicAdd(sW1c + c * 3 + 1, gy); atomicAdd(sW1c + c * 3 + 2, gz);
+            if constexpr (!DET) {
+                atomicAdd(sW1c + c * 3 + 0, gx); atomicAdd(sW1c + c * 3 + 1, gy); atomicAdd(sW1c + c * 3 + 2, gz);
+            }
         }
         __syncthreads();
+        if constexpr (DET) {
+            // (e') W1c partials += sum over the tile's rows of dz1 (x) d, ascending r
+            for (int e = tid; e < C * 3; e += BWD_THREADS) {
+                const int c = e / 3, x = e - c * 3;
+                float s = 0.0f;
+                for (int r = 0; r < rows; ++r) s = fmaf(h1[(size_t)r * LD + c], ds[r * 4 + x], s);
+                sW1c[e] += s;
+            }
+        }
         // (f) dd = W1c^T dz1: one warp per row
         for (int r = warp; r < rows; r += BWD_THREADS / 32) {
             float sx = 0.0f, sy = 0.0f, sz = 0.0f;
@@ -498,16 +598,35 @@ corr3d_bwd_stage1_kernel(const float* __restrict__ xyz1, const float* __restrict
 #pragma unroll
             for (int q = 0; q < 8; ++q) { du2s[r * 8 + q] = du2[q]; du1s[r * 8 + q] = du1[q]; }
             if (i < N1) {
-                const int j = jj[r];
+                if constexpr (DET) {
+                    float t[3];
 #pragma unroll
-                for (int x = 0; x < 3; ++x) {
-                    const float t = dds[r * 4 + x] + de[x];
-                    if (dxyz2 != nullptr) atomicAdd(dxyz2 + ((size_t)b * 3 + x) * N2 + j, t);
-                    if (dxyz1 != nullptr) atomicAdd(dxyz1 + ((size_t)b * 3 + x) * N1 + i, -t);
+                    for (int x = 0; x < 3; ++x) { t[x] = dds[r * 4 + x] + de[x]; dds[r * 4 + x] = t[x]; }
+                    if (dxyz2 != nullptr) det.xrows[row0 + r] = make_float4(t[0], t[1], t[2], 0.0f);
+                } else {
+                    const int j = jj[r];
+#pragma unroll
+                    for (int x = 0; x < 3; ++x) {
+                        const float t = dds[r * 4 + x] + de[x];
+                        if (dxyz2 != nullptr) atomicAdd(dxyz2 + ((size_t)b * 3 + x) * N2 + j, t);
+                        if (dxyz1 != nullptr) atomicAdd(dxyz1 + ((size_t)b * 3 + x) * N1 + i, -t);
+                    }
                 }
             }
         }
         __syncthreads();
+        if constexpr (DET) {
+            // (g') the point's own t rows, summed in ascending s, leave dxyz1[i] (this CTA owns point i)
+            if (dxyz1 != nullptr)
+                for (int pt = tid; pt < TP && i0 + pt < N1; pt += BWD_THREADS)
+#pragma unroll
+                    for (int x = 0; x < 3; ++x) {
+                        float s = 0.0f;
+                        for (int q = 0; q < k; ++q) s += dds[(pt * k + q) * 4 + x];
+                        float* p = dxyz1 + ((size_t)b * 3 + x) * N1 + i0 + pt;
+                        *p = *p - s;
+                    }
+        }
         {
             const int t = tid & 127, half = tid >> 7;
             if (t < WN_SMALL)
@@ -625,15 +744,20 @@ linear_bwd_x_kernel(const float* __restrict__ D, const float* __restrict__ Wm, f
 }
 
 // dW[o, coff + c] += sum_{b,n} D[b,n,o] * X[b,c,n]; column c == Cin is the constant 1 (-> dbias[o]).  Split-K over B*N.
+// DET: split z writes its partials to part[z][o][c] (c < Cx) instead; linear_bwd_w_reduce_kernel sums them.  There the
+// bias column is present when bias_col is set, whether or not dbias is wanted, so the split plan (and with it every sum
+// order) does not depend on which gradients the caller asks for.
+template <bool DET>
 __global__ void __launch_bounds__(256)
 linear_bwd_w_kernel(const float* __restrict__ D, const float* __restrict__ X, float* __restrict__ dW, float* __restrict__ dbias,
-                    int Cout, int ldw, int coff, int Cin, int N, int64_t BN, int64_t chunk) {
+                    int Cout, int ldw, int coff, int Cin, int N, int64_t BN, int64_t chunk, float* __restrict__ part,
+                    int bias_col) {
     __shared__ __align__(16) float Ds[LB_K][LB_T];       // [p][o]
     __shared__ __align__(16) float Xs[LB_K][LB_T];       // [p][c]
     const int o0 = blockIdx.x * LB_T, c0 = blockIdx.y * LB_T;
     const int64_t p_begin = blockIdx.z * chunk, p_end = min(BN, p_begin + chunk);
     const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;      // tx -> 4 in-channels, ty -> 4 out-channels
-    const int Cx = dbias ? Cin + 1 : Cin;
+    const int Cx = (DET ? bias_col : dbias != nullptr) ? Cin + 1 : Cin;
     float acc[4][4] = {};
     for (int64_t p0 = p_begin; p0 < p_end; p0 += LB_K) {
         __syncthreads();
@@ -671,40 +795,238 @@ linear_bwd_w_kernel(const float* __restrict__ D, const float* __restrict__ X, fl
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             const int c = c0 + tx * 4 + j;
-            if (c < Cin) { if (dW) atomicAdd(dW + (size_t)o * ldw + coff + c, acc[a][j]); }
-            else if (c == Cin && dbias) atomicAdd(dbias + o, acc[a][j]);
+            if constexpr (DET) {
+                if (c < Cx) part[((size_t)blockIdx.z * Cout + o) * Cx + c] = acc[a][j];
+            } else {
+                if (c < Cin) { if (dW) atomicAdd(dW + (size_t)o * ldw + coff + c, acc[a][j]); }
+                else if (c == Cin && dbias) atomicAdd(dbias + o, acc[a][j]);
+            }
         }
     }
 }
 
-static cudaError_t launch_linear_bwd_w(const float* D, const float* X, float* dW, float* dbias, int Cout, int ldw, int coff,
-                                       int Cin, int B, int N, cudaStream_t st) {
-    const int64_t BN = (int64_t)B * N;
-    const int tiles = ceil_div(Cout, LB_T) * ceil_div((dbias ? Cin + 1 : Cin), LB_T);
+// dW[o, coff + c] (c < Cin) and dbias[o] (c == Cin < Cx) = the splits' partials of linear_bwd_w_kernel<true>, ascending z
+__global__ void __launch_bounds__(256)
+linear_bwd_w_reduce_kernel(const float* __restrict__ part, int splits, float* __restrict__ dW, float* __restrict__ dbias,
+                           int Cout, int ldw, int coff, int Cin, int Cx) {
+    for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < (int64_t)Cout * Cx; e += (int64_t)gridDim.x * blockDim.x) {
+        const int o = (int)(e / Cx), c = (int)(e - (int64_t)o * Cx);
+        float s = 0.0f;
+        for (int z = 0; z < splits; ++z) s += __ldg(part + (size_t)z * Cout * Cx + e);
+        if (c < Cin) { if (dW) dW[(size_t)o * ldw + coff + c] = s; }
+        else if (dbias) dbias[o] = s;
+    }
+}
+
+// split-K plan of linear_bwd_w_kernel: number of splits, and the rows of B*N each takes
+static int64_t linear_bwd_w_splits(int Cout, int Cx, int64_t BN, int64_t* chunk_out) {
+    const int tiles = ceil_div(Cout, LB_T) * ceil_div(Cx, LB_T);
     int64_t splits = std::max<int64_t>(1, std::min<int64_t>((BN + 255) / 256, (2 * 148 + tiles - 1) / tiles));
     int64_t chunk = (BN + splits - 1) / splits;
     chunk = (chunk + LB_K - 1) / LB_K * LB_K;
-    splits = (BN + chunk - 1) / chunk;
-    linear_bwd_w_kernel<<<dim3(ceil_div(Cout, LB_T), ceil_div((dbias ? Cin + 1 : Cin), LB_T), (unsigned)splits), 256, 0, st>>>(
-        D, X, dW, dbias, Cout, ldw, coff, Cin, N, BN, chunk);
+    *chunk_out = chunk;
+    return (BN + chunk - 1) / chunk;
+}
+
+// bias_col: X gets the constant-1 column (always when dbias is wanted; on the DET path also when it is not).
+// DET: part holds linear_bwd_w_splits(Cout, Cx, B*N) * Cout * Cx floats (det_lpart_floats covers both calls).
+template <bool DET>
+static cudaError_t launch_linear_bwd_w(const float* D, const float* X, float* dW, float* dbias, bool bias_col, int Cout,
+                                       int ldw, int coff, int Cin, int B, int N, cudaStream_t st, float* part = nullptr) {
+    const int64_t BN = (int64_t)B * N;
+    const int Cx = bias_col ? Cin + 1 : Cin;
+    int64_t chunk;
+    const int64_t splits = linear_bwd_w_splits(Cout, Cx, BN, &chunk);
+    linear_bwd_w_kernel<DET><<<dim3(ceil_div(Cout, LB_T), ceil_div(Cx, LB_T), (unsigned)splits), 256, 0, st>>>(
+        D, X, dW, dbias, Cout, ldw, coff, Cin, N, BN, chunk, part, bias_col ? 1 : 0);
+    if (DET) {
+        cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return e;
+        linear_bwd_w_reduce_kernel<<<ceil_div((int64_t)Cout * Cx, 256), 256, 0, st>>>(part, (int)splits, dW, dbias, Cout, ldw,
+                                                                                      coff, Cin, Cx);
+    }
     return cudaGetLastError();
 }
 
-template <int KMAX>
+template <int KMAX, bool DET>
 static cudaError_t launch_bwd_stage1(const float* xyz1, const float* xyz2, const int64_t* knn12, const BwdScratch& s,
                                      const b200_corr3d_weights* w, float* dA1, float* dG2, float* dxyz1, float* dxyz2,
-                                     int64_t part_stride, int nparts, int B, int C, int N1, int N2, int k, cudaStream_t st) {
+                                     int64_t part_stride, int nparts, int B, int C, int N1, int N2, int k, cudaStream_t st,
+                                     DetRows det = DetRows{}) {
     int TP = 128 / k > 0 ? 128 / k : 1;
-    while (TP > 1 && s1_smem(TP, k, C) > 200 * 1024) TP /= 2;
-    if (s1_smem(TP, k, C) > 227 * 1024) return cudaErrorInvalidConfiguration;
-    const size_t smem = s1_smem(TP, k, C);
-    auto kern = corr3d_bwd_stage1_kernel<KMAX>;
+    while (TP > 1 && s1_smem(TP, k, C, DET) > 200 * 1024) TP /= 2;
+    if (s1_smem(TP, k, C, DET) > 227 * 1024) return cudaErrorInvalidConfiguration;
+    const size_t smem = s1_smem(TP, k, C, DET);
+    auto kern = corr3d_bwd_stage1_kernel<KMAX, DET>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     kern<<<nparts, BWD_THREADS, smem, st>>>(xyz1, xyz2, knn12, s.f.A1, s.f.G2, w->W2, s.f.W2T, s.f.W1cT, w->b2, w->n2_Wa, w->n2_ba,
                                            w->n2_Wb, w->n2_bb, s.f.n2WcT, w->n2_bc, s.dP, dA1, dG2, dxyz1, dxyz2, s.part,
-                                           part_stride, B, C, N1, N2, k, TP);
+                                           part_stride, B, C, N1, N2, k, TP, det);
     return cudaGetLastError();
+}
+
+// ---- deterministic path: inverse knn index (CSR) and the pull ------------------------------------------------------
+// key of row r = b*N + clamp(knn[r]) with the kernels' clamp rule; value = r
+__global__ void corr3d_det_keys_kernel(const int64_t* __restrict__ knn, int64_t R, int64_t rows_per_b, int N,
+                                       unsigned* __restrict__ keys, int* __restrict__ vals) {
+    for (int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; r < R; r += (int64_t)gridDim.x * blockDim.x) {
+        int64_t m = __ldg(knn + r);
+        m = m < 0 ? 0 : (m >= N ? N - 1 : m);
+        keys[r] = (unsigned)((r / rows_per_b) * N + m);
+        vals[r] = (int)r;
+    }
+}
+
+// offs[d] = the first sorted position whose key is >= d, d in [0, D]: destination d's rows are [offs[d], offs[d+1])
+__global__ void corr3d_det_offsets_kernel(const unsigned* __restrict__ keys, int64_t R, int64_t D, int* __restrict__ offs) {
+    for (int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; p <= R; p += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t lo = p > 0 ? (int64_t)keys[p - 1] + 1 : 0, hi = p < R ? (int64_t)keys[p] : D;
+        for (int64_t d = lo; d <= hi; ++d) offs[d] = (int)p;
+    }
+}
+
+// Destination d = b*N + n sums its rows (order[offs[d] .. offs[d+1])) in ascending row order from +0.0: dst[d][0..C)
+// from rows[r][0..C) (row stride c4of(C), 128-bit loads) and dxyz[b][0..3)[n] from xrows[r].  self_k > 0 (knn11):
+// the point's own rows d*self_k + s, summed in ascending s, are then subtracted from the dxyz sum.  NULL dst / dxyz: skipped.
+__global__ void __launch_bounds__(256)
+corr3d_det_pull_kernel(const int* __restrict__ order, const int* __restrict__ offs, const float* __restrict__ rows,
+                       float* __restrict__ dst, const float4* __restrict__ xrows, float* __restrict__ dxyz, int self_k, int C,
+                       int N, int64_t D) {
+    const int nq = dst ? c4of(C) / 4 : 0, items = nq + (dxyz ? 1 : 0);
+    for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < D * items; e += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t d = e / items;
+        const int q = (int)(e - d * items), p0 = __ldg(offs + d), p1 = __ldg(offs + d + 1);
+        float4 s = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+        if (q < nq) {
+            for (int p = p0; p < p1; ++p) {
+                const float4 v = __ldg(reinterpret_cast<const float4*>(rows + (size_t)__ldg(order + p) * (nq * 4)) + q);
+                s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+            }
+            float* out = dst + d * C + q * 4;
+            out[0] = s.x;
+            if (q * 4 + 1 < C) out[1] = s.y;
+            if (q * 4 + 2 < C) out[2] = s.z;
+            if (q * 4 + 3 < C) out[3] = s.w;
+        } else {
+            for (int p = p0; p < p1; ++p) {
+                const float4 v = __ldg(xrows + __ldg(order + p));
+                s.x += v.x; s.y += v.y; s.z += v.z;
+            }
+            float4 own = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+            for (int t = 0; t < self_k; ++t) {
+                const float4 v = __ldg(xrows + d * self_k + t);
+                own.x += v.x; own.y += v.y; own.z += v.z;
+            }
+            const int64_t b = d / N, n = d - b * N;
+            dxyz[(b * 3 + 0) * N + n] = s.x - own.x;
+            dxyz[(b * 3 + 1) * N + n] = s.y - own.y;
+            dxyz[(b * 3 + 2) * N + n] = s.z - own.z;
+        }
+    }
+}
+
+// Scratch of b200_corr3d_bwd_det: the float scratch of b200_corr3d_bwd, then the row buffers, the CSR lists of both
+// index sets, the sort's key / value buffers and its temporary storage.  Every region starts 256-byte aligned.
+struct DetScratch {
+    BwdScratch s;
+    DetRows rows;
+    float* lpart;                               // pass-4 split-K partials
+    unsigned *keys_in, *keys_out;
+    int *vals_in, *order11, *order12, *offs11, *offs12;
+    void* sort_tmp;
+    size_t sort_bytes, total;
+};
+
+static int key_bits(int64_t D) {                // bits of the largest key D - 1 (at least 1)
+    int b = 1;
+    while (b < 32 && (int64_t(1) << b) < D) ++b;
+    return b;
+}
+
+static cudaError_t sort_bytes(int64_t R, int64_t D, size_t* bytes) {
+    *bytes = 0;
+    return cub::DeviceRadixSort::SortPairs(nullptr, *bytes, (const unsigned*)nullptr, (unsigned*)nullptr, (const int*)nullptr,
+                                           (int*)nullptr, (int)R, 0, key_bits(D));
+}
+
+// pass-4 partials of the DET path: the call over feat1 always carries the bias column (Cx = Cin + 1, B*N1 rows), the
+// call over feat2 never does (Cx = Cin, B*N2 rows); the two run one after the other on one buffer
+static int64_t det_lpart_floats(int B, int Cin, int Cout, int N1, int N2) {
+    int64_t c1, c2;
+    return std::max(linear_bwd_w_splits(Cout, Cin + 1, (int64_t)B * N1, &c1) * Cout * (Cin + 1),
+                    linear_bwd_w_splits(Cout, Cin, (int64_t)B * N2, &c2) * Cout * Cin);
+}
+
+static cudaError_t carve_det(char* base, int B, int Cin, int Cout, int N1, int N2, int k, DetScratch* out) {
+    DetScratch& d = *out;
+    const int64_t R = (int64_t)B * N1 * k, D11 = (int64_t)B * N1, D12 = (int64_t)B * N2;
+    size_t sb11 = 0, sb12 = 0;
+    cudaError_t e = sort_bytes(R, D11, &sb11);
+    if (e == cudaSuccess) e = sort_bytes(R, D12, &sb12);
+    if (e != cudaSuccess) return e;
+    d.sort_bytes = std::max(sb11, sb12);
+    size_t off = 0;
+    auto take = [&](size_t bytes) { char* p = base ? base + off : nullptr; off += (bytes + 255) & ~size_t(255); return p; };
+    const int64_t nf = carve_bwd(nullptr, B, Cout, N1, N2).total;
+    d.s = carve_bwd(reinterpret_cast<float*>(take(sizeof(float) * nf)), B, Cout, N1, N2);
+    d.rows.rows = reinterpret_cast<float*>(take(sizeof(float) * R * c4of(Cout)));
+    d.rows.xrows = reinterpret_cast<float4*>(take(sizeof(float4) * R));
+    d.rows.wslice = reinterpret_cast<float*>(take(sizeof(float) * (size_t)bwd_parts(Cout) * (BWD_THREADS / 32) * 9 * Cout));
+    d.lpart = reinterpret_cast<float*>(take(sizeof(float) * det_lpart_floats(B, Cin, Cout, N1, N2)));
+    d.keys_in = reinterpret_cast<unsigned*>(take(sizeof(unsigned) * R));
+    d.keys_out = reinterpret_cast<unsigned*>(take(sizeof(unsigned) * R));
+    d.vals_in = reinterpret_cast<int*>(take(sizeof(int) * R));
+    d.order11 = reinterpret_cast<int*>(take(sizeof(int) * R));
+    d.order12 = reinterpret_cast<int*>(take(sizeof(int) * R));
+    d.offs11 = reinterpret_cast<int*>(take(sizeof(int) * (D11 + 1)));
+    d.offs12 = reinterpret_cast<int*>(take(sizeof(int) * (D12 + 1)));
+    d.sort_tmp = take(d.sort_bytes);
+    d.total = off;
+    return cudaSuccess;
+}
+
+// knn -> order (rows grouped by destination, ascending inside a group) and offs (D + 1 segment offsets)
+static cudaError_t build_csr(const int64_t* knn, int B, int N1, int N, int k, const DetScratch& d, int* order, int* offs,
+                             cudaStream_t st) {
+    const int64_t R = (int64_t)B * N1 * k, D = (int64_t)B * N;
+    const int grid = (int)std::min<int64_t>(ceil_div(R + 1, 256), 148 * 8);
+    corr3d_det_keys_kernel<<<grid, 256, 0, st>>>(knn, R, (int64_t)N1 * k, N, d.keys_in, d.vals_in);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    size_t bytes = d.sort_bytes;
+    e = cub::DeviceRadixSort::SortPairs(d.sort_tmp, bytes, d.keys_in, d.keys_out, d.vals_in, order, (int)R, 0, key_bits(D), st);
+    if (e != cudaSuccess) return e;
+    corr3d_det_offsets_kernel<<<grid, 256, 0, st>>>(d.keys_out, R, D, offs);
+    return cudaGetLastError();
+}
+
+static cudaError_t launch_pull(const int* order, const int* offs, const float* rows, float* dst, const float4* xrows, float* dxyz,
+                               int self_k, int C, int N, int64_t D, cudaStream_t st) {
+    const int64_t items = D * ((dst ? c4of(C) / 4 : 0) + (dxyz ? 1 : 0));
+    if (items == 0) return cudaSuccess;
+    corr3d_det_pull_kernel<<<(int)std::min<int64_t>(ceil_div(items, 256), 148 * 16), 256, 0, st>>>(order, offs, rows, dst, xrows,
+                                                                                                  dxyz, self_k, C, N, D);
+    return cudaGetLastError();
+}
+
+// the argument checks of both entries (fn names the entry in the messages)
+static int bwd_check(const char* fn, const float* xyz1, const float* feat1, const float* xyz2, const float* feat2,
+                     const int64_t* knn12, const int64_t* knn11, const b200_corr3d_weights* w, const float* grad_out,
+                     const float* fwd_scratch, const b200_corr3d_grads* grads, const void* scratch, int B, int Cin, int Cout,
+                     int N1, int N2, int k) {
+    B200_REQUIRE((B == 0) || (xyz1 && feat1 && xyz2 && feat2 && knn12 && knn11 && w && grad_out && fwd_scratch && grads && scratch),
+                 "%s: null pointer", fn);
+    B200_REQUIRE(B >= 0 && Cin >= 1 && Cout >= 1 && N1 >= 1 && N2 >= 1, "%s: bad sizes", fn);
+    B200_REQUIRE(k >= 1 && k <= 32, "%s: k must be in [1,32] (got %d)", fn, k);
+    B200_REQUIRE(Cout <= 512, "%s: Cout=%d exceeds 512", fn, Cout);
+    B200_REQUIRE(B <= 65535, "%s: B exceeds the grid limit", fn);
+    B200_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 15) == 0 && (reinterpret_cast<uintptr_t>(fwd_scratch) & 15) == 0,
+                 "%s: scratch and fwd_scratch must be 16-byte aligned", fn);
+    B200_REQUIRE(w != nullptr && grads != nullptr, "%s: null weight or gradient struct", fn);
+    B200_REQUIRE(w->W1 && w->b1 && w->W2 && w->b2 && w->n1_Wa && w->n1_ba && w->n1_Wb && w->n1_bb && w->n1_Wc && w->n1_bc &&
+                 w->n2_Wa && w->n2_ba && w->n2_Wb && w->n2_bb && w->n2_Wc && w->n2_bc, "%s: null weight pointer", fn);
+    return B200_OK;
 }
 
 }  // namespace b200
@@ -714,26 +1036,37 @@ extern "C" int64_t b200_corr3d_bwd_scratch_floats(int B, int Cin, int Cout, int 
     return b200::carve_bwd(nullptr, B, Cout, N1, N2).total;
 }
 
-extern "C" int b200_corr3d_bwd(const float* xyz1, const float* feat1, const float* xyz2, const float* feat2,
-                               const int64_t* knn12, const int64_t* knn11, const b200_corr3d_weights* w, const float* grad_out,
-                               const float* fwd_scratch, const b200_corr3d_grads* grads, float* scratch, int B, int Cin,
-                               int Cout, int N1, int N2, int k, b200_stream_t stream) {
-    using namespace b200;
-    B200_REQUIRE((B == 0) || (xyz1 && feat1 && xyz2 && feat2 && knn12 && knn11 && w && grad_out && fwd_scratch && grads && scratch),
-                 "b200_corr3d_bwd: null pointer");
-    B200_REQUIRE(B >= 0 && Cin >= 1 && Cout >= 1 && N1 >= 1 && N2 >= 1, "b200_corr3d_bwd: bad sizes");
-    B200_REQUIRE(k >= 1 && k <= 32, "b200_corr3d_bwd: k must be in [1,32] (got %d)", k);
-    B200_REQUIRE(Cout <= 512, "b200_corr3d_bwd: Cout=%d exceeds 512", Cout);
-    B200_REQUIRE(B <= 65535, "b200_corr3d_bwd: B exceeds the grid limit");
-    B200_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 15) == 0 && (reinterpret_cast<uintptr_t>(fwd_scratch) & 15) == 0,
-                 "b200_corr3d_bwd: scratch and fwd_scratch must be 16-byte aligned");
-    B200_REQUIRE(w != nullptr && grads != nullptr, "b200_corr3d_bwd: null weight or gradient struct");
-    B200_REQUIRE(w->W1 && w->b1 && w->W2 && w->b2 && w->n1_Wa && w->n1_ba && w->n1_Wb && w->n1_bb && w->n1_Wc && w->n1_bc &&
-                 w->n2_Wa && w->n2_ba && w->n2_Wb && w->n2_bb && w->n2_Wc && w->n2_bc, "b200_corr3d_bwd: null weight pointer");
+
+extern "C" int64_t b200_corr3d_bwd_det_scratch_bytes(int B, int Cin, int Cout, int N1, int N2, int k) {
+    if (B < 1 || Cin < 1 || Cout < 1 || N1 < 1 || N2 < 1 || k < 1) return 0;
+    b200::DetScratch d;
+    const cudaError_t e = b200::carve_det(nullptr, B, Cin, Cout, N1, N2, k, &d);
+    if (e != cudaSuccess) return b200::cuda_fail(e, "b200_corr3d_bwd_det_scratch_bytes (cub::DeviceRadixSort temporary size)");
+    return (int64_t)d.total;
+}
+
+namespace b200 {
+
+// The body of both entries: DET = false is b200_corr3d_bwd (float atomics), DET = true b200_corr3d_bwd_det.
+template <bool DET>
+static int corr3d_bwd_run(const char* fn, const float* xyz1, const float* feat1, const float* xyz2, const float* feat2,
+                          const int64_t* knn12, const int64_t* knn11, const b200_corr3d_weights* w, const float* grad_out,
+                          const float* fwd_scratch, const b200_corr3d_grads* grads, float* scratch, int B, int Cin, int Cout,
+                          int N1, int N2, int k, b200_stream_t stream) {
+    const int rc = bwd_check(fn, xyz1, feat1, xyz2, feat2, knn12, knn11, w, grad_out, fwd_scratch, grads, scratch, B, Cin, Cout,
+                             N1, N2, k);
+    if (rc != B200_OK) return rc;
     if (B == 0) return B200_OK;
+    if (DET)
+        B200_REQUIRE((int64_t)B * N1 * k <= INT_MAX && (int64_t)B * N2 <= INT_MAX, "%s: B*N1*k and B*N2 must be below 2^31", fn);
     cudaStream_t st = as_stream(stream);
     const b200_corr3d_grads& g = *grads;
-    const BwdScratch s = carve_bwd(scratch, B, Cout, N1, N2);
+    DetScratch d{};
+    if (DET) {
+        const cudaError_t e = carve_det(reinterpret_cast<char*>(scratch), B, Cin, Cout, N1, N2, k, &d);
+        if (e != cudaSuccess) return cuda_fail(e, "cub::DeviceRadixSort (temporary size)");
+    }
+    const BwdScratch s = DET ? d.s : carve_bwd(scratch, B, Cout, N1, N2);
     const float* P = carve(const_cast<float*>(fwd_scratch), B, Cout, N1, N2).P;
     const int Kin = 2 * Cin + 3;
     const PartLayout L = part_layout(Cout);
@@ -745,35 +1078,46 @@ extern "C" int b200_corr3d_bwd(const float* xyz1, const float* feat1, const floa
     const bool need_dA1 = g.feat1 || g.W1 || g.b1, need_dG2 = g.feat2 || g.W1;
     if (!need_s1 && !need_n1 && !g.xyz1) return B200_OK;
 
-    if (g.xyz1) B200_CUDA(cudaMemsetAsync(g.xyz1, 0, sizeof(float) * 3 * B * (size_t)N1, st));
-    if (g.xyz2) B200_CUDA(cudaMemsetAsync(g.xyz2, 0, sizeof(float) * 3 * B * (size_t)N2, st));
-    if (g.W1) B200_CUDA(cudaMemsetAsync(g.W1, 0, sizeof(float) * (size_t)Cout * Kin, st));
-    if (g.b1) B200_CUDA(cudaMemsetAsync(g.b1, 0, sizeof(float) * Cout, st));
-    if (need_s1) B200_CUDA(cudaMemsetAsync(s.dP, 0, sizeof(float) * (size_t)B * N1 * Cout, st));
-    if (need_s1 && need_dG2) B200_CUDA(cudaMemsetAsync(s.dG2, 0, sizeof(float) * (size_t)B * N2 * Cout, st));
+    if (DET) {
+        // every output is written whole, nothing accumulates: no zero-fill.  need_s1 covers g.xyz1, g.xyz2 and need_dG2.
+        if (need_s1) B200_CUDA(build_csr(knn11, B, N1, N1, k, d, d.order11, d.offs11, st));
+        if (need_dG2 || g.xyz2) B200_CUDA(build_csr(knn12, B, N1, N2, k, d, d.order12, d.offs12, st));
+    } else {
+        if (g.xyz1) B200_CUDA(cudaMemsetAsync(g.xyz1, 0, sizeof(float) * 3 * B * (size_t)N1, st));
+        if (g.xyz2) B200_CUDA(cudaMemsetAsync(g.xyz2, 0, sizeof(float) * 3 * B * (size_t)N2, st));
+        if (g.W1) B200_CUDA(cudaMemsetAsync(g.W1, 0, sizeof(float) * (size_t)Cout * Kin, st));
+        if (g.b1) B200_CUDA(cudaMemsetAsync(g.b1, 0, sizeof(float) * Cout, st));
+        if (need_s1) B200_CUDA(cudaMemsetAsync(s.dP, 0, sizeof(float) * (size_t)B * N1 * Cout, st));
+        if (need_s1 && need_dG2) B200_CUDA(cudaMemsetAsync(s.dG2, 0, sizeof(float) * (size_t)B * N2 * Cout, st));
+    }
 
     // pass 1: stage-2 backward (dP, weight_net1, dxyz1 via e)
     {
         const int rows = S2_TP * k;
         const size_t smem = ((size_t)Cout * 17 + (size_t)rows * (8 + 8 + 4 + 8 + 8 + 1) + (size_t)Cout * 9) * sizeof(float);
-        cudaError_t e = cudaFuncSetAttribute(corr3d_bwd_stage2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        auto kern = corr3d_bwd_stage2_kernel<DET>;
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return cuda_fail(e, "corr3d_bwd_stage2_kernel(attr)");
-        corr3d_bwd_stage2_kernel<<<nparts, BWD_THREADS, smem, st>>>(
+        kern<<<nparts, BWD_THREADS, smem, st>>>(
             xyz1, knn11, P, grad_out, w->n1_Wa, w->n1_ba, w->n1_Wb, w->n1_bb, w->n1_Wc, w->n1_bc, need_s1 ? s.dP : nullptr,
-            g.xyz1, s.part, L.total, B, Cout, N1, k, (need_n1 || g.xyz1) ? 1 : 0);
+            g.xyz1, s.part, L.total, B, Cout, N1, k, (need_n1 || g.xyz1) ? 1 : 0, d.rows);
         B200_LAUNCH_CHECK("corr3d_bwd_stage2_kernel");
     }
+    if (DET && need_s1)        // dP and dxyz1 = pulled de - own de; pass 2 reads dP
+        B200_CUDA(launch_pull(d.order11, d.offs11, d.rows.rows, s.dP, d.rows.xrows, g.xyz1, k, Cout, N1, (int64_t)B * N1, st));
     if (need_s1) {
         const cudaError_t ep = corr3d_prep_and_linears(feat1, feat2, w, s.f, B, Cin, Cout, N1, N2, st);
         if (ep != cudaSuccess) return cuda_fail(ep, "corr3d_prep_weights / pointwise_linear_kernel");
         float* dA1 = need_dA1 ? s.dA1 : nullptr;
         float* dG2 = need_dG2 ? s.dG2 : nullptr;
         cudaError_t e;
-        if (k <= 4) e = launch_bwd_stage1<4>(xyz1, xyz2, knn12, s, w, dA1, dG2, g.xyz1, g.xyz2, L.total, nparts, B, Cout, N1, N2, k, st);
-        else if (k <= 8) e = launch_bwd_stage1<8>(xyz1, xyz2, knn12, s, w, dA1, dG2, g.xyz1, g.xyz2, L.total, nparts, B, Cout, N1, N2, k, st);
-        else if (k <= 16) e = launch_bwd_stage1<16>(xyz1, xyz2, knn12, s, w, dA1, dG2, g.xyz1, g.xyz2, L.total, nparts, B, Cout, N1, N2, k, st);
-        else e = launch_bwd_stage1<32>(xyz1, xyz2, knn12, s, w, dA1, dG2, g.xyz1, g.xyz2, L.total, nparts, B, Cout, N1, N2, k, st);
+        if (k <= 4) e = launch_bwd_stage1<4, DET>(xyz1, xyz2, knn12, s, w, dA1, dG2, g.xyz1, g.xyz2, L.total, nparts, B, Cout, N1, N2, k, st, d.rows);
+        else if (k <= 8) e = launch_bwd_stage1<8, DET>(xyz1, xyz2, knn12, s, w, dA1, dG2, g.xyz1, g.xyz2, L.total, nparts, B, Cout, N1, N2, k, st, d.rows);
+        else if (k <= 16) e = launch_bwd_stage1<16, DET>(xyz1, xyz2, knn12, s, w, dA1, dG2, g.xyz1, g.xyz2, L.total, nparts, B, Cout, N1, N2, k, st, d.rows);
+        else e = launch_bwd_stage1<32, DET>(xyz1, xyz2, knn12, s, w, dA1, dG2, g.xyz1, g.xyz2, L.total, nparts, B, Cout, N1, N2, k, st, d.rows);
         if (e != cudaSuccess) return cuda_fail(e, "corr3d_bwd_stage1_kernel");
+        if (DET && (dG2 || g.xyz2))
+            B200_CUDA(launch_pull(d.order12, d.offs12, d.rows.rows, dG2, d.rows.xrows, g.xyz2, 0, Cout, N2, (int64_t)B * N2, st));
     }
     corr3d_bwd_reduce_kernel<<<ceil_div(L.total, 256), 256, 0, st>>>(s.part, L.total, nparts, g, Cout, Cin, need_s1 ? 1 : 0,
                                                                       need_n1 ? 1 : 0);
@@ -789,8 +1133,28 @@ extern "C" int b200_corr3d_bwd(const float* xyz1, const float* feat1, const floa
                                                                                              Cin, N2);
     B200_LAUNCH_CHECK("linear_bwd_x_kernel");
     cudaError_t e = cudaSuccess;
-    if (g.W1 || g.b1) e = launch_linear_bwd_w(s.dA1, feat1, g.W1, g.b1, Cout, Kin, 0, Cin, B, N1, st);
-    if (e == cudaSuccess && g.W1) e = launch_linear_bwd_w(s.dG2, feat2, g.W1, nullptr, Cout, Kin, Cin, Cin, B, N2, st);
+    if (g.W1 || g.b1)
+        e = launch_linear_bwd_w<DET>(s.dA1, feat1, g.W1, g.b1, DET || g.b1, Cout, Kin, 0, Cin, B, N1, st, d.lpart);
+    if (e == cudaSuccess && g.W1)
+        e = launch_linear_bwd_w<DET>(s.dG2, feat2, g.W1, nullptr, false, Cout, Kin, Cin, Cin, B, N2, st, d.lpart);
     if (e != cudaSuccess) return cuda_fail(e, "linear_bwd_w_kernel");
     return B200_OK;
+}
+
+}  // namespace b200
+
+extern "C" int b200_corr3d_bwd(const float* xyz1, const float* feat1, const float* xyz2, const float* feat2,
+                               const int64_t* knn12, const int64_t* knn11, const b200_corr3d_weights* w, const float* grad_out,
+                               const float* fwd_scratch, const b200_corr3d_grads* grads, float* scratch, int B, int Cin,
+                               int Cout, int N1, int N2, int k, b200_stream_t stream) {
+    return b200::corr3d_bwd_run<false>("b200_corr3d_bwd", xyz1, feat1, xyz2, feat2, knn12, knn11, w, grad_out, fwd_scratch,
+                                       grads, scratch, B, Cin, Cout, N1, N2, k, stream);
+}
+
+extern "C" int b200_corr3d_bwd_det(const float* xyz1, const float* feat1, const float* xyz2, const float* feat2,
+                                   const int64_t* knn12, const int64_t* knn11, const b200_corr3d_weights* w,
+                                   const float* grad_out, const float* fwd_scratch, const b200_corr3d_grads* grads,
+                                   float* scratch, int B, int Cin, int Cout, int N1, int N2, int k, b200_stream_t stream) {
+    return b200::corr3d_bwd_run<true>("b200_corr3d_bwd_det", xyz1, feat1, xyz2, feat2, knn12, knn11, w, grad_out, fwd_scratch,
+                                      grads, scratch, B, Cin, Cout, N1, N2, k, stream);
 }

@@ -26,7 +26,8 @@ built for; anything else goes to the reference's own function, untouched.  ``sta
 ``install(train=...)`` additionally sends calls that DO need a graph to this library's forward and backward, unless
 ``torch.use_deterministic_algorithms(True)`` is set and the op's backward sums with float atomics: those go to the
 reference.  ``train`` is a collection of op names from ``TRAINABLE``:
-- "Correlation3D": ``pwc3d.Correlation3DFunction``, b200_corr3d_fwd / b200_corr3d_bwd;
+- "Correlation3D": ``pwc3d.Correlation3DFunction``, b200_corr3d_fwd / b200_corr3d_bwd.  Under deterministic mode its
+  backward is b200_corr3d_bwd_det, which has no atomics, so this one also trains here under deterministic mode;
 - "PointConv": ``PointConvDownSampling`` / ``PointConvNoSampling`` through ``pointconv.PointConvFunction``,
   b200_pointconv_fwd_linear / b200_pointconv_bwd, followed by the module's own ``norm_fn`` and ``activation_fn``, so a
   training-mode BatchNorm1d or SyncBatchNorm runs as the reference runs it;
@@ -172,7 +173,7 @@ def _corr3d_forward(self, xyz1, feat1, xyz2, feat2, knn_indices_1in1=None):
     import torch.nn as nn
     plain = all(isinstance(c.norm_fn, nn.Identity) for mlp in (self.cost_mlp, self.weight_net1, self.weight_net2) for c in mlp.convs)
     fits = _all_cuda_f32(xyz1, feat1, xyz2, feat2) and plain and self.k <= 32 and feat1.shape[1] <= 512
-    if fits and "Correlation3D" in _TRAIN and _needs_graph(self, xyz1, feat1, xyz2, feat2) and not torch.are_deterministic_algorithms_enabled():
+    if fits and "Correlation3D" in _TRAIN and _needs_graph(self, xyz1, feat1, xyz2, feat2):
         _count("Correlation3D.forward", "b200")
         knn12 = ops.k_nearest_neighbor(input_xyz=xyz2.detach(), query_xyz=xyz1.detach(), k=self.k)
         if knn_indices_1in1 is None:

@@ -8,7 +8,8 @@ The whole forward is the fused sm_100a path of ``b200_corr3d_fwd`` (+ ``b200_knn
 By default the module is forward-only: ``forward`` refuses to run while gradients are enabled for any input/parameter
 that requires them.  ``Correlation3D(..., differentiable=True)`` and the functional ``correlation3d`` train through
 ``Correlation3DFunction`` instead, whose backward is ``b200_corr3d_bwd`` (gradients of both clouds, both feature maps
-and all 16 parameters; only the inputs, the indices and the forward's per-point ``P`` rows are kept for it).
+and all 16 parameters; only the inputs, the indices and the forward's per-point ``P`` rows are kept for it), or
+``b200_corr3d_bwd_det`` under ``torch.use_deterministic_algorithms(True)``: no float atomics, bit-reproducible.
 """
 import ctypes
 
@@ -16,7 +17,7 @@ import torch
 import torch.nn as nn
 from torch.autograd.function import once_differentiable
 
-from ._lib import Corr3dGrads, Corr3dWeights, check, lib, require_dense
+from ._lib import B200Error, Corr3dGrads, Corr3dWeights, check, lib, require_dense
 from .ops import k_nearest_neighbor
 
 __all__ = ["Correlation3D", "Correlation3DFunction", "correlation3d", "correlation3d_forward", "pack_weights",
@@ -108,14 +109,13 @@ class Correlation3DFunction(torch.autograd.Function):
 
     Tensors are CUDA, contiguous fp32 (indices int64).  Forward is b200_corr3d_fwd, the same call as
     correlation3d_forward (bit-identical output); its scratch is kept for the backward, which reads P from it.
-    Backward is b200_corr3d_bwd in fp32; gradients autograd does not ask for are not computed.  The gradients are
-    summed with float atomics, so this raises under torch.use_deterministic_algorithms(True)."""
+    Backward is fp32; gradients autograd does not ask for are not computed.  It is b200_corr3d_bwd, which sums
+    gradients with float atomics, or, when torch.are_deterministic_algorithms_enabled() is true as the backward runs,
+    b200_corr3d_bwd_det: no atomics, every gradient the same bit for bit on every run, and each sample's input gradients
+    independent of the rest of the batch (the sum order is stated in include/b200flow.h)."""
 
     @staticmethod
     def forward(ctx, xyz1, feat1, xyz2, feat2, knn12, knn11, precision, *params):
-        if torch.are_deterministic_algorithms_enabled():
-            raise RuntimeError("rpeflow_b200.correlation3d: the backward sums gradients with float atomics and is not "
-                               "deterministic; torch.use_deterministic_algorithms(True) is set")
         # a non-contiguous or non-fp32 argument used to be read through its raw pointer: silently wrong out and gradients
         require_dense("Correlation3DFunction", xyz1=xyz1, feat1=feat1, xyz2=xyz2, feat2=feat2, knn12=knn12, knn11=knn11,
                       **dict(zip(Corr3dWeights.NAMES, params)))
@@ -142,13 +142,21 @@ class Correlation3DFunction(torch.autograd.Function):
         w = Corr3dWeights(**{n: p.data_ptr() for n, p in zip(Corr3dWeights.NAMES, params)})
         g = Corr3dGrads(**{n: (t.data_ptr() if t is not None else None)
                            for n, t in zip(Corr3dGrads.NAMES, grads_in + grads_w)})
-        bwd_scratch = torch.empty((lib.b200_corr3d_bwd_scratch_floats(B, Cin, Cout, N1, N2, k),), dtype=torch.float32,
-                                  device=xyz1.device)
         with torch.cuda.device(xyz1.device):
-            check(lib.b200_corr3d_bwd(xyz1.data_ptr(), feat1.data_ptr(), xyz2.data_ptr(), feat2.data_ptr(),
+            if torch.are_deterministic_algorithms_enabled():
+                entry = "b200_corr3d_bwd_det"
+                nbytes = lib.b200_corr3d_bwd_det_scratch_bytes(B, Cin, Cout, N1, N2, k)
+                if nbytes < 0:
+                    raise B200Error(f"b200_corr3d_bwd_det_scratch_bytes failed: {lib.b200_last_error().decode()}")
+                bwd_scratch = torch.empty((nbytes,), dtype=torch.uint8, device=xyz1.device)
+            else:
+                entry = "b200_corr3d_bwd"
+                bwd_scratch = torch.empty((lib.b200_corr3d_bwd_scratch_floats(B, Cin, Cout, N1, N2, k),),
+                                          dtype=torch.float32, device=xyz1.device)
+            check(getattr(lib, entry)(xyz1.data_ptr(), feat1.data_ptr(), xyz2.data_ptr(), feat2.data_ptr(),
                                       knn12.data_ptr(), knn11.data_ptr(), ctypes.byref(w), grad_out.data_ptr(),
                                       scratch.data_ptr(), ctypes.byref(g), bwd_scratch.data_ptr(), B, Cin, Cout, N1, N2, k,
-                                      torch.cuda.current_stream(xyz1.device).cuda_stream), "b200_corr3d_bwd")
+                                      torch.cuda.current_stream(xyz1.device).cuda_stream), entry)
         return (*grads_in, None, None, None, *grads_w)
 
 
